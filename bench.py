@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — embed+detect FPS of the watermark hot path on B200 (BASELINE.json metric), one JSON line.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload video4k|image1080p|image4k|image8k|batch256|image512|all]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload video4k|image1080p|image4k|image8k|batch256|image512|all] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference ...      # the reference path on the host CPU cores (oracle port, all threads)
 
@@ -255,6 +255,9 @@ def main():
     ap.add_argument("--run-mb", type=int, default=0, help="WM_OPT_RUN_MB: MB of device frames per run of the video driver (A/B)")
     ap.add_argument("--host-run", type=int, default=0, help="WM_OPT_HOST_RUN_FRAMES for the e2e video path (A/B)")
     ap.add_argument("--e2e-frames", type=int, default=0, help="frames per e2e pass (0 = 128 for video, 96 for images)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of each workload computed (rank 0's frames) as "
+                    "DIR/<workload>_<array>.npy in float32: per frame a and correlation of each mask type, and a fixed sample of "
+                    "%d watermarked pixels per mask type (all of them when fewer)" % DUMP_PIXELS)
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
@@ -424,6 +427,9 @@ def run_workload(args, wl, torch, dist, dev, rank, local_rank, world, secondary=
         t1 = time.time()
         ms = e0.elapsed_time(e1)
         launches = wm.launch_count - l0
+        # before anything else runs on the frames: the passes below recompute or overwrite the outputs
+        outputs = last_step_outputs(torch, dev, d_out, a_host, c_host, kind, layout == pkg.ROW_MAJOR, rows, cols) \
+            if args.dump_outputs and rank == 0 else None
         # per-kernel durations for the roofline: one more pass with CUDA-event brackets around every kernel family of every call, the video
         # driver's slots serialised (wm option 4) so that a bracket holds one kernel family and nothing else
         if kind == "video":
@@ -587,7 +593,33 @@ def run_workload(args, wl, torch, dist, dev, rank, local_rank, world, secondary=
         "clocks": clocks,
         "results": {"a_nvf": float(a_host[0][0]), "a_me": float(a_host[1][0]), "corr_nvf": float(c_host[0][0]), "corr_me": float(c_host[1][0])},
     }
+    if outputs is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in outputs.items():
+            np.save(os.path.join(args.dump_outputs, "%s_%s.npy" % (wl, name)), arr)
     return line
+
+
+DUMP_PIXELS = 1 << 20  # per mask type: the dumps of a `--workload all` run (11 outputs) stay under 64 MB
+
+
+def last_step_outputs(torch, dev, d_out, a_host, c_host, kind, row_major, rows, cols):
+    """What a caller of the timed path holds after its last step, as float32 arrays: per frame the strength factor `a` and the
+    correlation of each mask type, and the watermarked frames as a seeded sample of logical (frame, row, col) positions that is the
+    same in every run with the same frame count and shape."""
+    count = d_out[0].shape[0]
+    npx = rows * cols
+    n = count * npx
+    pick = np.arange(n) if n <= DUMP_PIXELS else np.sort(np.random.default_rng(28390211).choice(n, DUMP_PIXELS, replace=False))
+    f, r, c = pick // npx, pick % npx // cols, pick % cols
+    idx = torch.from_numpy(f * npx + (r * cols + c if row_major else c * rows + r)).to(dev)
+    masks = [("me", 0, 1)] if kind == "video" else [("nvf", 0, 0), ("me", 1, 1)]  # (name, index in d_out, index in a_host / c_host)
+    out = {}
+    for name, k, s in masks:
+        out[name + "_a"] = a_host[s].astype(np.float32)
+        out[name + "_corr"] = c_host[s].astype(np.float32)
+        out[name + "_out_sample"] = d_out[k].reshape(-1).index_select(0, idx).float().cpu().numpy()
+    return out
 
 
 def run_e2e(args, pkg, torch, dist, dev, wm, wl, d_in, a_host, c_host, first, world):
