@@ -60,6 +60,7 @@ struct Slot {
     void* stage_base = nullptr; size_t stage_base_cap = 0;
     void* stage_out = nullptr; size_t stage_out_cap = 0;
     void* maskp = nullptr; size_t maskp_cap = 0;  // NVF mask planes of a batch when p > 3 (k_nvfp)
+    void* gray = nullptr; size_t gray_cap = 0;    // f32 gray planes of a packed RGB / BGR batch (k_packed_gray)
     std::vector<TimedLaunch> timed;
     // direct delivery of synchronous single-image ops (slot 0 only): mapped pinned result + device sequence / completion counters
     HostResult* hres = nullptr;      // pinned host memory
@@ -122,14 +123,32 @@ int fail(wm_ctx* c, int code, const std::string& msg)
 
 struct View {  // an image reduced to lines x pixels
     void* ptr; int L, P; long long ld, pstride; int channels; int dtype; bool transposed;
+    bool packed, bgr;  // WM_PACKED_RGB / WM_PACKED_BGR: L = rows, P = cols (pixels), ld in bytes (>= 3 P), channels 3, dtype u8
 };
 
-int make_view(wm_ctx* ctx, const wm_image* im, View* v, bool allow_rgb)
+// allow_packed: the caller handles packed 8-bit RGB / BGR images (the embed and detect entry points)
+int make_view(wm_ctx* ctx, const wm_image* im, View* v, bool allow_rgb, bool allow_packed = false)
 {
     if (!im || !im->data) return fail(ctx, WM_ERR_ARG, "null image");
     if (im->rows != ctx->rows || im->cols != ctx->cols)
         return fail(ctx, WM_ERR_DIMS, "image dims " + std::to_string(im->rows) + "x" + std::to_string(im->cols) +
                                           " != watermark dims " + std::to_string(ctx->rows) + "x" + std::to_string(ctx->cols));
+    v->packed = im->layout == WM_PACKED_RGB || im->layout == WM_PACKED_BGR;
+    v->bgr = im->layout == WM_PACKED_BGR;
+    if (v->packed) {
+        if (!allow_packed) return fail(ctx, WM_ERR_ARG, "packed RGB / BGR images are taken by the wm_embed* and wm_detect* entry points only");
+        if (im->dtype != WM_U8 || im->channels != 3) return fail(ctx, WM_ERR_ARG, "a packed RGB / BGR image has dtype WM_U8 and 3 channels");
+        v->transposed = false;
+        v->L = (int)im->rows;
+        v->P = (int)im->cols;
+        v->ld = im->ld > 0 ? im->ld : 3LL * v->P;
+        if (v->ld < 3LL * v->P) return fail(ctx, WM_ERR_ARG, "packed image: ld (bytes) smaller than 3 * cols");
+        v->pstride = 0;
+        v->channels = 3;
+        v->dtype = WM_U8;
+        v->ptr = im->data;
+        return WM_OK;
+    }
     if (im->layout != WM_COL_MAJOR && im->layout != WM_ROW_MAJOR) return fail(ctx, WM_ERR_ARG, "bad layout");
     if (im->dtype != WM_F32 && im->dtype != WM_U8) return fail(ctx, WM_ERR_ARG, "bad dtype");
     const int ch = im->channels <= 0 ? 1 : im->channels;
@@ -158,8 +177,9 @@ bool vec_ok(const void* p, long long ld, long long bstride, long long pstride, i
 // apply kernel's base / out addressing all see the same number.
 int resolve_stride(wm_ctx* ctx, const View& v, int batch, int64_t* stride, const char* what)
 {
-    const long long one = v.pstride * (v.channels - 1) + (long long)v.L * v.ld;  // elements spanned by one image
-    if (*stride == 0) *stride = v.pstride * v.channels;
+    // elements (bytes for packed images: one interleaved plane) spanned by one image
+    const long long one = v.packed ? (long long)v.L * v.ld : v.pstride * (v.channels - 1) + (long long)v.L * v.ld;
+    if (*stride == 0) *stride = v.packed ? one : v.pstride * v.channels;
     if (batch > 1 && *stride < one) return fail(ctx, WM_ERR_ARG, std::string(what) + " batch stride smaller than one image");
     return WM_OK;
 }
@@ -167,7 +187,8 @@ int resolve_stride(wm_ctx* ctx, const View& v, int batch, int64_t* stride, const
 void byte_range(const View& v, int64_t stride, int batch, uintptr_t* lo, uintptr_t* hi)
 {
     const long long es = v.dtype == WM_F32 ? 4 : 1;
-    const long long last = (long long)(batch - 1) * stride + v.pstride * (v.channels - 1) + (long long)(v.L - 1) * v.ld + v.P;
+    const long long last = (long long)(batch - 1) * stride + (long long)(v.L - 1) * v.ld +
+                           (v.packed ? 3LL * v.P : v.pstride * (v.channels - 1) + v.P);
     *lo = (uintptr_t)v.ptr;
     *hi = (uintptr_t)v.ptr + (uintptr_t)(last * es);
 }
@@ -502,6 +523,28 @@ int enqueue_nvf_planes(wm_ctx* ctx, Slot& s, const View& v, long long bstride, i
     return WM_OK;
 }
 
+// Packed RGB / BGR batch: its gray goes into the slot's dense f32 planes, and *v / *stride become that gray batch, so the op runs on it
+// exactly as on a caller's dense f32 gray batch (same tiles, launch plan and partial sums: the scalars of the composed path).
+int enqueue_packed_gray(wm_ctx* ctx, Slot& s, View* v, int64_t* stride, int batch)
+{
+    const size_t plane = (size_t)v->L * v->P, need = plane * sizeof(float) * batch;
+    if (need > s.gray_cap) {  // queued work and captured graphs may still read the old planes
+        if (!s.queue.empty()) { const int r = finish_slot(ctx, s); if (r < 0) return r; }
+        CU(cudaStreamSynchronize(s.stream));
+        clear_graphs(ctx);
+        const int rc = ensure_stage(ctx, &s.gray, &s.gray_cap, need);
+        if (rc) return rc;
+    }
+    launch_packed_gray((const uint8_t*)v->ptr, v->ld, *stride, batch, v->bgr, (float*)s.gray, v->L, v->P, vec_ok(v->ptr, v->ld, *stride, 0, WM_U8),
+                       8 * ctx->sms, s.stream);
+    ctx->launches++;
+    CU(cudaGetLastError());
+    v->ptr = s.gray; v->ld = v->P; v->pstride = (long long)plane; v->channels = 1; v->dtype = WM_F32;
+    v->packed = v->bgr = false;
+    *stride = (int64_t)plane;
+    return WM_OK;
+}
+
 size_t stats_part_offset(const Plan& pl, int batch) { return (size_t)batch * (size_t)pl.nsweep * NTOT; }
 
 // the pieces of a slot that direct delivery needs (created on first use)
@@ -532,15 +575,24 @@ int do_embed(wm_ctx* ctx, int slot, const wm_image* in, const wm_image* base, wm
     if (batch < 1 || batch > 65535) return fail(ctx, WM_ERR_ARG, "batch must be 1..65535");
     View vi, vb, vo;
     int rc;
-    if ((rc = make_view(ctx, in, &vi, false))) return rc;
-    if ((rc = make_view(ctx, base ? base : in, &vb, true))) return rc;
-    if ((rc = make_view(ctx, out, &vo, true))) return rc;
+    if ((rc = make_view(ctx, in, &vi, false, true))) return rc;
+    if ((rc = make_view(ctx, base ? base : in, &vb, true, true))) return rc;
+    if ((rc = make_view(ctx, out, &vo, true, true))) return rc;
+    const bool packed = vi.packed;
+    if (packed || vb.packed || vo.packed) {
+        if (!packed) return fail(ctx, WM_ERR_ARG, "a packed RGB / BGR base or output needs the same packed image as the input");
+        if (!vb.packed || vb.ptr != vi.ptr || vb.ld != vi.ld || vb.bgr != vi.bgr)
+            return fail(ctx, WM_ERR_ARG, "with a packed RGB / BGR input, base must be NULL or the same image (pointer, layout, ld)");
+        if (!vo.packed || vo.bgr != vi.bgr) return fail(ctx, WM_ERR_ARG, "with a packed RGB / BGR input, out must be a packed image of the same layout");
+        if (!base) base_stride = in_stride;  // NULL base: the input batch itself
+    }
     if (vb.transposed != vi.transposed || vo.transposed != vi.transposed) return fail(ctx, WM_ERR_ARG, "in/base/out layouts differ");
     if (vb.dtype != vi.dtype) return fail(ctx, WM_ERR_ARG, "base dtype must equal input dtype");
     if (vo.channels != vb.channels) return fail(ctx, WM_ERR_ARG, "out channels != base channels");
     if ((rc = resolve_stride(ctx, vi, batch, &in_stride, "in"))) return rc;
     if ((rc = resolve_stride(ctx, vb, batch, &base_stride, "base"))) return rc;
     if ((rc = resolve_stride(ctx, vo, batch, &out_stride, "out"))) return rc;
+    if (packed && batch > 1 && base_stride != in_stride) return fail(ctx, WM_ERR_ARG, "with a packed RGB / BGR input, base must be the same batch (stride)");
     {
         uintptr_t ilo, ihi, olo, ohi;
         byte_range(vi, in_stride, batch, &ilo, &ihi);
@@ -549,6 +601,7 @@ int do_embed(wm_ctx* ctx, int slot, const wm_image* in, const wm_image* base, wm
     }
     CU(cudaSetDevice(ctx->device));
     Slot& s = ctx->slots[slot];
+    if (packed && (rc = enqueue_packed_gray(ctx, s, &vi, &in_stride, batch))) return rc;
     const Geo g = geo(vi.L, vi.P);
     const bool narrow = ctx->opt_narrow_u8 && vi.dtype == WM_U8 && tma_ok(ctx, vi, in_stride, batch);
     const Plan pl = plan(ctx, g, batch, vi.dtype, narrow);
@@ -611,6 +664,7 @@ int do_embed(wm_ctx* ctx, int slot, const wm_image* in, const wm_image* base, wm
             ea.b0 = sb.b0; ea.nblk_base = sb.base; ea.nblk_extra = sb.extra;
             const dim3 grid(sb.base + (sb.extra > 0 ? 1 : 0), sb.nb);
             if (ts) launch_apply_ts(vi.dtype, kmask, vi.transposed, narrow, grid, s.stream, tmI, tmW, tmO, ea);
+            else if (packed) launch_apply_packed(kmask, tma, grid, s.stream, tmI, tmW, ea);
             else launch_apply(vi.dtype, vo.dtype, kmask, vi.transposed, tma, grid, s.stream, tmI, tmW, ea);
         }
     }
@@ -628,10 +682,11 @@ int do_detect(wm_ctx* ctx, int slot, const wm_image* img, int64_t img_stride, in
     if (batch < 1 || batch > 65535) return fail(ctx, WM_ERR_ARG, "batch must be 1..65535");
     View v;
     int rc;
-    if ((rc = make_view(ctx, img, &v, false))) return rc;
+    if ((rc = make_view(ctx, img, &v, false, true))) return rc;
     if ((rc = resolve_stride(ctx, v, batch, &img_stride, "image"))) return rc;
     CU(cudaSetDevice(ctx->device));
     Slot& s = ctx->slots[slot];
+    if (v.packed && (rc = enqueue_packed_gray(ctx, s, &v, &img_stride, batch))) return rc;
     const Geo g = geo(v.L, v.P);
     bool tma = tma_ok(ctx, v, img_stride, batch);
     const bool narrow = ctx->opt_narrow_u8 && v.dtype == WM_U8 && tma && !dbg_u;
@@ -771,6 +826,7 @@ void free_slot(Slot& s)
     if (s.stage_base) cudaFree(s.stage_base);
     if (s.stage_out) cudaFree(s.stage_out);
     if (s.maskp) cudaFree(s.maskp);
+    if (s.gray) cudaFree(s.gray);
     if (s.hres) cudaFreeHost(s.hres);
     if (s.dl_words) cudaFree(s.dl_words);
     for (auto& t : s.timed) { cudaEventDestroy(t.e0); cudaEventDestroy(t.e1); }
@@ -1079,6 +1135,14 @@ struct HostGeo { int64_t L, P, ld, ps; int ch; size_t es; };
 static int host_geo(wm_ctx* ctx, const wm_image* im, HostGeo* g)
 {
     if (!im || !im->data) return fail(ctx, WM_ERR_ARG, "null image");
+    if (im->layout == WM_PACKED_RGB || im->layout == WM_PACKED_BGR) {  // one plane of rows x 3 cols bytes, pitch ld
+        if (im->dtype != WM_U8 || im->channels != 3) return fail(ctx, WM_ERR_ARG, "a packed RGB / BGR image has dtype WM_U8 and 3 channels");
+        g->L = im->rows; g->P = 3 * im->cols;
+        g->ld = im->ld > 0 ? im->ld : g->P;
+        if (g->L < 1 || g->P < 1 || g->ld < g->P) return fail(ctx, WM_ERR_ARG, "packed image: ld (bytes) smaller than 3 * cols");
+        g->ch = 1; g->ps = g->L * g->ld; g->es = 1;
+        return WM_OK;
+    }
     if (im->layout != WM_COL_MAJOR && im->layout != WM_ROW_MAJOR) return fail(ctx, WM_ERR_ARG, "bad layout");
     if (im->dtype != WM_F32 && im->dtype != WM_U8) return fail(ctx, WM_ERR_ARG, "bad dtype");
     const bool tr = im->layout == WM_COL_MAJOR;
@@ -1179,7 +1243,9 @@ int wm_embed_verify_host_batch(wm_ctx* ctx, int slot, const wm_image* in, const 
                                int64_t base_stride, int64_t out_stride, int batch, int mask, float* a_host, float* corr_host, int* status_host)
 {
     if (!ctx || !out) return WM_ERR_ARG;
-    if ((out->channels > 1) || out->dtype != (in ? in->dtype : out->dtype))
+    // a packed RGB / BGR output is verified through its gray, like the reference's detection on the gray of the saved image
+    const bool packed_out = out->layout == WM_PACKED_RGB || out->layout == WM_PACKED_BGR;
+    if (!packed_out && ((out->channels > 1) || out->dtype != (in ? in->dtype : out->dtype)))
         return fail(ctx, WM_ERR_ARG, "embed + verify needs a gray output of the input's dtype (detectWatermark takes the gray image)");
     int rc = wm_embed_host_batch(ctx, slot, in, base, out, in_stride, base_stride, out_stride, batch, mask, a_host, status_host);
     if (rc) return rc;
@@ -1291,6 +1357,7 @@ int wm_debug_set_coeffs(wm_ctx* ctx, const float* c)
 int wm_debug_detect_planes(wm_ctx* ctx, const wm_image* img, int mask, float* u_dev, float* eu_dev, float* corr_host)
 {
     if (!ctx || !img || !u_dev || !eu_dev) return WM_ERR_ARG;
+    if (img->layout == WM_PACKED_RGB || img->layout == WM_PACKED_BGR) return fail(ctx, WM_ERR_ARG, "detector planes: gray f32 images only, not packed RGB / BGR");
     if (img->dtype != WM_F32 || (mask == WM_MASK_NVF && ctx->p != 3)) return fail(ctx, WM_ERR_ARG, "detector planes: f32 images, 3x3 masks");
     Slot& s = ctx->slots[0];
     if (!s.queue.empty()) { const int r = finish_slot(ctx, s); if (r < 0) return r; }

@@ -32,6 +32,16 @@ void launch_apply_ts(int dtype, int mask, bool tr, bool narrow, dim3 grid, cudaS
 #undef WM_TS
 }
 
+void launch_apply_packed(int mask, bool tma, dim3 grid, cudaStream_t st, const CUtensorMap& tmI, const CUtensorMap& tmW, const EmbedArgs& a)
+{
+#define WM_PK(TMA)                                                                                                                 \
+    if (mask == 2) WM_LAUNCH((k_apply<float, uint8_t, 2, false, TMA, false, true>), embed_smem(TMA, false), tmI, tmW, a);          \
+    else if (mask == WM_MASK_ME) WM_LAUNCH((k_apply<float, uint8_t, 0, false, TMA, false, true>), embed_smem(TMA, false), tmI, tmW, a); \
+    else WM_LAUNCH((k_apply<float, uint8_t, 1, false, TMA, false, true>), embed_smem(TMA, false), tmI, tmW, a);
+    if (tma) { WM_PK(true) } else { WM_PK(false) }
+#undef WM_PK
+}
+
 void launch_apply(int in_dtype, int out_dtype, int mask, bool tr, bool tma, dim3 grid, cudaStream_t st, const CUtensorMap& tmI,
                   const CUtensorMap& tmW, const EmbedArgs& a)
 {
