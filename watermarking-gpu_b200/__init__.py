@@ -20,7 +20,8 @@ LIB_PATH = os.path.join(_HERE, "libwm_b200.so")
 ME, NVF = 0, 1                      # Watermark.hpp:10-14
 COL_MAJOR, ROW_MAJOR = 0, 1
 PACKED_RGB, PACKED_BGR = 2, 3       # interleaved 8-bit colour (rows, cols, 3), row pitch in bytes
-PACKED = (PACKED_RGB, PACKED_BGR)
+PACKED_RGBA, PACKED_BGRA = 4, 5     # the same with a fourth byte per pixel (rows, cols, 4), copied through by the embed
+PACKED_BYTES = {PACKED_RGB: 3, PACKED_BGR: 3, PACKED_RGBA: 4, PACKED_BGRA: 4}  # bytes per pixel of each packed layout
 F32, U8 = 0, 1
 OK, SINGULAR, ZERO_MASK = 0, 1, 2
 OPT_FP16_PRODUCTS, OPT_KERNEL_TIMING, OPT_USE_TMA, OPT_SERIAL_SLOTS, OPT_CUDA_GRAPHS, OPT_MMA_ACCUM, OPT_SPLIT_COST = 1, 2, 3, 4, 5, 6, 7
@@ -159,21 +160,21 @@ def _dtype_code(a):
 class DeviceArray:
     """A device buffer holding an image (rows, cols[, 3]) in a given layout; owned via the C ABI.
 
-    Planar layouts hold (rows, cols) or (3, rows, cols) images, `ld` in elements.  PACKED_RGB / PACKED_BGR hold a (rows, cols, 3)
-    uint8 image as interleaved rows of 3 * cols bytes with a row pitch of `ld` bytes (0 = dense)."""
+    Planar layouts hold (rows, cols) or (3, rows, cols) images, `ld` in elements.  The packed layouts hold a (rows, cols, n) uint8
+    image, n = PACKED_BYTES[layout], as interleaved rows of n * cols bytes with a row pitch of `ld` bytes (0 = dense)."""
 
     def __init__(self, wm, rows, cols, layout=COL_MAJOR, dtype=F32, channels=1, ld=0):
-        if layout in PACKED:
-            dtype, channels = U8, 3
+        if layout in PACKED_BYTES:
+            dtype, channels = U8, PACKED_BYTES[layout]
         self.wm, self.rows, self.cols, self.layout, self.dtype, self.channels = wm, rows, cols, layout, dtype, channels
         P = rows if layout == COL_MAJOR else cols
         Ln = cols if layout == COL_MAJOR else rows
-        if layout in PACKED:
-            P = 3 * cols  # bytes of a row
+        if layout in PACKED_BYTES:
+            P = channels * cols  # bytes of a row
         self.ld = ld if ld else P
         self.P, self.L = P, Ln
         self.itemsize = 4 if dtype == F32 else 1
-        planes = 1 if layout in PACKED else self.channels
+        planes = 1 if layout in PACKED_BYTES else self.channels
         self.nbytes = planes * Ln * self.ld * self.itemsize
         self.ptr = lib().wm_dev_alloc(wm._h, self.nbytes)
         if not self.ptr:
@@ -181,10 +182,11 @@ class DeviceArray:
 
     @classmethod
     def from_numpy(cls, wm, img, layout=COL_MAJOR, ld=0):
-        """img: (rows, cols) or (3, rows, cols) numpy array in logical (row, col) indexing; (rows, cols, 3) uint8 for a packed layout."""
+        """img: (rows, cols) or (3, rows, cols) numpy array in logical (row, col) indexing; (rows, cols, PACKED_BYTES[layout]) uint8
+        for a packed layout."""
         img = np.asarray(img)
-        if layout in PACKED:
-            d = cls(wm, img.shape[0], img.shape[1], layout, U8, 3, ld)
+        if layout in PACKED_BYTES:
+            d = cls(wm, img.shape[0], img.shape[1], layout, ld=ld)
             d.upload(img)
             return d
         ch = 1 if img.ndim == 2 else img.shape[0]
@@ -194,7 +196,7 @@ class DeviceArray:
         return d
 
     def _to_mem(self, img):
-        if self.layout in PACKED:
+        if self.layout in PACKED_BYTES:
             buf = np.zeros((self.L, self.ld), np.uint8)
             buf[:, :self.P] = img.reshape(self.rows, self.P)
             return buf
@@ -211,12 +213,12 @@ class DeviceArray:
             raise WatermarkError(rc, "upload failed")
 
     def numpy(self):
-        if self.layout in PACKED:
+        if self.layout in PACKED_BYTES:
             buf = np.empty((self.L, self.ld), np.uint8)
             rc = lib().wm_dev_download(self.wm._h, buf.ctypes.data, self.ptr, buf.nbytes)
             if rc:
                 raise WatermarkError(rc, "download failed")
-            return np.ascontiguousarray(buf[:, :self.P].reshape(self.rows, self.cols, 3))
+            return np.ascontiguousarray(buf[:, :self.P].reshape(self.rows, self.cols, self.channels))
         buf = np.empty((self.channels, self.L, self.ld), _NP_DT[self.dtype])
         rc = lib().wm_dev_download(self.wm._h, buf.ctypes.data, self.ptr, buf.nbytes)
         if rc:
@@ -336,10 +338,11 @@ class Watermark:
 
     # -- hot path, host (numpy) arrays: H2D + compute + D2H inside the call -------------------------
     def _host_desc(self, arr, layout):
-        if layout in PACKED:  # (rows, cols, 3) uint8, pixels and channels contiguous; rows may be pitched (a view of a wider buffer)
-            if arr.dtype != np.uint8 or arr.ndim != 3 or arr.shape[2] != 3 or arr.strides[1:] != (3, 1):
-                raise TypeError("a packed RGB / BGR host image is a (rows, cols, 3) uint8 array with contiguous pixels")
-            return image_desc(arr.ctypes.data, self.rows, self.cols, layout, U8, arr.strides[0], 3, 0)
+        if layout in PACKED_BYTES:  # (rows, cols, n) uint8, pixels and channels contiguous; rows may be pitched (a view of a wider buffer)
+            n = PACKED_BYTES[layout]
+            if arr.dtype != np.uint8 or arr.ndim != 3 or arr.shape[2] != n or arr.strides[1:] != (n, 1):
+                raise TypeError("a packed host image of this layout is a (rows, cols, %d) uint8 array with contiguous pixels" % n)
+            return image_desc(arr.ctypes.data, self.rows, self.cols, layout, U8, arr.strides[0], n, 0)
         ch = 1 if arr.ndim == 2 else arr.shape[0]
         return image_desc(arr.ctypes.data, self.rows, self.cols, layout, _dtype_code(arr), 0, ch, 0)
 

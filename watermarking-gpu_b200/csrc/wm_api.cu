@@ -121,30 +121,54 @@ int fail(wm_ctx* c, int code, const std::string& msg)
             return fail(ctx, WM_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_));        \
     } while (0)
 
+// The packed 8-bit layouts: bytes per pixel (0 = not a packed layout) and whether B comes before R.  Every other place reads these two
+// facts from here, so a packed layout is described once.
+struct PackedFmt { int bytes; bool bgr; const char* name; };
+PackedFmt packed_fmt(int layout)
+{
+    switch (layout) {
+    case WM_PACKED_RGB: return {3, false, "RGB"};
+    case WM_PACKED_BGR: return {3, true, "BGR"};
+    case WM_PACKED_RGBA: return {4, false, "RGBA"};
+    case WM_PACKED_BGRA: return {4, true, "BGRA"};
+    default: return {0, false, ""};
+    }
+}
+// dtype, channels and row pitch of a packed image; *ld receives the pitch in bytes (0 = dense)
+int check_packed(wm_ctx* ctx, const wm_image* im, const PackedFmt& f, long long* ld)
+{
+    const std::string what = std::string("a packed ") + f.name + " image";
+    if (im->dtype != WM_U8 || im->channels != f.bytes)
+        return fail(ctx, WM_ERR_ARG, what + " has dtype WM_U8 and " + std::to_string(f.bytes) + " channels");
+    *ld = im->ld > 0 ? im->ld : (long long)f.bytes * im->cols;
+    if (*ld < (long long)f.bytes * im->cols) return fail(ctx, WM_ERR_ARG, what + ": ld (bytes) smaller than " + std::to_string(f.bytes) + " * cols");
+    return WM_OK;
+}
+
 struct View {  // an image reduced to lines x pixels
     void* ptr; int L, P; long long ld, pstride; int channels; int dtype; bool transposed;
-    bool packed, bgr;  // WM_PACKED_RGB / WM_PACKED_BGR: L = rows, P = cols (pixels), ld in bytes (>= 3 P), channels 3, dtype u8
+    int pxb; bool bgr;  // packed 8-bit images: bytes per pixel (3 or 4; 0 = not packed), B before R; L = rows, P = cols, ld in bytes, dtype u8
 };
 
-// allow_packed: the caller handles packed 8-bit RGB / BGR images (the embed and detect entry points)
+// allow_packed: the caller handles packed 8-bit images (the embed and detect entry points)
 int make_view(wm_ctx* ctx, const wm_image* im, View* v, bool allow_rgb, bool allow_packed = false)
 {
     if (!im || !im->data) return fail(ctx, WM_ERR_ARG, "null image");
     if (im->rows != ctx->rows || im->cols != ctx->cols)
         return fail(ctx, WM_ERR_DIMS, "image dims " + std::to_string(im->rows) + "x" + std::to_string(im->cols) +
                                           " != watermark dims " + std::to_string(ctx->rows) + "x" + std::to_string(ctx->cols));
-    v->packed = im->layout == WM_PACKED_RGB || im->layout == WM_PACKED_BGR;
-    v->bgr = im->layout == WM_PACKED_BGR;
-    if (v->packed) {
-        if (!allow_packed) return fail(ctx, WM_ERR_ARG, "packed RGB / BGR images are taken by the wm_embed* and wm_detect* entry points only");
-        if (im->dtype != WM_U8 || im->channels != 3) return fail(ctx, WM_ERR_ARG, "a packed RGB / BGR image has dtype WM_U8 and 3 channels");
+    const PackedFmt f = packed_fmt(im->layout);
+    v->pxb = f.bytes;
+    v->bgr = f.bgr;
+    if (v->pxb) {
+        if (!allow_packed) return fail(ctx, WM_ERR_ARG, std::string("packed ") + f.name + " images are taken by the wm_embed* and wm_detect* entry points only");
+        int rc;
+        if ((rc = check_packed(ctx, im, f, &v->ld))) return rc;
         v->transposed = false;
         v->L = (int)im->rows;
         v->P = (int)im->cols;
-        v->ld = im->ld > 0 ? im->ld : 3LL * v->P;
-        if (v->ld < 3LL * v->P) return fail(ctx, WM_ERR_ARG, "packed image: ld (bytes) smaller than 3 * cols");
         v->pstride = 0;
-        v->channels = 3;
+        v->channels = f.bytes;
         v->dtype = WM_U8;
         v->ptr = im->data;
         return WM_OK;
@@ -170,6 +194,12 @@ bool vec_ok(const void* p, long long ld, long long bstride, long long pstride, i
     const uintptr_t al = dtype == WM_F32 ? 16 : 4;
     return ((uintptr_t)p % al == 0) && (ld % 4 == 0) && (bstride % 4 == 0) && (pstride % 4 == 0);
 }
+// alignment level of a packed image's rows (launch_packed_gray): 2 = pointer, ld and batch stride are multiples of 16 bytes, 1 = of 4 bytes, 0
+int packed_align(const void* p, long long ld, long long bstride)
+{
+    auto al = [&](long long m) { return (uintptr_t)p % (uintptr_t)m == 0 && ld % m == 0 && bstride % m == 0; };
+    return al(16) ? 2 : al(4) ? 1 : 0;
+}
 
 
 // batch stride conventions (include/wm_b200.h): 0 means dense (plane_stride * channels, i.e. L * ld * channels for dense planes); a stride
@@ -178,8 +208,8 @@ bool vec_ok(const void* p, long long ld, long long bstride, long long pstride, i
 int resolve_stride(wm_ctx* ctx, const View& v, int batch, int64_t* stride, const char* what)
 {
     // elements (bytes for packed images: one interleaved plane) spanned by one image
-    const long long one = v.packed ? (long long)v.L * v.ld : v.pstride * (v.channels - 1) + (long long)v.L * v.ld;
-    if (*stride == 0) *stride = v.packed ? one : v.pstride * v.channels;
+    const long long one = v.pxb ? (long long)v.L * v.ld : v.pstride * (v.channels - 1) + (long long)v.L * v.ld;
+    if (*stride == 0) *stride = v.pxb ? one : v.pstride * v.channels;
     if (batch > 1 && *stride < one) return fail(ctx, WM_ERR_ARG, std::string(what) + " batch stride smaller than one image");
     return WM_OK;
 }
@@ -188,7 +218,7 @@ void byte_range(const View& v, int64_t stride, int batch, uintptr_t* lo, uintptr
 {
     const long long es = v.dtype == WM_F32 ? 4 : 1;
     const long long last = (long long)(batch - 1) * stride + (long long)(v.L - 1) * v.ld +
-                           (v.packed ? 3LL * v.P : v.pstride * (v.channels - 1) + v.P);
+                           (v.pxb ? (long long)v.pxb * v.P : v.pstride * (v.channels - 1) + v.P);
     *lo = (uintptr_t)v.ptr;
     *hi = (uintptr_t)v.ptr + (uintptr_t)(last * es);
 }
@@ -523,8 +553,8 @@ int enqueue_nvf_planes(wm_ctx* ctx, Slot& s, const View& v, long long bstride, i
     return WM_OK;
 }
 
-// Packed RGB / BGR batch: its gray goes into the slot's dense f32 planes, and *v / *stride become that gray batch, so the op runs on it
-// exactly as on a caller's dense f32 gray batch (same tiles, launch plan and partial sums: the scalars of the composed path).
+// Packed batch: its gray goes into the slot's dense f32 planes, and *v / *stride become that gray batch, so the op runs on it exactly as
+// on a caller's dense f32 gray batch (same tiles, launch plan and partial sums: the scalars of the composed path).
 int enqueue_packed_gray(wm_ctx* ctx, Slot& s, View* v, int64_t* stride, int batch)
 {
     const size_t plane = (size_t)v->L * v->P, need = plane * sizeof(float) * batch;
@@ -535,12 +565,13 @@ int enqueue_packed_gray(wm_ctx* ctx, Slot& s, View* v, int64_t* stride, int batc
         const int rc = ensure_stage(ctx, &s.gray, &s.gray_cap, need);
         if (rc) return rc;
     }
-    launch_packed_gray((const uint8_t*)v->ptr, v->ld, *stride, batch, v->bgr, (float*)s.gray, v->L, v->P, vec_ok(v->ptr, v->ld, *stride, 0, WM_U8),
+    launch_packed_gray((const uint8_t*)v->ptr, v->ld, *stride, batch, v->pxb, v->bgr, (float*)s.gray, v->L, v->P, packed_align(v->ptr, v->ld, *stride),
                        8 * ctx->sms, s.stream);
     ctx->launches++;
     CU(cudaGetLastError());
     v->ptr = s.gray; v->ld = v->P; v->pstride = (long long)plane; v->channels = 1; v->dtype = WM_F32;
-    v->packed = v->bgr = false;
+    v->pxb = 0;
+    v->bgr = false;
     *stride = (int64_t)plane;
     return WM_OK;
 }
@@ -578,12 +609,12 @@ int do_embed(wm_ctx* ctx, int slot, const wm_image* in, const wm_image* base, wm
     if ((rc = make_view(ctx, in, &vi, false, true))) return rc;
     if ((rc = make_view(ctx, base ? base : in, &vb, true, true))) return rc;
     if ((rc = make_view(ctx, out, &vo, true, true))) return rc;
-    const bool packed = vi.packed;
-    if (packed || vb.packed || vo.packed) {
-        if (!packed) return fail(ctx, WM_ERR_ARG, "a packed RGB / BGR base or output needs the same packed image as the input");
-        if (!vb.packed || vb.ptr != vi.ptr || vb.ld != vi.ld || vb.bgr != vi.bgr)
-            return fail(ctx, WM_ERR_ARG, "with a packed RGB / BGR input, base must be NULL or the same image (pointer, layout, ld)");
-        if (!vo.packed || vo.bgr != vi.bgr) return fail(ctx, WM_ERR_ARG, "with a packed RGB / BGR input, out must be a packed image of the same layout");
+    const int pxb = vi.pxb;  // packed input: bytes per pixel
+    if (pxb || vb.pxb || vo.pxb) {
+        if (!pxb) return fail(ctx, WM_ERR_ARG, "a packed base or output needs the same packed image as the input");
+        if (vb.pxb != pxb || vb.ptr != vi.ptr || vb.ld != vi.ld || vb.bgr != vi.bgr)
+            return fail(ctx, WM_ERR_ARG, "with a packed input, base must be NULL or the same image (pointer, layout, ld)");
+        if (vo.pxb != pxb || vo.bgr != vi.bgr) return fail(ctx, WM_ERR_ARG, "with a packed input, out must be a packed image of the same layout");
         if (!base) base_stride = in_stride;  // NULL base: the input batch itself
     }
     if (vb.transposed != vi.transposed || vo.transposed != vi.transposed) return fail(ctx, WM_ERR_ARG, "in/base/out layouts differ");
@@ -592,7 +623,7 @@ int do_embed(wm_ctx* ctx, int slot, const wm_image* in, const wm_image* base, wm
     if ((rc = resolve_stride(ctx, vi, batch, &in_stride, "in"))) return rc;
     if ((rc = resolve_stride(ctx, vb, batch, &base_stride, "base"))) return rc;
     if ((rc = resolve_stride(ctx, vo, batch, &out_stride, "out"))) return rc;
-    if (packed && batch > 1 && base_stride != in_stride) return fail(ctx, WM_ERR_ARG, "with a packed RGB / BGR input, base must be the same batch (stride)");
+    if (pxb && batch > 1 && base_stride != in_stride) return fail(ctx, WM_ERR_ARG, "with a packed input, base must be the same batch (stride)");
     {
         uintptr_t ilo, ihi, olo, ohi;
         byte_range(vi, in_stride, batch, &ilo, &ihi);
@@ -601,7 +632,7 @@ int do_embed(wm_ctx* ctx, int slot, const wm_image* in, const wm_image* base, wm
     }
     CU(cudaSetDevice(ctx->device));
     Slot& s = ctx->slots[slot];
-    if (packed && (rc = enqueue_packed_gray(ctx, s, &vi, &in_stride, batch))) return rc;
+    if (pxb && (rc = enqueue_packed_gray(ctx, s, &vi, &in_stride, batch))) return rc;
     const Geo g = geo(vi.L, vi.P);
     const bool narrow = ctx->opt_narrow_u8 && vi.dtype == WM_U8 && tma_ok(ctx, vi, in_stride, batch);
     const Plan pl = plan(ctx, g, batch, vi.dtype, narrow);
@@ -631,8 +662,9 @@ int do_embed(wm_ctx* ctx, int slot, const wm_image* in, const wm_image* base, wm
     ea.channels = vb.channels;
     ea.same_base = (vb.ptr == vi.ptr && vb.ld == vi.ld && base_stride == in_stride && vb.channels == 1);
     ea.dl = deliver_args(s, direct && batch == 1);
-    ea.base_vec_ok = vec_ok(vb.ptr, vb.ld, base_stride, vb.channels > 1 ? vb.pstride : 0, vb.dtype);
-    ea.out_vec_ok = vec_ok(vo.ptr, vo.ld, out_stride, vo.channels > 1 ? vo.pstride : 0, vo.dtype);
+    // packed base / out: alignment levels (16-byte, word or byte accesses), as k_packed_gray reads them
+    ea.base_vec_ok = pxb ? packed_align(vb.ptr, vb.ld, base_stride) : vec_ok(vb.ptr, vb.ld, base_stride, vb.channels > 1 ? vb.pstride : 0, vb.dtype);
+    ea.out_vec_ok = pxb ? packed_align(vo.ptr, vo.ld, out_stride) : vec_ok(vo.ptr, vo.ld, out_stride, vo.channels > 1 ? vo.pstride : 0, vo.dtype);
     CUtensorMap tmI, tmW;
     memset(&tmI, 0, sizeof tmI);
     memset(&tmW, 0, sizeof tmW);
@@ -664,7 +696,7 @@ int do_embed(wm_ctx* ctx, int slot, const wm_image* in, const wm_image* base, wm
             ea.b0 = sb.b0; ea.nblk_base = sb.base; ea.nblk_extra = sb.extra;
             const dim3 grid(sb.base + (sb.extra > 0 ? 1 : 0), sb.nb);
             if (ts) launch_apply_ts(vi.dtype, kmask, vi.transposed, narrow, grid, s.stream, tmI, tmW, tmO, ea);
-            else if (packed) launch_apply_packed(kmask, tma, grid, s.stream, tmI, tmW, ea);
+            else if (pxb) launch_apply_packed(kmask, pxb, tma, grid, s.stream, tmI, tmW, ea);
             else launch_apply(vi.dtype, vo.dtype, kmask, vi.transposed, tma, grid, s.stream, tmI, tmW, ea);
         }
     }
@@ -686,7 +718,7 @@ int do_detect(wm_ctx* ctx, int slot, const wm_image* img, int64_t img_stride, in
     if ((rc = resolve_stride(ctx, v, batch, &img_stride, "image"))) return rc;
     CU(cudaSetDevice(ctx->device));
     Slot& s = ctx->slots[slot];
-    if (v.packed && (rc = enqueue_packed_gray(ctx, s, &v, &img_stride, batch))) return rc;
+    if (v.pxb && (rc = enqueue_packed_gray(ctx, s, &v, &img_stride, batch))) return rc;
     const Geo g = geo(v.L, v.P);
     bool tma = tma_ok(ctx, v, img_stride, batch);
     const bool narrow = ctx->opt_narrow_u8 && v.dtype == WM_U8 && tma && !dbg_u;
@@ -1135,11 +1167,13 @@ struct HostGeo { int64_t L, P, ld, ps; int ch; size_t es; };
 static int host_geo(wm_ctx* ctx, const wm_image* im, HostGeo* g)
 {
     if (!im || !im->data) return fail(ctx, WM_ERR_ARG, "null image");
-    if (im->layout == WM_PACKED_RGB || im->layout == WM_PACKED_BGR) {  // one plane of rows x 3 cols bytes, pitch ld
-        if (im->dtype != WM_U8 || im->channels != 3) return fail(ctx, WM_ERR_ARG, "a packed RGB / BGR image has dtype WM_U8 and 3 channels");
-        g->L = im->rows; g->P = 3 * im->cols;
-        g->ld = im->ld > 0 ? im->ld : g->P;
-        if (g->L < 1 || g->P < 1 || g->ld < g->P) return fail(ctx, WM_ERR_ARG, "packed image: ld (bytes) smaller than 3 * cols");
+    const PackedFmt f = packed_fmt(im->layout);
+    if (f.bytes) {  // one plane of rows x (bytes per pixel * cols) bytes, pitch ld
+        long long ld;
+        const int rc = check_packed(ctx, im, f, &ld);
+        if (rc) return rc;
+        g->L = im->rows; g->P = f.bytes * im->cols; g->ld = ld;
+        if (g->L < 1 || g->P < 1) return fail(ctx, WM_ERR_ARG, "packed image: rows and cols must be positive");
         g->ch = 1; g->ps = g->L * g->ld; g->es = 1;
         return WM_OK;
     }
@@ -1243,8 +1277,8 @@ int wm_embed_verify_host_batch(wm_ctx* ctx, int slot, const wm_image* in, const 
                                int64_t base_stride, int64_t out_stride, int batch, int mask, float* a_host, float* corr_host, int* status_host)
 {
     if (!ctx || !out) return WM_ERR_ARG;
-    // a packed RGB / BGR output is verified through its gray, like the reference's detection on the gray of the saved image
-    const bool packed_out = out->layout == WM_PACKED_RGB || out->layout == WM_PACKED_BGR;
+    // a packed output is verified through its gray, like the reference's detection on the gray of the saved image
+    const bool packed_out = packed_fmt(out->layout).bytes != 0;
     if (!packed_out && ((out->channels > 1) || out->dtype != (in ? in->dtype : out->dtype)))
         return fail(ctx, WM_ERR_ARG, "embed + verify needs a gray output of the input's dtype (detectWatermark takes the gray image)");
     int rc = wm_embed_host_batch(ctx, slot, in, base, out, in_stride, base_stride, out_stride, batch, mask, a_host, status_host);
@@ -1357,7 +1391,7 @@ int wm_debug_set_coeffs(wm_ctx* ctx, const float* c)
 int wm_debug_detect_planes(wm_ctx* ctx, const wm_image* img, int mask, float* u_dev, float* eu_dev, float* corr_host)
 {
     if (!ctx || !img || !u_dev || !eu_dev) return WM_ERR_ARG;
-    if (img->layout == WM_PACKED_RGB || img->layout == WM_PACKED_BGR) return fail(ctx, WM_ERR_ARG, "detector planes: gray f32 images only, not packed RGB / BGR");
+    if (packed_fmt(img->layout).bytes) return fail(ctx, WM_ERR_ARG, "detector planes: gray f32 images only, not packed images");
     if (img->dtype != WM_F32 || (mask == WM_MASK_NVF && ctx->p != 3)) return fail(ctx, WM_ERR_ARG, "detector planes: f32 images, 3x3 masks");
     Slot& s = ctx->slots[0];
     if (!s.queue.empty()) { const int r = finish_slot(ctx, s); if (r < 0) return r; }

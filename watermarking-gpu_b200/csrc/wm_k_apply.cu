@@ -32,13 +32,15 @@ void launch_apply_ts(int dtype, int mask, bool tr, bool narrow, dim3 grid, cudaS
 #undef WM_TS
 }
 
-void launch_apply_packed(int mask, bool tma, dim3 grid, cudaStream_t st, const CUtensorMap& tmI, const CUtensorMap& tmW, const EmbedArgs& a)
+void launch_apply_packed(int mask, int pixel_bytes, bool tma, dim3 grid, cudaStream_t st, const CUtensorMap& tmI, const CUtensorMap& tmW,
+                         const EmbedArgs& a)
 {
-#define WM_PK(TMA)                                                                                                                 \
-    if (mask == 2) WM_LAUNCH((k_apply<float, uint8_t, 2, false, TMA, false, true>), embed_smem(TMA, false), tmI, tmW, a);          \
-    else if (mask == WM_MASK_ME) WM_LAUNCH((k_apply<float, uint8_t, 0, false, TMA, false, true>), embed_smem(TMA, false), tmI, tmW, a); \
-    else WM_LAUNCH((k_apply<float, uint8_t, 1, false, TMA, false, true>), embed_smem(TMA, false), tmI, tmW, a);
-    if (tma) { WM_PK(true) } else { WM_PK(false) }
+#define WM_PK(TMA, PB)                                                                                                                 \
+    if (mask == 2) WM_LAUNCH((k_apply<float, uint8_t, 2, false, TMA, false, PB>), embed_smem(TMA, false), tmI, tmW, a);               \
+    else if (mask == WM_MASK_ME) WM_LAUNCH((k_apply<float, uint8_t, 0, false, TMA, false, PB>), embed_smem(TMA, false), tmI, tmW, a);  \
+    else WM_LAUNCH((k_apply<float, uint8_t, 1, false, TMA, false, PB>), embed_smem(TMA, false), tmI, tmW, a);
+    if (pixel_bytes == 4) { if (tma) { WM_PK(true, 4) } else { WM_PK(false, 4) } }
+    else { if (tma) { WM_PK(true, 3) } else { WM_PK(false, 3) } }
 #undef WM_PK
 }
 

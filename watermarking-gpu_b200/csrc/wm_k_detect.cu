@@ -80,12 +80,17 @@ void launch_rgb2gray(const float* r, const float* g, const float* b, float* gray
     k_rgb2gray<<<blocks, 256, 0, st>>>(r, g, b, gray, ld_in, ld_out, L, P, wr, wg, wb);
 }
 
-void launch_packed_gray(const uint8_t* src, long long ld, long long bstride, int batch, bool bgr, float* gray, int L, int P, bool vec, int blocks,
-                        cudaStream_t st)
+void launch_packed_gray(const uint8_t* src, long long ld, long long bstride, int batch, int pixel_bytes, bool bgr, float* gray, int L, int P,
+                        int align, int blocks, cudaStream_t st)
 {
     const dim3 grid((unsigned)(blocks > batch ? blocks / batch : 1), (unsigned)batch);
-    if (bgr) k_packed_gray<true><<<grid, 256, 0, st>>>(src, ld, bstride, gray, L, P, vec);
-    else k_packed_gray<false><<<grid, 256, 0, st>>>(src, ld, bstride, gray, L, P, vec);
+    if (pixel_bytes == 4) {
+        if (bgr) k_packed_gray<4, true><<<grid, 256, 0, st>>>(src, ld, bstride, gray, L, P, align);
+        else k_packed_gray<4, false><<<grid, 256, 0, st>>>(src, ld, bstride, gray, L, P, align);
+    } else {
+        if (bgr) k_packed_gray<3, true><<<grid, 256, 0, st>>>(src, ld, bstride, gray, L, P, align);
+        else k_packed_gray<3, false><<<grid, 256, 0, st>>>(src, ld, bstride, gray, L, P, align);
+    }
 }
 
 void launch_transpose(const float* src, float* dst, int rows, int cols, cudaStream_t st)

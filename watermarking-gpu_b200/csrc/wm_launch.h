@@ -19,11 +19,14 @@ void launch_mask_from_errseq(float* plane, long long n, unsigned* scratch, cudaS
 void launch_transpose(const float* src, float* dst, int rows, int cols, cudaStream_t st);
 void launch_rgb2gray(const float* r, const float* g, const float* b, float* gray, long long ld_in, long long ld_out, int L, int P,
                      float wr, float wg, float wb, int blocks, cudaStream_t st);
-// packed 8-bit RGB / BGR batch (byte ld / stride) -> dense f32 gray planes [batch][L x P]
-void launch_packed_gray(const uint8_t* src, long long ld, long long bstride, int batch, bool bgr, float* gray, int L, int P, bool vec, int blocks,
-                        cudaStream_t st);
+// packed 8-bit batch of 3 (RGB / BGR) or 4 (RGBA / BGRA) bytes per pixel (byte ld / stride) -> dense f32 gray planes [batch][L x P];
+// align: 2 = src, ld and bstride are multiples of 16 bytes, 1 = of 4 bytes, 0 = neither
+void launch_packed_gray(const uint8_t* src, long long ld, long long bstride, int batch, int pixel_bytes, bool bgr, float* gray, int L, int P,
+                        int align, int blocks, cudaStream_t st);
 // apply kernel of a packed image: input = its gray (f32, dense), base / out = the packed image and the packed output
-void launch_apply_packed(int mask, bool tma, dim3 grid, cudaStream_t st, const CUtensorMap& tmI, const CUtensorMap& tmW, const EmbedArgs& a);
+// (a.base_vec_ok / a.out_vec_ok: their alignment levels, as for launch_packed_gray)
+void launch_apply_packed(int mask, int pixel_bytes, bool tma, dim3 grid, cudaStream_t st, const CUtensorMap& tmI, const CUtensorMap& tmW,
+                         const EmbedArgs& a);
 }  // namespace wm
 
 // dtype / mask codes shared with include/wm_b200.h
