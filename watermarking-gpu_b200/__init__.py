@@ -51,7 +51,7 @@ class wm_image(C.Structure):
 class wm_video_ctx(C.Structure):
     _fields_ = [("watermark", C.c_void_p), ("height", C.c_int32), ("width", C.c_int32),
                 ("watermark_interval", C.c_int32), ("linesize", C.c_int32), ("frame_stride", C.c_int64),
-                ("frames_on_device", C.c_int32), ("reserved", C.c_int32)]
+                ("frames_on_device", C.c_int32), ("layout", C.c_int32)]
 
 
 class WatermarkError(RuntimeError):
@@ -462,13 +462,17 @@ class Watermark:
 
 
 class VideoProcessingContext:
-    """videoprocessingcontext.hpp:13-29 minus the ffmpeg handles: frames come from memory."""
+    """videoprocessingcontext.hpp:13-29 minus the ffmpeg handles: frames come from memory.
 
-    def __init__(self, watermark, height, width, watermark_interval, linesize=0, frame_stride=0, frames_on_device=False):
+    layout 0 (Y planes) or a packed colour layout (PACKED_RGB / BGR / RGBA / BGRA: e.g. the BGR frames of cv2.VideoCapture); linesize is
+    the row pitch in bytes (default: dense rows of PACKED_BYTES[layout] * width bytes)."""
+
+    def __init__(self, watermark, height, width, watermark_interval, linesize=0, frame_stride=0, frames_on_device=False, layout=0):
         self.watermarkObj, self.height, self.width = watermark, height, width
         self.watermarkInterval = watermark_interval
-        self._c = wm_video_ctx(watermark._h, height, width, watermark_interval, linesize or width, frame_stride,
-                               int(frames_on_device), 0)
+        self.layout = layout
+        self._c = wm_video_ctx(watermark._h, height, width, watermark_interval, linesize or PACKED_BYTES.get(layout, 1) * width,
+                               frame_stride, int(frames_on_device), layout)
 
 
 def process_frames(ctx, mode, frames_ptr, out_ptr, first_index, n_frames, scalars):

@@ -57,8 +57,17 @@ def build(force=False, verbose=False):
 
 def build_facade_test(force=False):
     """C++ smoke/parity program over the Watermark façade (csrc/Watermark.hpp), linked against the .so."""
-    src = os.path.join(ROOT, "tests", "cpp", "test_facade.cpp")
-    exe = os.path.join(ROOT, "tests", "cpp", "test_facade")
+    return _build_cpp_test("test_facade", force)
+
+
+def build_video_packed_test(force=False):
+    """C++ program running processFramesInMemory (csrc/videoprocessingcontext.hpp) on packed BGR frames, linked against the .so."""
+    return _build_cpp_test("test_video_packed", force)
+
+
+def _build_cpp_test(name, force):
+    src = os.path.join(ROOT, "tests", "cpp", name + ".cpp")
+    exe = os.path.join(ROOT, "tests", "cpp", name)
     if not os.path.exists(src):
         return None
     deps = [src, os.path.join(CSRC, "Watermark.hpp"), os.path.join(CSRC, "videoprocessingcontext.hpp"), LIB]
@@ -89,4 +98,5 @@ def build_generator(force=False):
 if __name__ == "__main__":
     print(build(force="--force" in sys.argv, verbose="-v" in sys.argv))
     print(build_facade_test(force="--force" in sys.argv))
+    print(build_video_packed_test(force="--force" in sys.argv))
     print(build_generator(force="--force" in sys.argv))

@@ -101,10 +101,13 @@ inline float detectFrameWatermark(const VideoProcessingContext& data, int& frame
 // frames per launch sequence with copies and kernels overlapped, on ONE GPU (one Watermark object) or SEVERAL (one object per
 // device: contiguous chunks of the global frame index, one host thread per device, the gate of main.cpp:346,395 on the global
 // index).  `out` receives the Y planes without row padding (gated-off frames copied through), as embedWatermarkFrame writes them.
+// layout 0 (Y planes) or a packed colour layout (WM_PACKED_RGB / BGR / RGBA / BGRA, e.g. the BGR frames of cv2.VideoCapture): `linesize`
+// is then the row pitch in bytes and `out` receives dense height x (bytes per pixel * width) frames (wm_video_ctx in wm_b200.h).
 inline int64_t processFramesInMemory(const std::vector<const Watermark*>& watermarkPerGpu, const int height, const int width,
                                      const int watermarkInterval, const int linesize, const int mode, const uint8_t* frames,
-                                     uint8_t* out, const int64_t firstIndex, const int64_t nFrames, float* scalars)
+                                     uint8_t* out, const int64_t firstIndex, const int64_t nFrames, float* scalars, const int layout = 0)
 {
+    const int64_t bpp = layout == WM_PACKED_RGB || layout == WM_PACKED_BGR ? 3 : layout == WM_PACKED_RGBA || layout == WM_PACKED_BGRA ? 4 : 1;
     const int ngpus = (int)watermarkPerGpu.size();
     if (ngpus < 1) throw std::runtime_error("processFramesInMemory: no Watermark object\n");
     if (mode == WM_VIDEO_EMBED_VERIFY && ngpus > 1) throw std::runtime_error("processFramesInMemory: EMBED_VERIFY runs on one GPU per call\n");
@@ -115,10 +118,10 @@ inline int64_t processFramesInMemory(const std::vector<const Watermark*>& waterm
     for (int g = 0; g < ngpus; g++) {
         int64_t first = 0, count = 0;
         wm_shard_frames(nFrames, g, ngpus, &first, &count);
-        ctx[(size_t)g] = wm_video_ctx{watermarkPerGpu[(size_t)g]->handle(), height, width, watermarkInterval, linesize, 0, 0, 0};
+        ctx[(size_t)g] = wm_video_ctx{watermarkPerGpu[(size_t)g]->handle(), height, width, watermarkInterval, linesize, 0, 0, layout};
         pc.push_back(&ctx[(size_t)g]);
         in.push_back(frames + first * (int64_t)height * linesize);
-        ou.push_back(out ? out + first * (int64_t)height * width : nullptr);
+        ou.push_back(out ? out + first * (int64_t)height * bpp * width : nullptr);
     }
     const int64_t n = ngpus == 1 ? wm_process_frames(pc[0], mode, in[0], ou[0], firstIndex, nFrames, scalars)
                                  : wm_process_frames_multi(pc.data(), ngpus, mode, in.data(), out ? ou.data() : nullptr, firstIndex, nFrames, scalars);

@@ -553,11 +553,9 @@ int enqueue_nvf_planes(wm_ctx* ctx, Slot& s, const View& v, long long bstride, i
     return WM_OK;
 }
 
-// Packed batch: its gray goes into the slot's dense f32 planes, and *v / *stride become that gray batch, so the op runs on it exactly as
-// on a caller's dense f32 gray batch (same tiles, launch plan and partial sums: the scalars of the composed path).
-int enqueue_packed_gray(wm_ctx* ctx, Slot& s, View* v, int64_t* stride, int batch)
+// the slot's f32 gray planes hold at least `need` bytes
+int reserve_gray(wm_ctx* ctx, Slot& s, size_t need)
 {
-    const size_t plane = (size_t)v->L * v->P, need = plane * sizeof(float) * batch;
     if (need > s.gray_cap) {  // queued work and captured graphs may still read the old planes
         if (!s.queue.empty()) { const int r = finish_slot(ctx, s); if (r < 0) return r; }
         CU(cudaStreamSynchronize(s.stream));
@@ -565,6 +563,15 @@ int enqueue_packed_gray(wm_ctx* ctx, Slot& s, View* v, int64_t* stride, int batc
         const int rc = ensure_stage(ctx, &s.gray, &s.gray_cap, need);
         if (rc) return rc;
     }
+    return WM_OK;
+}
+// Packed batch: its gray goes into the slot's dense f32 planes, and *v / *stride become that gray batch, so the op runs on it exactly as
+// on a caller's dense f32 gray batch (same tiles, launch plan and partial sums: the scalars of the composed path).
+int enqueue_packed_gray(wm_ctx* ctx, Slot& s, View* v, int64_t* stride, int batch)
+{
+    const size_t plane = (size_t)v->L * v->P;
+    const int rc = reserve_gray(ctx, s, plane * sizeof(float) * batch);
+    if (rc) return rc;
     launch_packed_gray((const uint8_t*)v->ptr, v->ld, *stride, batch, v->pxb, v->bgr, (float*)s.gray, v->L, v->P, packed_align(v->ptr, v->ld, *stride),
                        8 * ctx->sms, s.stream);
     ctx->launches++;
@@ -1464,11 +1471,16 @@ int64_t wm_process_frames(const wm_video_ctx* v, int mode, const uint8_t* frames
     if (v->height != ctx->rows || v->width != ctx->cols) return fail(ctx, WM_ERR_DIMS, "frame dims != watermark dims");
     if (v->watermark_interval < 1) return fail(ctx, WM_ERR_ARG, "watermark_interval must be >= 1");
     if (embed_mode && !out) return fail(ctx, WM_ERR_ARG, "embed needs an output buffer");
+    // Y planes (layout 0 or WM_ROW_MAJOR) have one byte per pixel; packed colour frames packed_fmt's bytes per pixel
+    const PackedFmt pf = packed_fmt(v->layout);
+    if (v->layout != 0 && v->layout != WM_ROW_MAJOR && !pf.bytes)
+        return fail(ctx, WM_ERR_ARG, "bad frame layout " + std::to_string(v->layout) + " (0 / WM_ROW_MAJOR: Y planes, or a WM_PACKED_* layout)");
     const int64_t H = v->height, Wd = v->width;
-    const int64_t linesize = v->linesize > 0 ? v->linesize : Wd;
-    if (linesize < Wd) return fail(ctx, WM_ERR_ARG, "linesize < width");
+    const int64_t rowb = (pf.bytes ? pf.bytes : 1) * Wd;  // bytes of a frame row without padding
+    const int64_t linesize = v->linesize > 0 ? v->linesize : rowb;
+    if (linesize < rowb) return fail(ctx, WM_ERR_ARG, pf.bytes ? "linesize < bytes per pixel * width" : "linesize < width");
     const int64_t fstride = v->frame_stride > 0 ? v->frame_stride : H * linesize;
-    const int64_t ostride = H * Wd;
+    const int64_t ostride = H * rowb;
     CU(cudaSetDevice(ctx->device));
     int rc;
     for (int i = 0; i < NSLOTS; i++)
@@ -1485,17 +1497,24 @@ int64_t wm_process_frames(const wm_video_ctx* v, int mode, const uint8_t* frames
     for (int64_t i = 0; i < n_frames; i++) {
         if ((first_index + i) % K == 0) continue;
         if (embed_mode)
-            CU(cudaMemcpy2DAsync(out + i * ostride, Wd, frames + i * fstride, linesize, Wd, H, through, ctx->slots[i % NSLOTS].stream));
+            CU(cudaMemcpy2DAsync(out + i * ostride, rowb, frames + i * fstride, linesize, rowb, H, through, ctx->slots[i % NSLOTS].stream));
     }
     // gated frames: equally spaced in memory, so a run of them is ONE batched launch sequence (image index in
     // blockIdx.y); runs go round-robin over the slots so copies, kernels and the per-frame solves of different runs overlap
-    const int64_t fbytes = H * Wd;
+    const int64_t fbytes = H * rowb;
     // frames per run: big enough to amortise a launch's ramp and second-stage tail, small enough that several runs are in
     // flight on different slots (round 1, 4K u8: 4 / 7 / 10 / 19 / 37 frames per run gave 17.1k / 18.2k / 19.0k / 18.5k / 18.2k frames/s; with the
-    // round-2 kernels 7 / 9 / 11 / 13 / 16 / 24 / 32 frames per run give 25.2k / 25.2k / 25.5k / 25.6k / 25.8k / 25.8k / 25.8k: WM_OPT_RUN_MB = 136)
+    // round-2 kernels 7 / 9 / 11 / 13 / 16 / 24 / 32 frames per run give 25.2k / 25.2k / 25.5k / 25.6k / 25.8k / 25.8k / 25.8k: WM_OPT_RUN_MB = 136).
+    // Packed frames count their packed bytes only, not the 4 B/px of gray planes a run also fills: EMBED_VERIFY on a B200 at 1080p / 4K,
+    // BGR / BGRA, gave 3-6 % more frames/s than counting packed + gray bytes (22 vs 9 frames per run at 1080p BGR, 5 vs 2 at 4K BGR)
     int64_t B = v->frames_on_device ? std::max<int64_t>(1, std::min<int64_t>(32, ((int64_t)ctx->opt_run_mb << 20) / fbytes)) : ctx->opt_host_run;
     // even runs (37 frames at 7 per run: 7,6,6,6,6,6 rather than 7,7,7,7,7,2)
     const int64_t nruns = ngated > 0 ? (ngated + B - 1) / B : 0;
+    // packed frames: each slot that takes a run computes its gray into its own f32 planes.  They are sized once for the longest run these
+    // options allow, so calls whose even runs differ by a frame (other frame counts, first indices) do not regrow them with a stream sync
+    if (pf.bytes)
+        for (int64_t r = 0; r < std::min<int64_t>(nruns, ctx->opt_serial ? 1 : NSLOTS); r++)
+            if ((rc = reserve_gray(ctx, ctx->slots[r], (size_t)(H * Wd) * sizeof(float) * (size_t)B))) return rc;
     const int64_t run_base = nruns ? ngated / nruns : 0, run_extra = nruns ? ngated % nruns : 0;
     B = run_base + (run_extra ? 1 : 0);
     for (int64_t g = 0, run = 0, nbr = 0; run < nruns; g += nbr, run++) {
@@ -1506,7 +1525,8 @@ int64_t wm_process_frames(const wm_video_ctx* v, int mode, const uint8_t* frames
         const int64_t i = i0 + g * K;
         wm_image fin;
         memset(&fin, 0, sizeof fin);
-        fin.rows = H; fin.cols = Wd; fin.channels = 1; fin.layout = WM_ROW_MAJOR; fin.dtype = WM_U8;
+        fin.rows = H; fin.cols = Wd; fin.dtype = WM_U8;
+        fin.channels = pf.bytes ? pf.bytes : 1; fin.layout = pf.bytes ? v->layout : WM_ROW_MAJOR;
         int64_t in_stride;
         if (v->frames_on_device) {
             fin.data = (void*)(frames + i * fstride); fin.ld = linesize;  // strided reads: no repack pass needed
@@ -1516,23 +1536,23 @@ int64_t wm_process_frames(const wm_video_ctx* v, int mode, const uint8_t* frames
             // padding is small and whose linesize keeps the rows 16-byte aligned goes up WITH its padding as one linear copy (a 2-D copy is
             // programmed row by row) and the kernels read it in place with ld = linesize, as they do for frames that are already on the
             // device; other paddings are dropped by a 2-D copy.
-            const bool keep_pad = ctx->opt_padded_upload && linesize != Wd && linesize % 16 == 0 && (linesize - Wd) * 8 <= Wd;
+            const bool keep_pad = ctx->opt_padded_upload && linesize != rowb && linesize % 16 == 0 && (linesize - rowb) * 8 <= rowb;
             const int64_t sbytes = keep_pad ? H * linesize : fbytes;  // bytes of one staged frame
             if (sbytes * nb > (int64_t)s.stage_in_cap && !s.queue.empty()) { const int r = finish_slot(ctx, s); if (r < 0) return r; }
             if ((rc = ensure_stage(ctx, &s.stage_in, &s.stage_in_cap, (size_t)(sbytes * B)))) return rc;
-            if ((linesize == Wd || keep_pad) && K * fstride == sbytes)  // the frames of the run are contiguous on the host too: one copy
+            if ((linesize == rowb || keep_pad) && K * fstride == sbytes)  // the frames of the run are contiguous on the host too: one copy
                 CU(cudaMemcpyAsync(s.stage_in, frames + i * fstride, (size_t)(sbytes * nb), cudaMemcpyHostToDevice, s.stream));
             else for (int j = 0; j < nb; j++) {
                 const uint8_t* src = frames + (i + j * K) * fstride;
-                if (linesize == Wd || keep_pad) CU(cudaMemcpyAsync((uint8_t*)s.stage_in + j * sbytes, src, (size_t)sbytes, cudaMemcpyHostToDevice, s.stream));
-                else CU(cudaMemcpy2DAsync((uint8_t*)s.stage_in + j * sbytes, Wd, src, linesize, Wd, H, cudaMemcpyHostToDevice, s.stream));
+                if (linesize == rowb || keep_pad) CU(cudaMemcpyAsync((uint8_t*)s.stage_in + j * sbytes, src, (size_t)sbytes, cudaMemcpyHostToDevice, s.stream));
+                else CU(cudaMemcpy2DAsync((uint8_t*)s.stage_in + j * sbytes, rowb, src, linesize, rowb, H, cudaMemcpyHostToDevice, s.stream));
             }
-            fin.data = s.stage_in; fin.ld = keep_pad ? linesize : Wd;
+            fin.data = s.stage_in; fin.ld = keep_pad ? linesize : rowb;
             in_stride = sbytes;
         }
         if (embed_mode) {
             wm_image fout = fin;
-            fout.ld = Wd;
+            fout.ld = rowb;
             int64_t out_stride;
             if (v->frames_on_device) { fout.data = out + i * ostride; out_stride = K * ostride; }
             else {
