@@ -21,7 +21,8 @@ ME, NVF = 0, 1                      # Watermark.hpp:10-14
 COL_MAJOR, ROW_MAJOR = 0, 1
 PACKED_RGB, PACKED_BGR = 2, 3       # interleaved 8-bit colour (rows, cols, 3), row pitch in bytes
 PACKED_RGBA, PACKED_BGRA = 4, 5     # the same with a fourth byte per pixel (rows, cols, 4), copied through by the embed
-PACKED_BYTES = {PACKED_RGB: 3, PACKED_BGR: 3, PACKED_RGBA: 4, PACKED_BGRA: 4}  # bytes per pixel of each packed layout
+PACKED_YUYV, PACKED_UYVY = 6, 7     # packed 4:2:2 (rows, cols, 2): luma at [..., 0] / [..., 1], chroma copied through by the embed
+PACKED_BYTES = {PACKED_RGB: 3, PACKED_BGR: 3, PACKED_RGBA: 4, PACKED_BGRA: 4, PACKED_YUYV: 2, PACKED_UYVY: 2}  # bytes per pixel of each packed layout
 F32, U8 = 0, 1
 OK, SINGULAR, ZERO_MASK = 0, 1, 2
 OPT_FP16_PRODUCTS, OPT_KERNEL_TIMING, OPT_USE_TMA, OPT_SERIAL_SLOTS, OPT_CUDA_GRAPHS, OPT_MMA_ACCUM, OPT_SPLIT_COST = 1, 2, 3, 4, 5, 6, 7
@@ -464,8 +465,9 @@ class Watermark:
 class VideoProcessingContext:
     """videoprocessingcontext.hpp:13-29 minus the ffmpeg handles: frames come from memory.
 
-    layout 0 (Y planes) or a packed colour layout (PACKED_RGB / BGR / RGBA / BGRA: e.g. the BGR frames of cv2.VideoCapture); linesize is
-    the row pitch in bytes (default: dense rows of PACKED_BYTES[layout] * width bytes)."""
+    layout 0 (Y planes), a packed colour layout (PACKED_RGB / BGR / RGBA / BGRA: e.g. the BGR frames of cv2.VideoCapture) or a packed
+    4:2:2 layout (PACKED_YUYV / UYVY: e.g. a V4L2 webcam's YUYV); linesize is the row pitch in bytes (default: dense rows of
+    PACKED_BYTES[layout] * width bytes)."""
 
     def __init__(self, watermark, height, width, watermark_interval, linesize=0, frame_stride=0, frames_on_device=False, layout=0):
         self.watermarkObj, self.height, self.width = watermark, height, width

@@ -65,6 +65,11 @@ def build_video_packed_test(force=False):
     return _build_cpp_test("test_video_packed", force)
 
 
+def build_video_yuv422_test(force=False):
+    """C++ program running processFramesInMemory (csrc/videoprocessingcontext.hpp) on packed YUYV frames, linked against the .so."""
+    return _build_cpp_test("test_video_yuv422", force)
+
+
 def _build_cpp_test(name, force):
     src = os.path.join(ROOT, "tests", "cpp", name + ".cpp")
     exe = os.path.join(ROOT, "tests", "cpp", name)
@@ -99,4 +104,5 @@ if __name__ == "__main__":
     print(build(force="--force" in sys.argv, verbose="-v" in sys.argv))
     print(build_facade_test(force="--force" in sys.argv))
     print(build_video_packed_test(force="--force" in sys.argv))
+    print(build_video_yuv422_test(force="--force" in sys.argv))
     print(build_generator(force="--force" in sys.argv))

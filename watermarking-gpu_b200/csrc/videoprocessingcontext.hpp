@@ -101,13 +101,17 @@ inline float detectFrameWatermark(const VideoProcessingContext& data, int& frame
 // frames per launch sequence with copies and kernels overlapped, on ONE GPU (one Watermark object) or SEVERAL (one object per
 // device: contiguous chunks of the global frame index, one host thread per device, the gate of main.cpp:346,395 on the global
 // index).  `out` receives the Y planes without row padding (gated-off frames copied through), as embedWatermarkFrame writes them.
-// layout 0 (Y planes) or a packed colour layout (WM_PACKED_RGB / BGR / RGBA / BGRA, e.g. the BGR frames of cv2.VideoCapture): `linesize`
-// is then the row pitch in bytes and `out` receives dense height x (bytes per pixel * width) frames (wm_video_ctx in wm_b200.h).
+// layout 0 (Y planes), a packed colour layout (WM_PACKED_RGB / BGR / RGBA / BGRA, e.g. the BGR frames of cv2.VideoCapture) or a packed
+// 4:2:2 layout (WM_PACKED_YUYV / UYVY, e.g. a V4L2 webcam's YUYV): `linesize` is then the row pitch in bytes and `out` receives dense
+// height x (bytes per pixel * width) frames (wm_video_ctx in wm_b200.h).
 inline int64_t processFramesInMemory(const std::vector<const Watermark*>& watermarkPerGpu, const int height, const int width,
                                      const int watermarkInterval, const int linesize, const int mode, const uint8_t* frames,
                                      uint8_t* out, const int64_t firstIndex, const int64_t nFrames, float* scalars, const int layout = 0)
 {
-    const int64_t bpp = layout == WM_PACKED_RGB || layout == WM_PACKED_BGR ? 3 : layout == WM_PACKED_RGBA || layout == WM_PACKED_BGRA ? 4 : 1;
+    const int64_t bpp = layout == WM_PACKED_RGB || layout == WM_PACKED_BGR     ? 3
+                        : layout == WM_PACKED_RGBA || layout == WM_PACKED_BGRA ? 4
+                        : layout == WM_PACKED_YUYV || layout == WM_PACKED_UYVY ? 2
+                                                                               : 1;
     const int ngpus = (int)watermarkPerGpu.size();
     if (ngpus < 1) throw std::runtime_error("processFramesInMemory: no Watermark object\n");
     if (mode == WM_VIDEO_EMBED_VERIFY && ngpus > 1) throw std::runtime_error("processFramesInMemory: EMBED_VERIFY runs on one GPU per call\n");

@@ -60,7 +60,7 @@ struct Slot {
     void* stage_base = nullptr; size_t stage_base_cap = 0;
     void* stage_out = nullptr; size_t stage_out_cap = 0;
     void* maskp = nullptr; size_t maskp_cap = 0;  // NVF mask planes of a batch when p > 3 (k_nvfp)
-    void* gray = nullptr; size_t gray_cap = 0;    // f32 gray planes of a packed RGB / BGR batch (k_packed_gray)
+    void* gray = nullptr; size_t gray_cap = 0;    // gray planes of a packed batch: f32 (k_packed_gray) or the u8 luma of 4:2:2 (k_packed_luma)
     std::vector<TimedLaunch> timed;
     // direct delivery of synchronous single-image ops (slot 0 only): mapped pinned result + device sequence / completion counters
     HostResult* hres = nullptr;      // pinned host memory
@@ -121,18 +121,27 @@ int fail(wm_ctx* c, int code, const std::string& msg)
             return fail(ctx, WM_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_));        \
     } while (0)
 
-// The packed 8-bit layouts: bytes per pixel (0 = not a packed layout) and whether B comes before R.  Every other place reads these two
-// facts from here, so a packed layout is described once.
-struct PackedFmt { int bytes; bool bgr; const char* name; };
+// The packed 8-bit layouts: bytes per pixel (0 = not a packed layout), whether B comes before R, and the byte of a pixel that holds its
+// luma (-1: a colour layout, whose RGB gray is computed).  Every other place reads these facts from here, so a packed layout is described once.
+struct PackedFmt { int bytes; bool bgr; int luma; const char* name; };
 PackedFmt packed_fmt(int layout)
 {
     switch (layout) {
-    case WM_PACKED_RGB: return {3, false, "RGB"};
-    case WM_PACKED_BGR: return {3, true, "BGR"};
-    case WM_PACKED_RGBA: return {4, false, "RGBA"};
-    case WM_PACKED_BGRA: return {4, true, "BGRA"};
-    default: return {0, false, ""};
+    case WM_PACKED_RGB: return {3, false, -1, "RGB"};
+    case WM_PACKED_BGR: return {3, true, -1, "BGR"};
+    case WM_PACKED_RGBA: return {4, false, -1, "RGBA"};
+    case WM_PACKED_BGRA: return {4, true, -1, "BGRA"};
+    case WM_PACKED_YUYV: return {2, false, 0, "YUYV"};
+    case WM_PACKED_UYVY: return {2, false, 1, "UYVY"};
+    default: return {0, false, -1, ""};
     }
+}
+// bytes of the gray plane one image of a packed layout fills in a slot: f32 L x P for the RGB gray; for 4:2:2 the u8 luma at a pitch of
+// round_up(P, 16), so that its rows are TMA-loadable like a caller's Y plane at that pitch
+long long luma_pitch(int P) { return ((long long)P + 15) / 16 * 16; }
+size_t gray_plane_bytes(const PackedFmt& f, int L, int P)
+{
+    return f.luma >= 0 ? (size_t)L * (size_t)luma_pitch(P) : (size_t)L * (size_t)P * sizeof(float);
 }
 // dtype, channels and row pitch of a packed image; *ld receives the pitch in bytes (0 = dense)
 int check_packed(wm_ctx* ctx, const wm_image* im, const PackedFmt& f, long long* ld)
@@ -142,12 +151,14 @@ int check_packed(wm_ctx* ctx, const wm_image* im, const PackedFmt& f, long long*
         return fail(ctx, WM_ERR_ARG, what + " has dtype WM_U8 and " + std::to_string(f.bytes) + " channels");
     *ld = im->ld > 0 ? im->ld : (long long)f.bytes * im->cols;
     if (*ld < (long long)f.bytes * im->cols) return fail(ctx, WM_ERR_ARG, what + ": ld (bytes) smaller than " + std::to_string(f.bytes) + " * cols");
+    if (f.luma >= 0 && im->cols % 2) return fail(ctx, WM_ERR_ARG, what + " has an even number of cols (4:2:2 pairs pixels)");
     return WM_OK;
 }
 
 struct View {  // an image reduced to lines x pixels
     void* ptr; int L, P; long long ld, pstride; int channels; int dtype; bool transposed;
-    int pxb; bool bgr;  // packed 8-bit images: bytes per pixel (3 or 4; 0 = not packed), B before R; L = rows, P = cols, ld in bytes, dtype u8
+    int pxb; bool bgr;  // packed 8-bit images: bytes per pixel (2, 3 or 4; 0 = not packed), B before R; L = rows, P = cols, ld in bytes, dtype u8
+    int luma;           // packed 4:2:2: byte of a pixel holding the luma; -1 otherwise
 };
 
 // allow_packed: the caller handles packed 8-bit images (the embed and detect entry points)
@@ -160,6 +171,7 @@ int make_view(wm_ctx* ctx, const wm_image* im, View* v, bool allow_rgb, bool all
     const PackedFmt f = packed_fmt(im->layout);
     v->pxb = f.bytes;
     v->bgr = f.bgr;
+    v->luma = f.luma;
     if (v->pxb) {
         if (!allow_packed) return fail(ctx, WM_ERR_ARG, std::string("packed ") + f.name + " images are taken by the wm_embed* and wm_detect* entry points only");
         int rc;
@@ -194,11 +206,12 @@ bool vec_ok(const void* p, long long ld, long long bstride, long long pstride, i
     const uintptr_t al = dtype == WM_F32 ? 16 : 4;
     return ((uintptr_t)p % al == 0) && (ld % 4 == 0) && (bstride % 4 == 0) && (pstride % 4 == 0);
 }
-// alignment level of a packed image's rows (launch_packed_gray): 2 = pointer, ld and batch stride are multiples of 16 bytes, 1 = of 4 bytes, 0
-int packed_align(const void* p, long long ld, long long bstride)
+// alignment level of a packed image's rows (launch_packed_gray): 2 = pointer, ld and batch stride are multiples of `vec` bytes (16; 8 for the
+// 4:2:2 apply, whose thread accesses 8 bytes), 1 = of 4 bytes, 0
+int packed_align(const void* p, long long ld, long long bstride, long long vec = 16)
 {
     auto al = [&](long long m) { return (uintptr_t)p % (uintptr_t)m == 0 && ld % m == 0 && bstride % m == 0; };
-    return al(16) ? 2 : al(4) ? 1 : 0;
+    return al(vec) ? 2 : al(4) ? 1 : 0;
 }
 
 
@@ -565,21 +578,32 @@ int reserve_gray(wm_ctx* ctx, Slot& s, size_t need)
     }
     return WM_OK;
 }
-// Packed batch: its gray goes into the slot's dense f32 planes, and *v / *stride become that gray batch, so the op runs on it exactly as
-// on a caller's dense f32 gray batch (same tiles, launch plan and partial sums: the scalars of the composed path).
+// Packed batch: its gray goes into the slot's planes, and *v / *stride become that gray batch.
+// Colour layouts: the RGB gray, dense f32, so the op runs on it exactly as on a caller's dense f32 gray batch (same tiles, launch plan and
+// partial sums: the scalars of the composed path).  4:2:2 layouts: the luma, u8 at a pitch of round_up(P, 16), so the op runs on it exactly
+// as on a caller's u8 Y plane at that pitch (the same u8 kernels, narrow where TMA holds, and plan: the Y-plane bits).
 int enqueue_packed_gray(wm_ctx* ctx, Slot& s, View* v, int64_t* stride, int batch)
 {
-    const size_t plane = (size_t)v->L * v->P;
-    const int rc = reserve_gray(ctx, s, plane * sizeof(float) * batch);
+    const PackedFmt f = {v->pxb, v->bgr, v->luma, ""};
+    const size_t plane = gray_plane_bytes(f, v->L, v->P);
+    const int rc = reserve_gray(ctx, s, plane * batch);
     if (rc) return rc;
-    launch_packed_gray((const uint8_t*)v->ptr, v->ld, *stride, batch, v->pxb, v->bgr, (float*)s.gray, v->L, v->P, packed_align(v->ptr, v->ld, *stride),
-                       8 * ctx->sms, s.stream);
+    const int al = packed_align(v->ptr, v->ld, *stride);
+    if (f.luma >= 0) {
+        const long long lp = luma_pitch(v->P);
+        launch_packed_luma((const uint8_t*)v->ptr, v->ld, *stride, batch, f.luma, (uint8_t*)s.gray, lp, v->L, v->P, al, 8 * ctx->sms, s.stream);
+        v->ld = lp; v->dtype = WM_U8;
+    } else {
+        launch_packed_gray((const uint8_t*)v->ptr, v->ld, *stride, batch, v->pxb, v->bgr, (float*)s.gray, v->L, v->P, al, 8 * ctx->sms, s.stream);
+        v->ld = v->P; v->dtype = WM_F32;
+    }
     ctx->launches++;
     CU(cudaGetLastError());
-    v->ptr = s.gray; v->ld = v->P; v->pstride = (long long)plane; v->channels = 1; v->dtype = WM_F32;
+    v->ptr = s.gray; v->pstride = (long long)v->L * v->ld; v->channels = 1;
     v->pxb = 0;
     v->bgr = false;
-    *stride = (int64_t)plane;
+    v->luma = -1;
+    *stride = (int64_t)v->pstride;
     return WM_OK;
 }
 
@@ -616,12 +640,12 @@ int do_embed(wm_ctx* ctx, int slot, const wm_image* in, const wm_image* base, wm
     if ((rc = make_view(ctx, in, &vi, false, true))) return rc;
     if ((rc = make_view(ctx, base ? base : in, &vb, true, true))) return rc;
     if ((rc = make_view(ctx, out, &vo, true, true))) return rc;
-    const int pxb = vi.pxb;  // packed input: bytes per pixel
+    const int pxb = vi.pxb, luma = vi.luma;  // packed input: bytes per pixel, luma byte (4:2:2)
     if (pxb || vb.pxb || vo.pxb) {
         if (!pxb) return fail(ctx, WM_ERR_ARG, "a packed base or output needs the same packed image as the input");
-        if (vb.pxb != pxb || vb.ptr != vi.ptr || vb.ld != vi.ld || vb.bgr != vi.bgr)
+        if (vb.pxb != pxb || vb.ptr != vi.ptr || vb.ld != vi.ld || vb.bgr != vi.bgr || vb.luma != vi.luma)
             return fail(ctx, WM_ERR_ARG, "with a packed input, base must be NULL or the same image (pointer, layout, ld)");
-        if (vo.pxb != pxb || vo.bgr != vi.bgr) return fail(ctx, WM_ERR_ARG, "with a packed input, out must be a packed image of the same layout");
+        if (vo.pxb != pxb || vo.bgr != vi.bgr || vo.luma != vi.luma) return fail(ctx, WM_ERR_ARG, "with a packed input, out must be a packed image of the same layout");
         if (!base) base_stride = in_stride;  // NULL base: the input batch itself
     }
     if (vb.transposed != vi.transposed || vo.transposed != vi.transposed) return fail(ctx, WM_ERR_ARG, "in/base/out layouts differ");
@@ -669,9 +693,10 @@ int do_embed(wm_ctx* ctx, int slot, const wm_image* in, const wm_image* base, wm
     ea.channels = vb.channels;
     ea.same_base = (vb.ptr == vi.ptr && vb.ld == vi.ld && base_stride == in_stride && vb.channels == 1);
     ea.dl = deliver_args(s, direct && batch == 1);
-    // packed base / out: alignment levels (16-byte, word or byte accesses), as k_packed_gray reads them
-    ea.base_vec_ok = pxb ? packed_align(vb.ptr, vb.ld, base_stride) : vec_ok(vb.ptr, vb.ld, base_stride, vb.channels > 1 ? vb.pstride : 0, vb.dtype);
-    ea.out_vec_ok = pxb ? packed_align(vo.ptr, vo.ld, out_stride) : vec_ok(vo.ptr, vo.ld, out_stride, vo.channels > 1 ? vo.pstride : 0, vo.dtype);
+    // packed base / out: alignment levels (16-byte, or 8-byte for 4:2:2, word or byte accesses)
+    const long long pvec = luma >= 0 ? 8 : 16;
+    ea.base_vec_ok = pxb ? packed_align(vb.ptr, vb.ld, base_stride, pvec) : vec_ok(vb.ptr, vb.ld, base_stride, vb.channels > 1 ? vb.pstride : 0, vb.dtype);
+    ea.out_vec_ok = pxb ? packed_align(vo.ptr, vo.ld, out_stride, pvec) : vec_ok(vo.ptr, vo.ld, out_stride, vo.channels > 1 ? vo.pstride : 0, vo.dtype);
     CUtensorMap tmI, tmW;
     memset(&tmI, 0, sizeof tmI);
     memset(&tmW, 0, sizeof tmW);
@@ -699,11 +724,15 @@ int do_embed(wm_ctx* ctx, int slot, const wm_image* in, const wm_image* base, wm
         PdlScope pdl(ctx->opt_pdl && !ctx->opt_timing && !planes);  // the stats pass of this op precedes
         bool ts = ctx->opt_tma_store && tma && ea.same_base && vo.dtype == vi.dtype && vo.channels == 1 && !planes && tma_ok(ctx, vo, out_stride, batch);
         if (ts) ts = make_tmap(&tmO, vo.dtype, vo.ptr, g.P, g.L, batch, vo.ld, out_stride, TP, TL, TP);
-        for (const SubBatch& sb : pl.embed) {
+        // the packed apply runs NT-thread CTAs, EMBED_CTAS_PER_SM per SM: a plan made for the narrow u8 kernels (4:2:2 luma) is resized for it
+        std::vector<SubBatch> wide;
+        if (pxb && narrow) wide = partition(EMBED_CTAS_PER_SM * ctx->sms, batch, g.ntiles, ctx->opt_split_cost);
+        const std::vector<SubBatch>& apply_sb = wide.empty() ? pl.embed : wide;
+        for (const SubBatch& sb : apply_sb) {
             ea.b0 = sb.b0; ea.nblk_base = sb.base; ea.nblk_extra = sb.extra;
             const dim3 grid(sb.base + (sb.extra > 0 ? 1 : 0), sb.nb);
             if (ts) launch_apply_ts(vi.dtype, kmask, vi.transposed, narrow, grid, s.stream, tmI, tmW, tmO, ea);
-            else if (pxb) launch_apply_packed(kmask, pxb, tma, grid, s.stream, tmI, tmW, ea);
+            else if (pxb) launch_apply_packed(kmask, pxb, luma, tma, grid, s.stream, tmI, tmW, ea);
             else launch_apply(vi.dtype, vo.dtype, kmask, vi.transposed, tma, grid, s.stream, tmI, tmW, ea);
         }
     }
@@ -1471,10 +1500,11 @@ int64_t wm_process_frames(const wm_video_ctx* v, int mode, const uint8_t* frames
     if (v->height != ctx->rows || v->width != ctx->cols) return fail(ctx, WM_ERR_DIMS, "frame dims != watermark dims");
     if (v->watermark_interval < 1) return fail(ctx, WM_ERR_ARG, "watermark_interval must be >= 1");
     if (embed_mode && !out) return fail(ctx, WM_ERR_ARG, "embed needs an output buffer");
-    // Y planes (layout 0 or WM_ROW_MAJOR) have one byte per pixel; packed colour frames packed_fmt's bytes per pixel
+    // Y planes (layout 0 or WM_ROW_MAJOR) have one byte per pixel; packed frames packed_fmt's bytes per pixel
     const PackedFmt pf = packed_fmt(v->layout);
     if (v->layout != 0 && v->layout != WM_ROW_MAJOR && !pf.bytes)
         return fail(ctx, WM_ERR_ARG, "bad frame layout " + std::to_string(v->layout) + " (0 / WM_ROW_MAJOR: Y planes, or a WM_PACKED_* layout)");
+    if (pf.luma >= 0 && v->width % 2) return fail(ctx, WM_ERR_ARG, std::string("packed ") + pf.name + " frames have an even width (4:2:2 pairs pixels)");
     const int64_t H = v->height, Wd = v->width;
     const int64_t rowb = (pf.bytes ? pf.bytes : 1) * Wd;  // bytes of a frame row without padding
     const int64_t linesize = v->linesize > 0 ? v->linesize : rowb;
@@ -1510,11 +1540,11 @@ int64_t wm_process_frames(const wm_video_ctx* v, int mode, const uint8_t* frames
     int64_t B = v->frames_on_device ? std::max<int64_t>(1, std::min<int64_t>(32, ((int64_t)ctx->opt_run_mb << 20) / fbytes)) : ctx->opt_host_run;
     // even runs (37 frames at 7 per run: 7,6,6,6,6,6 rather than 7,7,7,7,7,2)
     const int64_t nruns = ngated > 0 ? (ngated + B - 1) / B : 0;
-    // packed frames: each slot that takes a run computes its gray into its own f32 planes.  They are sized once for the longest run these
-    // options allow, so calls whose even runs differ by a frame (other frame counts, first indices) do not regrow them with a stream sync
+    // packed frames: each slot that takes a run computes its gray (or luma) into its own planes.  They are sized once for the longest run
+    // these options allow, so calls whose even runs differ by a frame (other frame counts, first indices) do not regrow them with a stream sync
     if (pf.bytes)
         for (int64_t r = 0; r < std::min<int64_t>(nruns, ctx->opt_serial ? 1 : NSLOTS); r++)
-            if ((rc = reserve_gray(ctx, ctx->slots[r], (size_t)(H * Wd) * sizeof(float) * (size_t)B))) return rc;
+            if ((rc = reserve_gray(ctx, ctx->slots[r], gray_plane_bytes(pf, (int)H, (int)Wd) * (size_t)B))) return rc;
     const int64_t run_base = nruns ? ngated / nruns : 0, run_extra = nruns ? ngated % nruns : 0;
     B = run_base + (run_extra ? 1 : 0);
     for (int64_t g = 0, run = 0, nbr = 0; run < nruns; g += nbr, run++) {

@@ -32,15 +32,19 @@ void launch_apply_ts(int dtype, int mask, bool tr, bool narrow, dim3 grid, cudaS
 #undef WM_TS
 }
 
-void launch_apply_packed(int mask, int pixel_bytes, bool tma, dim3 grid, cudaStream_t st, const CUtensorMap& tmI, const CUtensorMap& tmW,
+void launch_apply_packed(int mask, int pixel_bytes, int luma, bool tma, dim3 grid, cudaStream_t st, const CUtensorMap& tmI, const CUtensorMap& tmW,
                          const EmbedArgs& a)
 {
-#define WM_PK(TMA, PB)                                                                                                                 \
-    if (mask == 2) WM_LAUNCH((k_apply<float, uint8_t, 2, false, TMA, false, PB>), embed_smem(TMA, false), tmI, tmW, a);               \
-    else if (mask == WM_MASK_ME) WM_LAUNCH((k_apply<float, uint8_t, 0, false, TMA, false, PB>), embed_smem(TMA, false), tmI, tmW, a);  \
-    else WM_LAUNCH((k_apply<float, uint8_t, 1, false, TMA, false, PB>), embed_smem(TMA, false), tmI, tmW, a);
-    if (pixel_bytes == 4) { if (tma) { WM_PK(true, 4) } else { WM_PK(false, 4) } }
-    else { if (tma) { WM_PK(true, 3) } else { WM_PK(false, 3) } }
+#define WM_PK(PIX, TMA, PB, OFF)                                                                                                       \
+    if (mask == 2) WM_LAUNCH((k_apply<PIX, uint8_t, 2, false, TMA, false, PB, OFF>), embed_smem(TMA, sizeof(PIX) == 1), tmI, tmW, a);   \
+    else if (mask == WM_MASK_ME) WM_LAUNCH((k_apply<PIX, uint8_t, 0, false, TMA, false, PB, OFF>), embed_smem(TMA, sizeof(PIX) == 1), tmI, tmW, a); \
+    else WM_LAUNCH((k_apply<PIX, uint8_t, 1, false, TMA, false, PB, OFF>), embed_smem(TMA, sizeof(PIX) == 1), tmI, tmW, a);
+    if (pixel_bytes == 2) {  // 4:2:2: the input is the u8 luma plane
+        if (luma) { if (tma) { WM_PK(uint8_t, true, 2, 1) } else { WM_PK(uint8_t, false, 2, 1) } }
+        else { if (tma) { WM_PK(uint8_t, true, 2, 0) } else { WM_PK(uint8_t, false, 2, 0) } }
+    }
+    else if (pixel_bytes == 4) { if (tma) { WM_PK(float, true, 4, 0) } else { WM_PK(float, false, 4, 0) } }
+    else { if (tma) { WM_PK(float, true, 3, 0) } else { WM_PK(float, false, 3, 0) } }
 #undef WM_PK
 }
 

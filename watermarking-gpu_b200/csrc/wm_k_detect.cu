@@ -93,6 +93,14 @@ void launch_packed_gray(const uint8_t* src, long long ld, long long bstride, int
     }
 }
 
+void launch_packed_luma(const uint8_t* src, long long ld, long long bstride, int batch, int luma, uint8_t* dst, long long lp, int L, int P,
+                        int align, int blocks, cudaStream_t st)
+{
+    const dim3 grid((unsigned)(blocks > batch ? blocks / batch : 1), (unsigned)batch);
+    if (luma) k_packed_luma<1><<<grid, 256, 0, st>>>(src, ld, bstride, dst, lp, L, P, align);
+    else k_packed_luma<0><<<grid, 256, 0, st>>>(src, ld, bstride, dst, lp, L, P, align);
+}
+
 void launch_transpose(const float* src, float* dst, int rows, int cols, cudaStream_t st)
 {
     const dim3 blk(32, 8), grd((unsigned)((cols + 31) / 32), (unsigned)((rows + 31) / 32));

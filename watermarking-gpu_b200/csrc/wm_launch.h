@@ -23,9 +23,14 @@ void launch_rgb2gray(const float* r, const float* g, const float* b, float* gray
 // align: 2 = src, ld and bstride are multiples of 16 bytes, 1 = of 4 bytes, 0 = neither
 void launch_packed_gray(const uint8_t* src, long long ld, long long bstride, int batch, int pixel_bytes, bool bgr, float* gray, int L, int P,
                         int align, int blocks, cudaStream_t st);
-// apply kernel of a packed image: input = its gray (f32, dense), base / out = the packed image and the packed output
-// (a.base_vec_ok / a.out_vec_ok: their alignment levels, as for launch_packed_gray)
-void launch_apply_packed(int mask, int pixel_bytes, bool tma, dim3 grid, cudaStream_t st, const CUtensorMap& tmI, const CUtensorMap& tmW,
+// packed 4:2:2 batch (byte ld / stride; luma at byte `luma` of a pixel: 0 YUYV, 1 UYVY; P even) -> u8 luma planes [batch][L x lp], lp a
+// multiple of 16; align as above
+void launch_packed_luma(const uint8_t* src, long long ld, long long bstride, int batch, int luma, uint8_t* dst, long long lp, int L, int P,
+                        int align, int blocks, cudaStream_t st);
+// apply kernel of a packed image: input = its gray (f32, dense) or, for 4:2:2 images (pixel_bytes 2), its u8 luma plane; base / out = the
+// packed image and the packed output (a.base_vec_ok / a.out_vec_ok: their alignment levels, as for launch_packed_gray; 4:2:2 images: level 2
+// means 8-byte aligned)
+void launch_apply_packed(int mask, int pixel_bytes, int luma, bool tma, dim3 grid, cudaStream_t st, const CUtensorMap& tmI, const CUtensorMap& tmW,
                          const EmbedArgs& a);
 }  // namespace wm
 
