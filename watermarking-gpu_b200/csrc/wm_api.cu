@@ -121,19 +121,21 @@ int fail(wm_ctx* c, int code, const std::string& msg)
             return fail(ctx, WM_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_));        \
     } while (0)
 
-// The packed 8-bit layouts: bytes per pixel (0 = not a packed layout), whether B comes before R, and the byte of a pixel that holds its
-// luma (-1: a colour layout, whose RGB gray is computed).  Every other place reads these facts from here, so a packed layout is described once.
-struct PackedFmt { int bytes; bool bgr; int luma; const char* name; };
+// The packed 8-bit layouts: bytes per pixel (0 = not a packed layout), whether B comes before R, the byte of a pixel that holds its
+// luma (-1: a colour layout, whose RGB gray is computed) and the bytes the packed apply kernel moves in one aligned access of a thread's
+// four pixels.  Every other place reads these facts from here, so a packed layout is described once.
+struct PackedFmt { int bytes; bool bgr; int luma; int apply_vec; const char* name; };
+constexpr PackedFmt PLANAR = {0, false, -1, 0, ""};
 PackedFmt packed_fmt(int layout)
 {
     switch (layout) {
-    case WM_PACKED_RGB: return {3, false, -1, "RGB"};
-    case WM_PACKED_BGR: return {3, true, -1, "BGR"};
-    case WM_PACKED_RGBA: return {4, false, -1, "RGBA"};
-    case WM_PACKED_BGRA: return {4, true, -1, "BGRA"};
-    case WM_PACKED_YUYV: return {2, false, 0, "YUYV"};
-    case WM_PACKED_UYVY: return {2, false, 1, "UYVY"};
-    default: return {0, false, -1, ""};
+    case WM_PACKED_RGB: return {3, false, -1, 16, "RGB"};
+    case WM_PACKED_BGR: return {3, true, -1, 16, "BGR"};
+    case WM_PACKED_RGBA: return {4, false, -1, 16, "RGBA"};
+    case WM_PACKED_BGRA: return {4, true, -1, 16, "BGRA"};
+    case WM_PACKED_YUYV: return {2, false, 0, 8, "YUYV"};
+    case WM_PACKED_UYVY: return {2, false, 1, 8, "UYVY"};
+    default: return PLANAR;
     }
 }
 // bytes of the gray plane one image of a packed layout fills in a slot: f32 L x P for the RGB gray; for 4:2:2 the u8 luma at a pitch of
@@ -143,46 +145,55 @@ size_t gray_plane_bytes(const PackedFmt& f, int L, int P)
 {
     return f.luma >= 0 ? (size_t)L * (size_t)luma_pitch(P) : (size_t)L * (size_t)P * sizeof(float);
 }
-// dtype, channels and row pitch of a packed image; *ld receives the pitch in bytes (0 = dense)
-int check_packed(wm_ctx* ctx, const wm_image* im, const PackedFmt& f, long long* ld)
-{
-    const std::string what = std::string("a packed ") + f.name + " image";
-    if (im->dtype != WM_U8 || im->channels != f.bytes)
-        return fail(ctx, WM_ERR_ARG, what + " has dtype WM_U8 and " + std::to_string(f.bytes) + " channels");
-    *ld = im->ld > 0 ? im->ld : (long long)f.bytes * im->cols;
-    if (*ld < (long long)f.bytes * im->cols) return fail(ctx, WM_ERR_ARG, what + ": ld (bytes) smaller than " + std::to_string(f.bytes) + " * cols");
-    if (f.luma >= 0 && im->cols % 2) return fail(ctx, WM_ERR_ARG, what + " has an even number of cols (4:2:2 pairs pixels)");
-    return WM_OK;
-}
-
-struct View {  // an image reduced to lines x pixels
+// An image reduced to planes of L lines x P pixels; ld and pstride are in elements.  A packed image is one plane of L = rows lines of
+// P = cols pixels, ld in bytes, dtype u8 and channels = bytes per pixel.
+struct View {
     void* ptr; int L, P; long long ld, pstride; int channels; int dtype; bool transposed;
-    int pxb; bool bgr;  // packed 8-bit images: bytes per pixel (2, 3 or 4; 0 = not packed), B before R; L = rows, P = cols, ld in bytes, dtype u8
-    int luma;           // packed 4:2:2: byte of a pixel holding the luma; -1 otherwise
+    int layout; PackedFmt fmt;  // fmt.bytes == 0: a planar image
+    bool packed() const { return fmt.bytes != 0; }
+    long long elem() const { return dtype == WM_F32 ? 4 : 1; }
+    int planes() const { return packed() ? 1 : channels; }
+    long long row_bytes() const { return (long long)P * (packed() ? fmt.bytes : elem()); }  // of a line's pixels, without its padding
+    long long pitch() const { return ld * elem(); }
+    long long plane_bytes() const { return pstride * elem(); }
+    long long extent() const { return (planes() - 1) * plane_bytes() + (L - 1) * pitch() + row_bytes(); }  // first byte to past the last pixel
 };
 
-// allow_packed: the caller handles packed 8-bit images (the embed and detect entry points)
-int make_view(wm_ctx* ctx, const wm_image* im, View* v, bool allow_rgb, bool allow_packed = false)
+// Compares an image on the device with the watermark's dims, before make_view checks the rest of it.  A host image is compared once it
+// is staged, so its descriptor is checked first.
+int check_dims(wm_ctx* ctx, const wm_image* im)
 {
     if (!im || !im->data) return fail(ctx, WM_ERR_ARG, "null image");
     if (im->rows != ctx->rows || im->cols != ctx->cols)
         return fail(ctx, WM_ERR_DIMS, "image dims " + std::to_string(im->rows) + "x" + std::to_string(im->cols) +
                                           " != watermark dims " + std::to_string(ctx->rows) + "x" + std::to_string(ctx->cols));
-    const PackedFmt f = packed_fmt(im->layout);
-    v->pxb = f.bytes;
-    v->bgr = f.bgr;
-    v->luma = f.luma;
-    if (v->pxb) {
+    return WM_OK;
+}
+// Checks an image descriptor and reduces it to a View.  allow_rgb: three planes are taken (base / out).  allow_packed: packed 8-bit
+// images are taken (the embed and detect entry points).  channels_from_layout: a packed image's channels field is not read but implied
+// by its layout (the video driver's frames, which have no such field).
+int make_view(wm_ctx* ctx, const wm_image* im, View* v, bool allow_rgb, bool allow_packed = false, bool channels_from_layout = false)
+{
+    if (!im || !im->data) return fail(ctx, WM_ERR_ARG, "null image");
+    if (im->rows < 1 || im->cols < 1) return fail(ctx, WM_ERR_ARG, "image rows and cols must be positive");
+    v->ptr = im->data;
+    v->layout = im->layout;
+    v->fmt = packed_fmt(im->layout);
+    if (v->packed()) {
+        const PackedFmt& f = v->fmt;
+        const std::string what = std::string("a packed ") + f.name + " image";
         if (!allow_packed) return fail(ctx, WM_ERR_ARG, std::string("packed ") + f.name + " images are taken by the wm_embed* and wm_detect* entry points only");
-        int rc;
-        if ((rc = check_packed(ctx, im, f, &v->ld))) return rc;
+        if (im->dtype != WM_U8 || (im->channels != f.bytes && !channels_from_layout))
+            return fail(ctx, WM_ERR_ARG, what + " has dtype WM_U8 and " + std::to_string(f.bytes) + " channels");
         v->transposed = false;
         v->L = (int)im->rows;
         v->P = (int)im->cols;
-        v->pstride = 0;
         v->channels = f.bytes;
         v->dtype = WM_U8;
-        v->ptr = im->data;
+        v->ld = im->ld > 0 ? im->ld : v->row_bytes();
+        if (v->ld < v->row_bytes()) return fail(ctx, WM_ERR_ARG, what + ": ld (bytes) smaller than " + std::to_string(f.bytes) + " * cols");
+        if (f.luma >= 0 && im->cols % 2) return fail(ctx, WM_ERR_ARG, what + " has an even number of cols (4:2:2 pairs pixels)");
+        v->pstride = (long long)v->L * v->ld;
         return WM_OK;
     }
     if (im->layout != WM_COL_MAJOR && im->layout != WM_ROW_MAJOR) return fail(ctx, WM_ERR_ARG, "bad layout");
@@ -197,7 +208,6 @@ int make_view(wm_ctx* ctx, const wm_image* im, View* v, bool allow_rgb, bool all
     v->pstride = im->plane_stride > 0 ? im->plane_stride : (long long)v->L * v->ld;
     v->channels = ch;
     v->dtype = im->dtype;
-    v->ptr = im->data;
     return WM_OK;
 }
 
@@ -220,20 +230,17 @@ int packed_align(const void* p, long long ld, long long bstride, long long vec =
 // apply kernel's base / out addressing all see the same number.
 int resolve_stride(wm_ctx* ctx, const View& v, int batch, int64_t* stride, const char* what)
 {
-    // elements (bytes for packed images: one interleaved plane) spanned by one image
-    const long long one = v.pxb ? (long long)v.L * v.ld : v.pstride * (v.channels - 1) + (long long)v.L * v.ld;
-    if (*stride == 0) *stride = v.pxb ? one : v.pstride * v.channels;
+    // elements spanned by one image, the padding of its last line included
+    const long long one = v.pstride * (v.planes() - 1) + (long long)v.L * v.ld;
+    if (*stride == 0) *stride = v.pstride * v.planes();
     if (batch > 1 && *stride < one) return fail(ctx, WM_ERR_ARG, std::string(what) + " batch stride smaller than one image");
     return WM_OK;
 }
 // [first, last) bytes touched by a batch
 void byte_range(const View& v, int64_t stride, int batch, uintptr_t* lo, uintptr_t* hi)
 {
-    const long long es = v.dtype == WM_F32 ? 4 : 1;
-    const long long last = (long long)(batch - 1) * stride + (long long)(v.L - 1) * v.ld +
-                           (v.pxb ? (long long)v.pxb * v.P : v.pstride * (v.channels - 1) + v.P);
     *lo = (uintptr_t)v.ptr;
-    *hi = (uintptr_t)v.ptr + (uintptr_t)(last * es);
+    *hi = (uintptr_t)v.ptr + (uintptr_t)((long long)(batch - 1) * stride * v.elem() + v.extent());
 }
 
 int finish_slot(wm_ctx* ctx, Slot& s);
@@ -584,7 +591,7 @@ int reserve_gray(wm_ctx* ctx, Slot& s, size_t need)
 // as on a caller's u8 Y plane at that pitch (the same u8 kernels, narrow where TMA holds, and plan: the Y-plane bits).
 int enqueue_packed_gray(wm_ctx* ctx, Slot& s, View* v, int64_t* stride, int batch)
 {
-    const PackedFmt f = {v->pxb, v->bgr, v->luma, ""};
+    const PackedFmt& f = v->fmt;
     const size_t plane = gray_plane_bytes(f, v->L, v->P);
     const int rc = reserve_gray(ctx, s, plane * batch);
     if (rc) return rc;
@@ -594,15 +601,14 @@ int enqueue_packed_gray(wm_ctx* ctx, Slot& s, View* v, int64_t* stride, int batc
         launch_packed_luma((const uint8_t*)v->ptr, v->ld, *stride, batch, f.luma, (uint8_t*)s.gray, lp, v->L, v->P, al, 8 * ctx->sms, s.stream);
         v->ld = lp; v->dtype = WM_U8;
     } else {
-        launch_packed_gray((const uint8_t*)v->ptr, v->ld, *stride, batch, v->pxb, v->bgr, (float*)s.gray, v->L, v->P, al, 8 * ctx->sms, s.stream);
+        launch_packed_gray((const uint8_t*)v->ptr, v->ld, *stride, batch, f.bytes, f.bgr, (float*)s.gray, v->L, v->P, al, 8 * ctx->sms, s.stream);
         v->ld = v->P; v->dtype = WM_F32;
     }
     ctx->launches++;
     CU(cudaGetLastError());
     v->ptr = s.gray; v->pstride = (long long)v->L * v->ld; v->channels = 1;
-    v->pxb = 0;
-    v->bgr = false;
-    v->luma = -1;
+    v->layout = WM_ROW_MAJOR;
+    v->fmt = PLANAR;
     *stride = (int64_t)v->pstride;
     return WM_OK;
 }
@@ -637,15 +643,16 @@ int do_embed(wm_ctx* ctx, int slot, const wm_image* in, const wm_image* base, wm
     if (batch < 1 || batch > 65535) return fail(ctx, WM_ERR_ARG, "batch must be 1..65535");
     View vi, vb, vo;
     int rc;
-    if ((rc = make_view(ctx, in, &vi, false, true))) return rc;
-    if ((rc = make_view(ctx, base ? base : in, &vb, true, true))) return rc;
-    if ((rc = make_view(ctx, out, &vo, true, true))) return rc;
-    const int pxb = vi.pxb, luma = vi.luma;  // packed input: bytes per pixel, luma byte (4:2:2)
-    if (pxb || vb.pxb || vo.pxb) {
-        if (!pxb) return fail(ctx, WM_ERR_ARG, "a packed base or output needs the same packed image as the input");
-        if (vb.pxb != pxb || vb.ptr != vi.ptr || vb.ld != vi.ld || vb.bgr != vi.bgr || vb.luma != vi.luma)
+    if ((rc = check_dims(ctx, in)) || (rc = make_view(ctx, in, &vi, false, true))) return rc;
+    if ((rc = check_dims(ctx, base ? base : in)) || (rc = make_view(ctx, base ? base : in, &vb, true, true))) return rc;
+    if ((rc = check_dims(ctx, out)) || (rc = make_view(ctx, out, &vo, true, true))) return rc;
+    // a packed input: base and out are packed images of its layout, so the apply kernel reads its format from them
+    const bool packed = vi.packed();
+    if (packed || vb.packed() || vo.packed()) {
+        if (!packed) return fail(ctx, WM_ERR_ARG, "a packed base or output needs the same packed image as the input");
+        if (vb.layout != vi.layout || vb.ptr != vi.ptr || vb.ld != vi.ld)
             return fail(ctx, WM_ERR_ARG, "with a packed input, base must be NULL or the same image (pointer, layout, ld)");
-        if (vo.pxb != pxb || vo.bgr != vi.bgr || vo.luma != vi.luma) return fail(ctx, WM_ERR_ARG, "with a packed input, out must be a packed image of the same layout");
+        if (vo.layout != vi.layout) return fail(ctx, WM_ERR_ARG, "with a packed input, out must be a packed image of the same layout");
         if (!base) base_stride = in_stride;  // NULL base: the input batch itself
     }
     if (vb.transposed != vi.transposed || vo.transposed != vi.transposed) return fail(ctx, WM_ERR_ARG, "in/base/out layouts differ");
@@ -654,7 +661,7 @@ int do_embed(wm_ctx* ctx, int slot, const wm_image* in, const wm_image* base, wm
     if ((rc = resolve_stride(ctx, vi, batch, &in_stride, "in"))) return rc;
     if ((rc = resolve_stride(ctx, vb, batch, &base_stride, "base"))) return rc;
     if ((rc = resolve_stride(ctx, vo, batch, &out_stride, "out"))) return rc;
-    if (pxb && batch > 1 && base_stride != in_stride) return fail(ctx, WM_ERR_ARG, "with a packed input, base must be the same batch (stride)");
+    if (packed && batch > 1 && base_stride != in_stride) return fail(ctx, WM_ERR_ARG, "with a packed input, base must be the same batch (stride)");
     {
         uintptr_t ilo, ihi, olo, ohi;
         byte_range(vi, in_stride, batch, &ilo, &ihi);
@@ -663,7 +670,7 @@ int do_embed(wm_ctx* ctx, int slot, const wm_image* in, const wm_image* base, wm
     }
     CU(cudaSetDevice(ctx->device));
     Slot& s = ctx->slots[slot];
-    if (pxb && (rc = enqueue_packed_gray(ctx, s, &vi, &in_stride, batch))) return rc;
+    if (packed && (rc = enqueue_packed_gray(ctx, s, &vi, &in_stride, batch))) return rc;
     const Geo g = geo(vi.L, vi.P);
     const bool narrow = ctx->opt_narrow_u8 && vi.dtype == WM_U8 && tma_ok(ctx, vi, in_stride, batch);
     const Plan pl = plan(ctx, g, batch, vi.dtype, narrow);
@@ -693,10 +700,9 @@ int do_embed(wm_ctx* ctx, int slot, const wm_image* in, const wm_image* base, wm
     ea.channels = vb.channels;
     ea.same_base = (vb.ptr == vi.ptr && vb.ld == vi.ld && base_stride == in_stride && vb.channels == 1);
     ea.dl = deliver_args(s, direct && batch == 1);
-    // packed base / out: alignment levels (16-byte, or 8-byte for 4:2:2, word or byte accesses)
-    const long long pvec = luma >= 0 ? 8 : 16;
-    ea.base_vec_ok = pxb ? packed_align(vb.ptr, vb.ld, base_stride, pvec) : vec_ok(vb.ptr, vb.ld, base_stride, vb.channels > 1 ? vb.pstride : 0, vb.dtype);
-    ea.out_vec_ok = pxb ? packed_align(vo.ptr, vo.ld, out_stride, pvec) : vec_ok(vo.ptr, vo.ld, out_stride, vo.channels > 1 ? vo.pstride : 0, vo.dtype);
+    // packed base / out: alignment levels (the apply kernel's vector access, word or byte accesses)
+    ea.base_vec_ok = packed ? packed_align(vb.ptr, vb.ld, base_stride, vb.fmt.apply_vec) : vec_ok(vb.ptr, vb.ld, base_stride, vb.channels > 1 ? vb.pstride : 0, vb.dtype);
+    ea.out_vec_ok = packed ? packed_align(vo.ptr, vo.ld, out_stride, vo.fmt.apply_vec) : vec_ok(vo.ptr, vo.ld, out_stride, vo.channels > 1 ? vo.pstride : 0, vo.dtype);
     CUtensorMap tmI, tmW;
     memset(&tmI, 0, sizeof tmI);
     memset(&tmW, 0, sizeof tmW);
@@ -726,13 +732,13 @@ int do_embed(wm_ctx* ctx, int slot, const wm_image* in, const wm_image* base, wm
         if (ts) ts = make_tmap(&tmO, vo.dtype, vo.ptr, g.P, g.L, batch, vo.ld, out_stride, TP, TL, TP);
         // the packed apply runs NT-thread CTAs, EMBED_CTAS_PER_SM per SM: a plan made for the narrow u8 kernels (4:2:2 luma) is resized for it
         std::vector<SubBatch> wide;
-        if (pxb && narrow) wide = partition(EMBED_CTAS_PER_SM * ctx->sms, batch, g.ntiles, ctx->opt_split_cost);
+        if (packed && narrow) wide = partition(EMBED_CTAS_PER_SM * ctx->sms, batch, g.ntiles, ctx->opt_split_cost);
         const std::vector<SubBatch>& apply_sb = wide.empty() ? pl.embed : wide;
         for (const SubBatch& sb : apply_sb) {
             ea.b0 = sb.b0; ea.nblk_base = sb.base; ea.nblk_extra = sb.extra;
             const dim3 grid(sb.base + (sb.extra > 0 ? 1 : 0), sb.nb);
             if (ts) launch_apply_ts(vi.dtype, kmask, vi.transposed, narrow, grid, s.stream, tmI, tmW, tmO, ea);
-            else if (pxb) launch_apply_packed(kmask, pxb, luma, tma, grid, s.stream, tmI, tmW, ea);
+            else if (packed) launch_apply_packed(kmask, vo.fmt.bytes, vo.fmt.luma, tma, grid, s.stream, tmI, tmW, ea);
             else launch_apply(vi.dtype, vo.dtype, kmask, vi.transposed, tma, grid, s.stream, tmI, tmW, ea);
         }
     }
@@ -750,11 +756,11 @@ int do_detect(wm_ctx* ctx, int slot, const wm_image* img, int64_t img_stride, in
     if (batch < 1 || batch > 65535) return fail(ctx, WM_ERR_ARG, "batch must be 1..65535");
     View v;
     int rc;
-    if ((rc = make_view(ctx, img, &v, false, true))) return rc;
+    if ((rc = check_dims(ctx, img)) || (rc = make_view(ctx, img, &v, false, true))) return rc;
     if ((rc = resolve_stride(ctx, v, batch, &img_stride, "image"))) return rc;
     CU(cudaSetDevice(ctx->device));
     Slot& s = ctx->slots[slot];
-    if (v.pxb && (rc = enqueue_packed_gray(ctx, s, &v, &img_stride, batch))) return rc;
+    if (v.packed() && (rc = enqueue_packed_gray(ctx, s, &v, &img_stride, batch))) return rc;
     const Geo g = geo(v.L, v.P);
     bool tma = tma_ok(ctx, v, img_stride, batch);
     const bool narrow = ctx->opt_narrow_u8 && v.dtype == WM_U8 && tma && !dbg_u;
@@ -1199,46 +1205,21 @@ int wm_detect(wm_ctx* ctx, const wm_image* img, int mask, float* corr_host)
 // DENSELY on the device with one 2-D copy (width = the contiguous dimension, source pitch = ld), exactly the repack the reference does
 // row by row (main.cpp:348-353), and results are copied back the same way, so neither copy touches a byte outside the image's
 // pixels — the caller's row and plane padding stays as it was.
-struct HostGeo { int64_t L, P, ld, ps; int ch; size_t es; };
-static int host_geo(wm_ctx* ctx, const wm_image* im, HostGeo* g)
-{
-    if (!im || !im->data) return fail(ctx, WM_ERR_ARG, "null image");
-    const PackedFmt f = packed_fmt(im->layout);
-    if (f.bytes) {  // one plane of rows x (bytes per pixel * cols) bytes, pitch ld
-        long long ld;
-        const int rc = check_packed(ctx, im, f, &ld);
-        if (rc) return rc;
-        g->L = im->rows; g->P = f.bytes * im->cols; g->ld = ld;
-        if (g->L < 1 || g->P < 1) return fail(ctx, WM_ERR_ARG, "packed image: rows and cols must be positive");
-        g->ch = 1; g->ps = g->L * g->ld; g->es = 1;
-        return WM_OK;
-    }
-    if (im->layout != WM_COL_MAJOR && im->layout != WM_ROW_MAJOR) return fail(ctx, WM_ERR_ARG, "bad layout");
-    if (im->dtype != WM_F32 && im->dtype != WM_U8) return fail(ctx, WM_ERR_ARG, "bad dtype");
-    const bool tr = im->layout == WM_COL_MAJOR;
-    g->L = tr ? im->cols : im->rows; g->P = tr ? im->rows : im->cols;
-    g->ld = im->ld > 0 ? im->ld : g->P;
-    if (g->L < 1 || g->P < 1 || g->ld < g->P) return fail(ctx, WM_ERR_ARG, "ld smaller than the contiguous dimension");
-    g->ch = im->channels <= 0 ? 1 : im->channels;
-    g->ps = im->plane_stride > 0 ? im->plane_stride : g->L * g->ld;
-    g->es = im->dtype == WM_F32 ? 4 : 1;
-    return WM_OK;
-}
-static size_t dense_bytes(const HostGeo& g) { return (size_t)(g.L * g.P * g.ch) * g.es; }
+static size_t dense_bytes(const View& v) { return (size_t)(v.L * v.row_bytes() * v.planes()); }
 // dense device planes <-> strided host planes
-static cudaError_t copy_planes(void* dev, void* host, const HostGeo& g, bool to_device, cudaStream_t st)
+static cudaError_t copy_planes(void* dev, void* host, const View& v, bool to_device, cudaStream_t st)
 {
-    for (int c = 0; c < g.ch; c++) {
-        char* d = (char*)dev + (size_t)c * (size_t)(g.L * g.P) * g.es;
-        char* h = (char*)host + (size_t)c * (size_t)g.ps * g.es;
-        if (g.ld == g.P) {  // dense rows: one linear copy (a 2-D copy is programmed row by row)
-            const size_t n = (size_t)(g.L * g.P) * g.es;
-            const cudaError_t e1 = to_device ? cudaMemcpyAsync(d, h, n, cudaMemcpyHostToDevice, st) : cudaMemcpyAsync(h, d, n, cudaMemcpyDeviceToHost, st);
+    const size_t rb = (size_t)v.row_bytes(), plane = (size_t)v.L * rb;
+    for (int c = 0; c < v.planes(); c++) {
+        char* d = (char*)dev + (size_t)c * plane;
+        char* h = (char*)host + (size_t)c * (size_t)v.plane_bytes();
+        if ((size_t)v.pitch() == rb) {  // dense rows: one linear copy (a 2-D copy is programmed row by row)
+            const cudaError_t e1 = to_device ? cudaMemcpyAsync(d, h, plane, cudaMemcpyHostToDevice, st) : cudaMemcpyAsync(h, d, plane, cudaMemcpyDeviceToHost, st);
             if (e1 != cudaSuccess) return e1;
             continue;
         }
-        const cudaError_t e = to_device ? cudaMemcpy2DAsync(d, (size_t)g.P * g.es, h, (size_t)g.ld * g.es, (size_t)g.P * g.es, (size_t)g.L, cudaMemcpyHostToDevice, st)
-                                        : cudaMemcpy2DAsync(h, (size_t)g.ld * g.es, d, (size_t)g.P * g.es, (size_t)g.P * g.es, (size_t)g.L, cudaMemcpyDeviceToHost, st);
+        const cudaError_t e = to_device ? cudaMemcpy2DAsync(d, rb, h, (size_t)v.pitch(), rb, (size_t)v.L, cudaMemcpyHostToDevice, st)
+                                        : cudaMemcpy2DAsync(h, (size_t)v.pitch(), d, rb, rb, (size_t)v.L, cudaMemcpyDeviceToHost, st);
         if (e != cudaSuccess) return e;
     }
     return cudaSuccess;
@@ -1251,15 +1232,15 @@ static wm_image dense_desc(const wm_image* im, void* dev)
 }
 
 // staging of a batch: image b of a strided host batch <-> image b of a dense device batch
-static cudaError_t copy_batch(void* dev, void* host, const HostGeo& g, int64_t host_stride, int batch, bool to_device, cudaStream_t st)
+static cudaError_t copy_batch(void* dev, const View& v, int64_t host_stride, int batch, bool to_device, cudaStream_t st)
 {
-    const int64_t hs = host_stride > 0 ? host_stride : g.ps * g.ch;
-    if (g.ld == g.P && g.ps == g.L * g.P && hs == g.ps * g.ch) {  // the whole batch is dense on the host too: one copy
-        const size_t n = dense_bytes(g) * (size_t)batch;
-        return to_device ? cudaMemcpyAsync(dev, host, n, cudaMemcpyHostToDevice, st) : cudaMemcpyAsync(host, dev, n, cudaMemcpyDeviceToHost, st);
+    const size_t n = dense_bytes(v);
+    const long long hs = (host_stride > 0 ? host_stride : v.pstride * v.planes()) * v.elem();  // bytes between host images
+    if (v.pitch() == v.row_bytes() && v.plane_bytes() == v.L * v.row_bytes() && (size_t)hs == n) {  // the whole batch is dense on the host too: one copy
+        return to_device ? cudaMemcpyAsync(dev, v.ptr, n * batch, cudaMemcpyHostToDevice, st) : cudaMemcpyAsync(v.ptr, dev, n * batch, cudaMemcpyDeviceToHost, st);
     }
     for (int b = 0; b < batch; b++) {
-        const cudaError_t e = copy_planes((char*)dev + (size_t)b * dense_bytes(g), (char*)host + (size_t)b * (size_t)hs * g.es, g, to_device, st);
+        const cudaError_t e = copy_planes((char*)dev + (size_t)b * n, (char*)v.ptr + (size_t)b * (size_t)hs, v, to_device, st);
         if (e != cudaSuccess) return e;
     }
     return cudaSuccess;
@@ -1282,27 +1263,26 @@ int wm_embed_host_batch(wm_ctx* ctx, int slot, const wm_image* in, const wm_imag
     CU(cudaSetDevice(ctx->device));
     Slot& s = ctx->slots[slot];
     const wm_image* b = base ? base : in;
-    HostGeo gi, gb, go;
+    View vi, vb, vo;
     int rc;
-    if ((rc = host_geo(ctx, in, &gi)) || (rc = host_geo(ctx, b, &gb)) || (rc = host_geo(ctx, out, &go))) return rc;
-    if (gi.ch != 1) return fail(ctx, WM_ERR_ARG, "the gray input has one channel");
-    if ((rc = grow_stage(ctx, s, &s.stage_in, &s.stage_in_cap, dense_bytes(gi) * batch))) return rc;
-    if ((rc = grow_stage(ctx, s, &s.stage_out, &s.stage_out_cap, dense_bytes(go) * batch))) return rc;
-    const bool base_is_in = b->data == in->data && gb.ch == 1 && gb.ld == gi.ld && b->dtype == in->dtype && b->layout == in->layout &&
+    if ((rc = make_view(ctx, in, &vi, false, true)) || (rc = make_view(ctx, b, &vb, true, true)) || (rc = make_view(ctx, out, &vo, true, true))) return rc;
+    if ((rc = grow_stage(ctx, s, &s.stage_in, &s.stage_in_cap, dense_bytes(vi) * batch))) return rc;
+    if ((rc = grow_stage(ctx, s, &s.stage_out, &s.stage_out_cap, dense_bytes(vo) * batch))) return rc;
+    const bool base_is_in = vb.ptr == vi.ptr && vb.planes() == 1 && vb.ld == vi.ld && vb.dtype == vi.dtype && vb.layout == vi.layout &&
                             (batch == 1 || base_stride == in_stride);
-    if (!base_is_in && (rc = grow_stage(ctx, s, &s.stage_base, &s.stage_base_cap, dense_bytes(gb) * batch))) return rc;
-    CU(copy_batch(s.stage_in, in->data, gi, in_stride, batch, true, s.stream));
+    if (!base_is_in && (rc = grow_stage(ctx, s, &s.stage_base, &s.stage_base_cap, dense_bytes(vb) * batch))) return rc;
+    CU(copy_batch(s.stage_in, vi, in_stride, batch, true, s.stream));
     wm_image din = dense_desc(in, s.stage_in), dbase, dout = dense_desc(out, s.stage_out);
     if (base_is_in) dbase = din;
     else {
-        CU(copy_batch(s.stage_base, b->data, gb, base_stride, batch, true, s.stream));
+        CU(copy_batch(s.stage_base, vb, base_stride, batch, true, s.stream));
         dbase = dense_desc(b, s.stage_base);
     }
     rc = do_embed(ctx, slot, &din, &dbase, &dout, 0, 0, 0, batch, mask);
     if (rc) return rc;
     s.queue.back().scalar = a_host;
     s.queue.back().status = status_host;
-    CU(copy_batch(s.stage_out, out->data, go, out_stride, batch, false, s.stream));
+    CU(copy_batch(s.stage_out, vo, out_stride, batch, false, s.stream));
     return WM_OK;
 }
 
@@ -1313,11 +1293,13 @@ int wm_embed_verify_host_batch(wm_ctx* ctx, int slot, const wm_image* in, const 
                                int64_t base_stride, int64_t out_stride, int batch, int mask, float* a_host, float* corr_host, int* status_host)
 {
     if (!ctx || !out) return WM_ERR_ARG;
+    View vo;
+    int rc = make_view(ctx, out, &vo, true, true);
+    if (rc) return rc;
     // a packed output is verified through its gray, like the reference's detection on the gray of the saved image
-    const bool packed_out = packed_fmt(out->layout).bytes != 0;
-    if (!packed_out && ((out->channels > 1) || out->dtype != (in ? in->dtype : out->dtype)))
+    if (!vo.packed() && (vo.channels > 1 || vo.dtype != (in ? in->dtype : vo.dtype)))
         return fail(ctx, WM_ERR_ARG, "embed + verify needs a gray output of the input's dtype (detectWatermark takes the gray image)");
-    int rc = wm_embed_host_batch(ctx, slot, in, base, out, in_stride, base_stride, out_stride, batch, mask, a_host, status_host);
+    rc = wm_embed_host_batch(ctx, slot, in, base, out, in_stride, base_stride, out_stride, batch, mask, a_host, status_host);
     if (rc) return rc;
     Slot& s = ctx->slots[slot];
     wm_image d = dense_desc(out, s.stage_out);
@@ -1334,12 +1316,11 @@ int wm_detect_host_batch(wm_ctx* ctx, int slot, const wm_image* img, int64_t img
     if (batch < 1 || batch > 65535) return fail(ctx, WM_ERR_ARG, "batch must be 1..65535");
     CU(cudaSetDevice(ctx->device));
     Slot& s = ctx->slots[slot];
-    HostGeo g;
+    View v;
     int rc;
-    if ((rc = host_geo(ctx, img, &g))) return rc;
-    if (g.ch != 1) return fail(ctx, WM_ERR_ARG, "detect takes a one-channel image");
-    if ((rc = grow_stage(ctx, s, &s.stage_in, &s.stage_in_cap, dense_bytes(g) * batch))) return rc;
-    CU(copy_batch(s.stage_in, img->data, g, img_stride, batch, true, s.stream));
+    if ((rc = make_view(ctx, img, &v, false, true))) return rc;
+    if ((rc = grow_stage(ctx, s, &s.stage_in, &s.stage_in_cap, dense_bytes(v) * batch))) return rc;
+    CU(copy_batch(s.stage_in, v, img_stride, batch, true, s.stream));
     wm_image d = dense_desc(img, s.stage_in);
     rc = do_detect(ctx, slot, &d, 0, batch, mask);
     if (rc) return rc;
@@ -1373,8 +1354,8 @@ int wm_rgb2gray(wm_ctx* ctx, const wm_image* rgb, wm_image* gray, float wr, floa
     if (!ctx) return WM_ERR_ARG;
     View vi, vo;
     int rc;
-    if ((rc = make_view(ctx, rgb, &vi, true))) return rc;
-    if ((rc = make_view(ctx, gray, &vo, false))) return rc;
+    if ((rc = check_dims(ctx, rgb)) || (rc = make_view(ctx, rgb, &vi, true))) return rc;
+    if ((rc = check_dims(ctx, gray)) || (rc = make_view(ctx, gray, &vo, false))) return rc;
     if (vi.channels != 3 || vi.dtype != WM_F32 || vo.dtype != WM_F32 || vi.transposed != vo.transposed)
         return fail(ctx, WM_ERR_ARG, "rgb2gray needs a 3-channel f32 input and a 1-channel f32 output of the same layout");
     CU(cudaSetDevice(ctx->device));
@@ -1427,11 +1408,13 @@ int wm_debug_set_coeffs(wm_ctx* ctx, const float* c)
 int wm_debug_detect_planes(wm_ctx* ctx, const wm_image* img, int mask, float* u_dev, float* eu_dev, float* corr_host)
 {
     if (!ctx || !img || !u_dev || !eu_dev) return WM_ERR_ARG;
-    if (packed_fmt(img->layout).bytes) return fail(ctx, WM_ERR_ARG, "detector planes: gray f32 images only, not packed images");
-    if (img->dtype != WM_F32 || (mask == WM_MASK_NVF && ctx->p != 3)) return fail(ctx, WM_ERR_ARG, "detector planes: f32 images, 3x3 masks");
+    View v;
+    int rc;
+    if ((rc = make_view(ctx, img, &v, false))) return rc;  // gray images only: packed images are refused here
+    if (v.dtype != WM_F32 || (mask == WM_MASK_NVF && ctx->p != 3)) return fail(ctx, WM_ERR_ARG, "detector planes: f32 images, 3x3 masks");
     Slot& s = ctx->slots[0];
     if (!s.queue.empty()) { const int r = finish_slot(ctx, s); if (r < 0) return r; }
-    const int rc = do_detect(ctx, 0, img, 0, 1, mask, u_dev, eu_dev);
+    rc = do_detect(ctx, 0, img, 0, 1, mask, u_dev, eu_dev);
     if (rc) return rc;
     s.queue.back().scalar = corr_host;
     return finish_slot(ctx, s);
@@ -1443,7 +1426,7 @@ int wm_debug_plane(wm_ctx* ctx, const wm_image* img, int what, float* dst_dev)
     if (what != WM_DBG_ERRSEQ && what != WM_DBG_MASK_NVF && what != WM_DBG_MASK_ME) return fail(ctx, WM_ERR_ARG, "plane must be ERRSEQ, MASK_NVF or MASK_ME");
     View v;
     int rc;
-    if ((rc = make_view(ctx, img, &v, false))) return rc;
+    if ((rc = check_dims(ctx, img)) || (rc = make_view(ctx, img, &v, false))) return rc;
     CU(cudaSetDevice(ctx->device));
     Slot& s = ctx->slots[0];
     if (!s.queue.empty()) { const int r = finish_slot(ctx, s); if (r < 0) return r; }
@@ -1500,19 +1483,21 @@ int64_t wm_process_frames(const wm_video_ctx* v, int mode, const uint8_t* frames
     if (v->height != ctx->rows || v->width != ctx->cols) return fail(ctx, WM_ERR_DIMS, "frame dims != watermark dims");
     if (v->watermark_interval < 1) return fail(ctx, WM_ERR_ARG, "watermark_interval must be >= 1");
     if (embed_mode && !out) return fail(ctx, WM_ERR_ARG, "embed needs an output buffer");
-    // Y planes (layout 0 or WM_ROW_MAJOR) have one byte per pixel; packed frames packed_fmt's bytes per pixel
-    const PackedFmt pf = packed_fmt(v->layout);
-    if (v->layout != 0 && v->layout != WM_ROW_MAJOR && !pf.bytes)
-        return fail(ctx, WM_ERR_ARG, "bad frame layout " + std::to_string(v->layout) + " (0 / WM_ROW_MAJOR: Y planes, or a WM_PACKED_* layout)");
-    if (pf.luma >= 0 && v->width % 2) return fail(ctx, WM_ERR_ARG, std::string("packed ") + pf.name + " frames have an even width (4:2:2 pairs pixels)");
-    const int64_t H = v->height, Wd = v->width;
-    const int64_t rowb = (pf.bytes ? pf.bytes : 1) * Wd;  // bytes of a frame row without padding
-    const int64_t linesize = v->linesize > 0 ? v->linesize : rowb;
-    if (linesize < rowb) return fail(ctx, WM_ERR_ARG, pf.bytes ? "linesize < bytes per pixel * width" : "linesize < width");
+    // a frame as an image: a Y plane (layout 0 or WM_ROW_MAJOR) or a packed frame, rows of linesize bytes (0 = dense)
+    wm_image frame;
+    memset(&frame, 0, sizeof frame);
+    frame.data = (void*)frames; frame.rows = v->height; frame.cols = v->width; frame.dtype = WM_U8;
+    frame.layout = v->layout ? v->layout : WM_ROW_MAJOR; frame.ld = v->linesize;
+    View fv;
+    int rc;
+    if ((rc = make_view(ctx, &frame, &fv, false, true, true))) return fail(ctx, rc, "frames (ld = linesize): " + ctx->err);
+    frame.channels = fv.channels;
+    const int64_t H = v->height;
+    const int64_t rowb = fv.row_bytes();  // bytes of a frame row without padding
+    const int64_t linesize = fv.pitch();
     const int64_t fstride = v->frame_stride > 0 ? v->frame_stride : H * linesize;
     const int64_t ostride = H * rowb;
     CU(cudaSetDevice(ctx->device));
-    int rc;
     for (int i = 0; i < NSLOTS; i++)
         if (!ctx->slots[i].queue.empty()) { const int r = finish_slot(ctx, ctx->slots[i]); if (r < 0) return r; }
     const float nanv = nanf("");
@@ -1542,9 +1527,9 @@ int64_t wm_process_frames(const wm_video_ctx* v, int mode, const uint8_t* frames
     const int64_t nruns = ngated > 0 ? (ngated + B - 1) / B : 0;
     // packed frames: each slot that takes a run computes its gray (or luma) into its own planes.  They are sized once for the longest run
     // these options allow, so calls whose even runs differ by a frame (other frame counts, first indices) do not regrow them with a stream sync
-    if (pf.bytes)
+    if (fv.packed())
         for (int64_t r = 0; r < std::min<int64_t>(nruns, ctx->opt_serial ? 1 : NSLOTS); r++)
-            if ((rc = reserve_gray(ctx, ctx->slots[r], gray_plane_bytes(pf, (int)H, (int)Wd) * (size_t)B))) return rc;
+            if ((rc = reserve_gray(ctx, ctx->slots[r], gray_plane_bytes(fv.fmt, fv.L, fv.P) * (size_t)B))) return rc;
     const int64_t run_base = nruns ? ngated / nruns : 0, run_extra = nruns ? ngated % nruns : 0;
     B = run_base + (run_extra ? 1 : 0);
     for (int64_t g = 0, run = 0, nbr = 0; run < nruns; g += nbr, run++) {
@@ -1553,10 +1538,7 @@ int64_t wm_process_frames(const wm_video_ctx* v, int mode, const uint8_t* frames
         const int si = ctx->opt_serial ? 0 : (int)(run % NSLOTS);
         Slot& s = ctx->slots[si];
         const int64_t i = i0 + g * K;
-        wm_image fin;
-        memset(&fin, 0, sizeof fin);
-        fin.rows = H; fin.cols = Wd; fin.dtype = WM_U8;
-        fin.channels = pf.bytes ? pf.bytes : 1; fin.layout = pf.bytes ? v->layout : WM_ROW_MAJOR;
+        wm_image fin = frame;
         int64_t in_stride;
         if (v->frames_on_device) {
             fin.data = (void*)(frames + i * fstride); fin.ld = linesize;  // strided reads: no repack pass needed
