@@ -51,6 +51,25 @@
  *     detect: the correlation of the luma.
  *   A mix of YUYV and UYVY, or of a 4:2:2 layout with a colour or planar layout, is refused with WM_ERR_ARG, as are wm_rgb2gray,
  *   wm_debug_plane and wm_debug_detect_planes.
+ *
+ * 10-bit luma planes, as 10-bit decoders hand them over (ffmpeg yuv420p10le / yuv422p10le / yuv444p10le / gray10le Y planes from HEVC
+ * Main10, AV1 10-bit or VP9 profile 2; NVDEC P010 / P210 surfaces):
+ *   WM_Y10     : the sample v (0..1023) of pixel (r,c) in bits 0-9 of the little-endian 16-bit word at data[r*ld + 2*c]; bits 10-15 are
+ *                ignored (yuv4xxp10le, gray10le).
+ *   WM_Y10_MSB : v in bits 6-15 of that word; bits 0-5 are ignored (P010 / P210).
+ *   (Their values are 10 and 11; 8 and 9 name no layout and are refused.)
+ *   dtype must be WM_U8 and channels 2 (bytes per pixel); `ld` is in BYTES (>= 2*cols and even, 0 = dense 2*cols); the data pointer and
+ *   batch strides (bytes) are even.  cols may be odd.  The arithmetic runs on the 8-bit-equivalent scale x = v * 0.25f, exact in f32 and
+ *   in fp16, on which the reference's arithmetic is defined (products of two pixels stay <= 255.75^2 = 65408, below fp16's 65504): by
+ *   definition, the strength factor's peak of 255 is 1020 on the 10-bit scale.  Taken by the same entry points as the other packed layouts:
+ *     embed: in_gray = the image, base = NULL or the same image, out = an image of the same layout, not overlapping in.  With y the f32
+ *            output of wm_embed on a dense f32 plane holding x (base = in, f32 out), out's sample is v' = (uint16_t)clamp(4.0f*y, 0, 1023)
+ *            (truncation, as the reference's .as(u8)); WM_Y10 writes v' with bits 10-15 zero, WM_Y10_MSB writes v' << 6 with bits 0-5
+ *            zero.  `a` is that f32 call's a.  WM_SINGULAR / WM_ZERO_MASK: out receives in's words unchanged, ignored bits included.
+ *            wm_embed_verify_host_batch detects on x' = v' / 4 of the written words.
+ *     detect: the correlation the f32 path gives on x.
+ *   A mix of WM_Y10 and WM_Y10_MSB, or of either with a planar or another packed layout, is refused with WM_ERR_ARG, as are wm_rgb2gray,
+ *   wm_debug_plane and wm_debug_detect_planes.
  */
 #ifndef WM_B200_H
 #define WM_B200_H
@@ -64,7 +83,7 @@ extern "C" {
 /* Watermark.hpp:10-14 — enum MASK_TYPE { ME, NVF } */
 enum { WM_MASK_ME = 0, WM_MASK_NVF = 1 };
 enum { WM_COL_MAJOR = 0, WM_ROW_MAJOR = 1, WM_PACKED_RGB = 2, WM_PACKED_BGR = 3, WM_PACKED_RGBA = 4, WM_PACKED_BGRA = 5, WM_PACKED_YUYV = 6,
-       WM_PACKED_UYVY = 7 };
+       WM_PACKED_UYVY = 7, WM_Y10 = 10, WM_Y10_MSB = 11 };
 enum { WM_F32 = 0, WM_U8 = 1 };
 
 /* return codes: 0 ok; >0 non-fatal (mirrors the reference's fall-backs); <0 errors */
@@ -89,7 +108,7 @@ typedef struct wm_image {
     int64_t ld;            /* leading dimension in elements, bytes for packed images (0 = dense) */
     int32_t channels;      /* 1, or 3 for the RGB base/out of makeWatermark (Watermark.cpp:171); bytes per pixel (2, 3 or 4) for packed images */
     int32_t layout;        /* WM_COL_MAJOR | WM_ROW_MAJOR | WM_PACKED_RGB | WM_PACKED_BGR | WM_PACKED_RGBA | WM_PACKED_BGRA | WM_PACKED_YUYV |
-                              WM_PACKED_UYVY */
+                              WM_PACKED_UYVY | WM_Y10 | WM_Y10_MSB */
     int32_t dtype;         /* WM_F32 | WM_U8 */
     int32_t reserved;
     int64_t plane_stride;  /* elements between channel planes (0 = dense) */
@@ -122,7 +141,7 @@ enum {
     WM_OPT_NARROW_U8 = 14,    /* 1 (default): the stats / apply kernels of u8 frames (TMA path) run on 128-thread CTAs, 4 warps x 8 lines of a tile, four CTAs per SM,
                                  like the sweep; 0: 256-thread CTAs, 8 warps x 4 lines, three per SM.  Same bits */
     WM_OPT_RUN_MB = 15,       /* frames of one run (one batched launch sequence) of wm_process_frames on DEVICE frames fill at most this many MB (default 136, at most
-                                 32 frames; packed frames count their packed bytes): large enough to amortise a launch's ramp and tail, small enough that a run's watermarked frames are still in L2 when
+                                 32 frames; packed frames count their packed bytes, 2 per pixel for 10-bit frames): large enough to amortise a launch's ramp and tail, small enough that a run's watermarked frames are still in L2 when
                                  the detector's kernels read them back */
     WM_OPT_HOST_RUN_FRAMES = 9, /* frames per run (one batched launch sequence + its copies) of wm_process_frames when frames are in HOST memory; default 4 */
     WM_OPT_F32_SOLVE = 8      /* 0 (default): the 8x8 system is summed and solved in f64 (pivot cut 1e-12 max|Rx|); 1: Rx / rx are rounded to f32
@@ -228,7 +247,11 @@ int64_t wm_launch_count(const wm_ctx *ctx); /* kernels launched by this ctx sinc
  * Packed 4:2:2 frames (layout = WM_PACKED_YUYV / UYVY: V4L2 YUYV, YUY2, 2vuy, ffmpeg yuyv422 / uyvy422): height rows of 2 * width bytes
  * (width even), `linesize` the row pitch in bytes (>= 2 * width, 0 = dense), `out` dense height x (2 * width) frames.  A gated frame gets
  * what wm_embed / wm_detect give it: `a` and the watermark from the luma (the bits of the Y-plane driver on the same luma), the chroma
- * copied unchanged, DETECT / EMBED_VERIFY correlate the luma.  Gated-off frames are copied through, both bytes of a pixel. */
+ * copied unchanged, DETECT / EMBED_VERIFY correlate the luma.  Gated-off frames are copied through, both bytes of a pixel.
+ * 10-bit luma frames (layout = WM_Y10 / WM_Y10_MSB: the Y plane of yuv420p10le and the like, or of NVDEC's P010): height rows of 2 * width
+ * bytes, `linesize` the row pitch in bytes (>= 2 * width and even, 0 = dense; frame_stride even), `out` dense height x (2 * width)
+ * frames.  A gated frame gets exactly what wm_embed / wm_detect give that image with the ME mask; EMBED_VERIFY detects on the written
+ * words.  Gated-off frames are copied through, all 16 bits of every word.  The chroma planes stay with the caller, as for 8-bit Y planes. */
 typedef struct wm_video_ctx {
     wm_ctx *watermark;        /* watermarkObj (non-owning) */
     int32_t height, width;
@@ -237,7 +260,8 @@ typedef struct wm_video_ctx {
     int64_t frame_stride;     /* bytes between consecutive frames in `frames` */
     int32_t frames_on_device; /* 1: `frames`/`out` are device pointers; 0: host (pinned recommended) */
     int32_t layout;           /* 0 or WM_ROW_MAJOR: Y planes; WM_PACKED_RGB | WM_PACKED_BGR | WM_PACKED_RGBA | WM_PACKED_BGRA: packed u8
-                                 colour frames; WM_PACKED_YUYV | WM_PACKED_UYVY: packed 4:2:2 frames; anything else is refused with WM_ERR_ARG */
+                                 colour frames; WM_PACKED_YUYV | WM_PACKED_UYVY: packed 4:2:2 frames; WM_Y10 | WM_Y10_MSB: 10-bit luma
+                                 frames; anything else is refused with WM_ERR_ARG */
 } wm_video_ctx;
 enum { WM_VIDEO_EMBED = 0, WM_VIDEO_DETECT = 1, WM_VIDEO_EMBED_VERIFY = 2 };
 /* Processes frames [first_index, first_index + n_frames) of a stream: frame i is gated by

@@ -22,7 +22,9 @@ COL_MAJOR, ROW_MAJOR = 0, 1
 PACKED_RGB, PACKED_BGR = 2, 3       # interleaved 8-bit colour (rows, cols, 3), row pitch in bytes
 PACKED_RGBA, PACKED_BGRA = 4, 5     # the same with a fourth byte per pixel (rows, cols, 4), copied through by the embed
 PACKED_YUYV, PACKED_UYVY = 6, 7     # packed 4:2:2 (rows, cols, 2): luma at [..., 0] / [..., 1], chroma copied through by the embed
-PACKED_BYTES = {PACKED_RGB: 3, PACKED_BGR: 3, PACKED_RGBA: 4, PACKED_BGRA: 4, PACKED_YUYV: 2, PACKED_UYVY: 2}  # bytes per pixel of each packed layout
+Y10, Y10_MSB = 10, 11               # 10-bit luma (rows, cols) uint16: the sample in bits 0-9 (yuv420p10le Y) / 6-15 (P010 Y)
+WORD_LAYOUTS = (Y10, Y10_MSB)       # one little-endian 16-bit word per pixel
+PACKED_BYTES = {PACKED_RGB: 3, PACKED_BGR: 3, PACKED_RGBA: 4, PACKED_BGRA: 4, PACKED_YUYV: 2, PACKED_UYVY: 2, Y10: 2, Y10_MSB: 2}  # bytes per pixel of each packed layout
 F32, U8 = 0, 1
 OK, SINGULAR, ZERO_MASK = 0, 1, 2
 OPT_FP16_PRODUCTS, OPT_KERNEL_TIMING, OPT_USE_TMA, OPT_SERIAL_SLOTS, OPT_CUDA_GRAPHS, OPT_MMA_ACCUM, OPT_SPLIT_COST = 1, 2, 3, 4, 5, 6, 7
@@ -162,7 +164,8 @@ class DeviceArray:
     """A device buffer holding an image (rows, cols[, 3]) in a given layout; owned via the C ABI.
 
     Planar layouts hold (rows, cols) or (3, rows, cols) images, `ld` in elements.  The packed layouts hold a (rows, cols, n) uint8
-    image, n = PACKED_BYTES[layout], as interleaved rows of n * cols bytes with a row pitch of `ld` bytes (0 = dense)."""
+    image, n = PACKED_BYTES[layout], as interleaved rows of n * cols bytes with a row pitch of `ld` bytes (0 = dense); the 10-bit layouts
+    (WORD_LAYOUTS) a (rows, cols) uint16 image, as rows of little-endian words."""
 
     def __init__(self, wm, rows, cols, layout=COL_MAJOR, dtype=F32, channels=1, ld=0):
         if layout in PACKED_BYTES:
@@ -197,6 +200,8 @@ class DeviceArray:
         return d
 
     def _to_mem(self, img):
+        if self.layout in WORD_LAYOUTS:
+            img = np.ascontiguousarray(np.asarray(img).astype("<u2", casting="same_kind")).view(np.uint8)
         if self.layout in PACKED_BYTES:
             buf = np.zeros((self.L, self.ld), np.uint8)
             buf[:, :self.P] = img.reshape(self.rows, self.P)
@@ -208,7 +213,8 @@ class DeviceArray:
         return buf
 
     def upload(self, img):
-        buf = np.ascontiguousarray(self._to_mem(np.asarray(img, _NP_DT[self.dtype])))
+        img = np.asarray(img) if self.layout in WORD_LAYOUTS else np.asarray(img, _NP_DT[self.dtype])
+        buf = np.ascontiguousarray(self._to_mem(img))
         rc = lib().wm_dev_upload(self.wm._h, self.ptr, buf.ctypes.data, buf.nbytes)
         if rc:
             raise WatermarkError(rc, "upload failed")
@@ -219,7 +225,10 @@ class DeviceArray:
             rc = lib().wm_dev_download(self.wm._h, buf.ctypes.data, self.ptr, buf.nbytes)
             if rc:
                 raise WatermarkError(rc, "download failed")
-            return np.ascontiguousarray(buf[:, :self.P].reshape(self.rows, self.cols, self.channels))
+            px = np.ascontiguousarray(buf[:, :self.P])
+            if self.layout in WORD_LAYOUTS:
+                return px.view("<u2").astype(np.uint16).reshape(self.rows, self.cols)
+            return px.reshape(self.rows, self.cols, self.channels)
         buf = np.empty((self.channels, self.L, self.ld), _NP_DT[self.dtype])
         rc = lib().wm_dev_download(self.wm._h, buf.ctypes.data, self.ptr, buf.nbytes)
         if rc:
@@ -339,6 +348,10 @@ class Watermark:
 
     # -- hot path, host (numpy) arrays: H2D + compute + D2H inside the call -------------------------
     def _host_desc(self, arr, layout):
+        if layout in WORD_LAYOUTS:  # (rows, cols) uint16, pixels contiguous; rows may be pitched
+            if arr.dtype != np.uint16 or arr.ndim != 2 or arr.strides[1] != 2:
+                raise TypeError("an image of a 10-bit layout is a (rows, cols) uint16 array with contiguous pixels")
+            return image_desc(arr.ctypes.data, self.rows, self.cols, layout, U8, arr.strides[0], 2, 0)
         if layout in PACKED_BYTES:  # (rows, cols, n) uint8, pixels and channels contiguous; rows may be pitched (a view of a wider buffer)
             n = PACKED_BYTES[layout]
             if arr.dtype != np.uint8 or arr.ndim != 3 or arr.shape[2] != n or arr.strides[1:] != (n, 1):
@@ -466,8 +479,8 @@ class VideoProcessingContext:
     """videoprocessingcontext.hpp:13-29 minus the ffmpeg handles: frames come from memory.
 
     layout 0 (Y planes), a packed colour layout (PACKED_RGB / BGR / RGBA / BGRA: e.g. the BGR frames of cv2.VideoCapture) or a packed
-    4:2:2 layout (PACKED_YUYV / UYVY: e.g. a V4L2 webcam's YUYV); linesize is the row pitch in bytes (default: dense rows of
-    PACKED_BYTES[layout] * width bytes)."""
+    4:2:2 layout (PACKED_YUYV / UYVY: e.g. a V4L2 webcam's YUYV) or a 10-bit luma layout (Y10 / Y10_MSB: the Y plane of yuv420p10le or
+    P010); linesize is the row pitch in bytes (default: dense rows of PACKED_BYTES[layout] * width bytes)."""
 
     def __init__(self, watermark, height, width, watermark_interval, linesize=0, frame_stride=0, frames_on_device=False, layout=0):
         self.watermarkObj, self.height, self.width = watermark, height, width

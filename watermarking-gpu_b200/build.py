@@ -70,6 +70,11 @@ def build_video_yuv422_test(force=False):
     return _build_cpp_test("test_video_yuv422", force)
 
 
+def build_video_y10_test(force=False):
+    """C++ program running processFramesInMemory (csrc/videoprocessingcontext.hpp) on 10-bit luma frames, linked against the .so."""
+    return _build_cpp_test("test_video_y10", force)
+
+
 def _build_cpp_test(name, force):
     src = os.path.join(ROOT, "tests", "cpp", name + ".cpp")
     exe = os.path.join(ROOT, "tests", "cpp", name)
@@ -105,4 +110,5 @@ if __name__ == "__main__":
     print(build_facade_test(force="--force" in sys.argv))
     print(build_video_packed_test(force="--force" in sys.argv))
     print(build_video_yuv422_test(force="--force" in sys.argv))
+    print(build_video_y10_test(force="--force" in sys.argv))
     print(build_generator(force="--force" in sys.argv))

@@ -102,8 +102,9 @@ inline float detectFrameWatermark(const VideoProcessingContext& data, int& frame
 // device: contiguous chunks of the global frame index, one host thread per device, the gate of main.cpp:346,395 on the global
 // index).  `out` receives the Y planes without row padding (gated-off frames copied through), as embedWatermarkFrame writes them.
 // layout 0 (Y planes), a packed colour layout (WM_PACKED_RGB / BGR / RGBA / BGRA, e.g. the BGR frames of cv2.VideoCapture) or a packed
-// 4:2:2 layout (WM_PACKED_YUYV / UYVY, e.g. a V4L2 webcam's YUYV): `linesize` is then the row pitch in bytes and `out` receives dense
-// height x (bytes per pixel * width) frames (wm_video_ctx in wm_b200.h).
+// 4:2:2 layout (WM_PACKED_YUYV / UYVY, e.g. a V4L2 webcam's YUYV) or a 10-bit luma layout (WM_Y10 / WM_Y10_MSB: the Y plane of
+// yuv420p10le / P010, 2 bytes per pixel): `linesize` is then the row pitch in bytes and `out` receives dense height x (bytes per pixel *
+// width) frames (wm_video_ctx in wm_b200.h).
 inline int64_t processFramesInMemory(const std::vector<const Watermark*>& watermarkPerGpu, const int height, const int width,
                                      const int watermarkInterval, const int linesize, const int mode, const uint8_t* frames,
                                      uint8_t* out, const int64_t firstIndex, const int64_t nFrames, float* scalars, const int layout = 0)
@@ -111,6 +112,7 @@ inline int64_t processFramesInMemory(const std::vector<const Watermark*>& waterm
     const int64_t bpp = layout == WM_PACKED_RGB || layout == WM_PACKED_BGR     ? 3
                         : layout == WM_PACKED_RGBA || layout == WM_PACKED_BGRA ? 4
                         : layout == WM_PACKED_YUYV || layout == WM_PACKED_UYVY ? 2
+                        : layout == WM_Y10 || layout == WM_Y10_MSB             ? 2
                                                                                : 1;
     const int ngpus = (int)watermarkPerGpu.size();
     if (ngpus < 1) throw std::runtime_error("processFramesInMemory: no Watermark object\n");

@@ -60,7 +60,7 @@ struct Slot {
     void* stage_base = nullptr; size_t stage_base_cap = 0;
     void* stage_out = nullptr; size_t stage_out_cap = 0;
     void* maskp = nullptr; size_t maskp_cap = 0;  // NVF mask planes of a batch when p > 3 (k_nvfp)
-    void* gray = nullptr; size_t gray_cap = 0;    // gray planes of a packed batch: f32 (k_packed_gray) or the u8 luma of 4:2:2 (k_packed_luma)
+    void* gray = nullptr; size_t gray_cap = 0;    // gray planes of a packed batch: f32 (k_packed_gray, k_packed_y10) or the u8 luma of 4:2:2 (k_packed_luma)
     std::vector<TimedLaunch> timed;
     // direct delivery of synchronous single-image ops (slot 0 only): mapped pinned result + device sequence / completion counters
     HostResult* hres = nullptr;      // pinned host memory
@@ -121,25 +121,28 @@ int fail(wm_ctx* c, int code, const std::string& msg)
             return fail(ctx, WM_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_));        \
     } while (0)
 
-// The packed 8-bit layouts: bytes per pixel (0 = not a packed layout), whether B comes before R, the byte of a pixel that holds its
-// luma (-1: a colour layout, whose RGB gray is computed) and the bytes the packed apply kernel moves in one aligned access of a thread's
-// four pixels.  Every other place reads these facts from here, so a packed layout is described once.
-struct PackedFmt { int bytes; bool bgr; int luma; int apply_vec; const char* name; };
-constexpr PackedFmt PLANAR = {0, false, -1, 0, ""};
+// The packed layouts: bytes per pixel (0 = not a packed layout), whether B comes before R, the byte of a pixel that holds its luma (-1: a
+// colour or 10-bit layout), the bytes the packed apply kernel moves in one aligned access of a thread's four pixels, and for the 10-bit
+// layouts the bit of the little-endian 16-bit word where the sample starts (-1 otherwise; their pointer, ld and batch strides are even).
+// Every other place reads these facts from here, so a packed layout is described once.
+struct PackedFmt { int bytes; bool bgr; int luma; int apply_vec; int shift; const char* name; };
+constexpr PackedFmt PLANAR = {0, false, -1, 0, -1, ""};
 PackedFmt packed_fmt(int layout)
 {
     switch (layout) {
-    case WM_PACKED_RGB: return {3, false, -1, 16, "RGB"};
-    case WM_PACKED_BGR: return {3, true, -1, 16, "BGR"};
-    case WM_PACKED_RGBA: return {4, false, -1, 16, "RGBA"};
-    case WM_PACKED_BGRA: return {4, true, -1, 16, "BGRA"};
-    case WM_PACKED_YUYV: return {2, false, 0, 8, "YUYV"};
-    case WM_PACKED_UYVY: return {2, false, 1, 8, "UYVY"};
+    case WM_PACKED_RGB: return {3, false, -1, 16, -1, "RGB"};
+    case WM_PACKED_BGR: return {3, true, -1, 16, -1, "BGR"};
+    case WM_PACKED_RGBA: return {4, false, -1, 16, -1, "RGBA"};
+    case WM_PACKED_BGRA: return {4, true, -1, 16, -1, "BGRA"};
+    case WM_PACKED_YUYV: return {2, false, 0, 8, -1, "YUYV"};
+    case WM_PACKED_UYVY: return {2, false, 1, 8, -1, "UYVY"};
+    case WM_Y10: return {2, false, -1, 8, 0, "Y10"};
+    case WM_Y10_MSB: return {2, false, -1, 8, 6, "Y10_MSB"};
     default: return PLANAR;
     }
 }
-// bytes of the gray plane one image of a packed layout fills in a slot: f32 L x P for the RGB gray; for 4:2:2 the u8 luma at a pitch of
-// round_up(P, 16), so that its rows are TMA-loadable like a caller's Y plane at that pitch
+// bytes of the gray plane one image of a packed layout fills in a slot: f32 L x P for the RGB gray and for x = v / 4 of the 10-bit
+// layouts; for 4:2:2 the u8 luma at a pitch of round_up(P, 16), so that its rows are TMA-loadable like a caller's Y plane at that pitch
 long long luma_pitch(int P) { return ((long long)P + 15) / 16 * 16; }
 size_t gray_plane_bytes(const PackedFmt& f, int L, int P)
 {
@@ -193,6 +196,7 @@ int make_view(wm_ctx* ctx, const wm_image* im, View* v, bool allow_rgb, bool all
         v->ld = im->ld > 0 ? im->ld : v->row_bytes();
         if (v->ld < v->row_bytes()) return fail(ctx, WM_ERR_ARG, what + ": ld (bytes) smaller than " + std::to_string(f.bytes) + " * cols");
         if (f.luma >= 0 && im->cols % 2) return fail(ctx, WM_ERR_ARG, what + " has an even number of cols (4:2:2 pairs pixels)");
+        if (f.shift >= 0 && ((uintptr_t)im->data % 2 || v->ld % 2)) return fail(ctx, WM_ERR_ARG, what + " has a 2-byte aligned pointer and an even ld (16-bit words)");
         v->pstride = (long long)v->L * v->ld;
         return WM_OK;
     }
@@ -228,8 +232,15 @@ int packed_align(const void* p, long long ld, long long bstride, long long vec =
 // batch stride conventions (include/wm_b200.h): 0 means dense (plane_stride * channels, i.e. L * ld * channels for dense planes); a stride
 // smaller than one image would make the images of a batch overlap.  Resolved once, so the tensor maps, the plain loaders and the
 // apply kernel's base / out addressing all see the same number.
+// a batch stride in bytes between images of a 10-bit layout keeps their 16-bit words aligned
+int check_word_stride(wm_ctx* ctx, const View& v, int64_t stride, const char* what)
+{
+    if (v.fmt.shift >= 0 && stride % 2) return fail(ctx, WM_ERR_ARG, std::string(what) + ": the batch stride of a " + v.fmt.name + " batch is even (16-bit words)");
+    return WM_OK;
+}
 int resolve_stride(wm_ctx* ctx, const View& v, int batch, int64_t* stride, const char* what)
 {
+    if (check_word_stride(ctx, v, *stride, what)) return WM_ERR_ARG;
     // elements spanned by one image, the padding of its last line included
     const long long one = v.pstride * (v.planes() - 1) + (long long)v.L * v.ld;
     if (*stride == 0) *stride = v.pstride * v.planes();
@@ -587,8 +598,9 @@ int reserve_gray(wm_ctx* ctx, Slot& s, size_t need)
 }
 // Packed batch: its gray goes into the slot's planes, and *v / *stride become that gray batch.
 // Colour layouts: the RGB gray, dense f32, so the op runs on it exactly as on a caller's dense f32 gray batch (same tiles, launch plan and
-// partial sums: the scalars of the composed path).  4:2:2 layouts: the luma, u8 at a pitch of round_up(P, 16), so the op runs on it exactly
-// as on a caller's u8 Y plane at that pitch (the same u8 kernels, narrow where TMA holds, and plan: the Y-plane bits).
+// partial sums: the scalars of the composed path).  10-bit layouts: x = v / 4, dense f32, the same way (the bits of the f32 path on x).
+// 4:2:2 layouts: the luma, u8 at a pitch of round_up(P, 16), so the op runs on it exactly as on a caller's u8 Y plane at that pitch (the
+// same u8 kernels, narrow where TMA holds, and plan: the Y-plane bits).
 int enqueue_packed_gray(wm_ctx* ctx, Slot& s, View* v, int64_t* stride, int batch)
 {
     const PackedFmt& f = v->fmt;
@@ -600,6 +612,9 @@ int enqueue_packed_gray(wm_ctx* ctx, Slot& s, View* v, int64_t* stride, int batc
         const long long lp = luma_pitch(v->P);
         launch_packed_luma((const uint8_t*)v->ptr, v->ld, *stride, batch, f.luma, (uint8_t*)s.gray, lp, v->L, v->P, al, 8 * ctx->sms, s.stream);
         v->ld = lp; v->dtype = WM_U8;
+    } else if (f.shift >= 0) {
+        launch_packed_y10((const uint8_t*)v->ptr, v->ld, *stride, batch, f.shift, (float*)s.gray, v->L, v->P, al, 8 * ctx->sms, s.stream);
+        v->ld = v->P; v->dtype = WM_F32;
     } else {
         launch_packed_gray((const uint8_t*)v->ptr, v->ld, *stride, batch, f.bytes, f.bgr, (float*)s.gray, v->L, v->P, al, 8 * ctx->sms, s.stream);
         v->ld = v->P; v->dtype = WM_F32;
@@ -738,7 +753,7 @@ int do_embed(wm_ctx* ctx, int slot, const wm_image* in, const wm_image* base, wm
             ea.b0 = sb.b0; ea.nblk_base = sb.base; ea.nblk_extra = sb.extra;
             const dim3 grid(sb.base + (sb.extra > 0 ? 1 : 0), sb.nb);
             if (ts) launch_apply_ts(vi.dtype, kmask, vi.transposed, narrow, grid, s.stream, tmI, tmW, tmO, ea);
-            else if (packed) launch_apply_packed(kmask, vo.fmt.bytes, vo.fmt.luma, tma, grid, s.stream, tmI, tmW, ea);
+            else if (packed) launch_apply_packed(kmask, vo.fmt.bytes, vo.fmt.luma, vo.fmt.shift, tma, grid, s.stream, tmI, tmW, ea);
             else launch_apply(vi.dtype, vo.dtype, kmask, vi.transposed, tma, grid, s.stream, tmI, tmW, ea);
         }
     }
@@ -1266,6 +1281,9 @@ int wm_embed_host_batch(wm_ctx* ctx, int slot, const wm_image* in, const wm_imag
     View vi, vb, vo;
     int rc;
     if ((rc = make_view(ctx, in, &vi, false, true)) || (rc = make_view(ctx, b, &vb, true, true)) || (rc = make_view(ctx, out, &vo, true, true))) return rc;
+    if ((rc = check_word_stride(ctx, vi, in_stride, "in")) || (rc = check_word_stride(ctx, vb, base_stride, "base")) ||
+        (rc = check_word_stride(ctx, vo, out_stride, "out")))
+        return rc;
     if ((rc = grow_stage(ctx, s, &s.stage_in, &s.stage_in_cap, dense_bytes(vi) * batch))) return rc;
     if ((rc = grow_stage(ctx, s, &s.stage_out, &s.stage_out_cap, dense_bytes(vo) * batch))) return rc;
     const bool base_is_in = vb.ptr == vi.ptr && vb.planes() == 1 && vb.ld == vi.ld && vb.dtype == vi.dtype && vb.layout == vi.layout &&
@@ -1318,7 +1336,7 @@ int wm_detect_host_batch(wm_ctx* ctx, int slot, const wm_image* img, int64_t img
     Slot& s = ctx->slots[slot];
     View v;
     int rc;
-    if ((rc = make_view(ctx, img, &v, false, true))) return rc;
+    if ((rc = make_view(ctx, img, &v, false, true)) || (rc = check_word_stride(ctx, v, img_stride, "image"))) return rc;
     if ((rc = grow_stage(ctx, s, &s.stage_in, &s.stage_in_cap, dense_bytes(v) * batch))) return rc;
     CU(copy_batch(s.stage_in, v, img_stride, batch, true, s.stream));
     wm_image d = dense_desc(img, s.stage_in);
@@ -1492,6 +1510,7 @@ int64_t wm_process_frames(const wm_video_ctx* v, int mode, const uint8_t* frames
     int rc;
     if ((rc = make_view(ctx, &frame, &fv, false, true, true))) return fail(ctx, rc, "frames (ld = linesize): " + ctx->err);
     frame.channels = fv.channels;
+    if ((rc = check_word_stride(ctx, fv, v->frame_stride, "frames (frame_stride)"))) return rc;
     const int64_t H = v->height;
     const int64_t rowb = fv.row_bytes();  // bytes of a frame row without padding
     const int64_t linesize = fv.pitch();

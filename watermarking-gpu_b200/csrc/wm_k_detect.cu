@@ -101,6 +101,14 @@ void launch_packed_luma(const uint8_t* src, long long ld, long long bstride, int
     else k_packed_luma<0><<<grid, 256, 0, st>>>(src, ld, bstride, dst, lp, L, P, align);
 }
 
+void launch_packed_y10(const uint8_t* src, long long ld, long long bstride, int batch, int shift, float* x, int L, int P, int align, int blocks,
+                       cudaStream_t st)
+{
+    const dim3 grid((unsigned)(blocks > batch ? blocks / batch : 1), (unsigned)batch);
+    if (shift) k_packed_y10<6><<<grid, 256, 0, st>>>(src, ld, bstride, x, L, P, align);
+    else k_packed_y10<0><<<grid, 256, 0, st>>>(src, ld, bstride, x, L, P, align);
+}
+
 void launch_transpose(const float* src, float* dst, int rows, int cols, cudaStream_t st)
 {
     const dim3 blk(32, 8), grd((unsigned)((cols + 31) / 32), (unsigned)((rows + 31) / 32));

@@ -27,11 +27,16 @@ void launch_packed_gray(const uint8_t* src, long long ld, long long bstride, int
 // multiple of 16; align as above
 void launch_packed_luma(const uint8_t* src, long long ld, long long bstride, int batch, int luma, uint8_t* dst, long long lp, int L, int P,
                         int align, int blocks, cudaStream_t st);
+// batch of a 10-bit layout (byte ld / stride, both even; the sample at bit `shift` of a little-endian 16-bit word: 0 WM_Y10, 6 WM_Y10_MSB) ->
+// dense f32 planes [batch][L x P] of x = v / 4; align: 2 = src, ld and bstride are multiples of 16 bytes, 1 = of 4 bytes, 0 = of 2 bytes
+void launch_packed_y10(const uint8_t* src, long long ld, long long bstride, int batch, int shift, float* x, int L, int P, int align, int blocks,
+                       cudaStream_t st);
 // apply kernel of a packed image: input = its gray (f32, dense) or, for 4:2:2 images (pixel_bytes 2), its u8 luma plane; base / out = the
 // packed image and the packed output (a.base_vec_ok / a.out_vec_ok: their alignment levels, as for launch_packed_gray; 4:2:2 images: level 2
-// means 8-byte aligned)
-void launch_apply_packed(int mask, int pixel_bytes, int luma, bool tma, dim3 grid, cudaStream_t st, const CUtensorMap& tmI, const CUtensorMap& tmW,
-                         const EmbedArgs& a);
+// means 8-byte aligned).  shift >= 0: a 10-bit layout, whose input is the f32 plane of launch_packed_y10; the base values come from that
+// plane and the base words are only read when the output is the input (status != 0); out_vec_ok level 2 means 8-byte aligned.
+void launch_apply_packed(int mask, int pixel_bytes, int luma, int shift, bool tma, dim3 grid, cudaStream_t st, const CUtensorMap& tmI,
+                         const CUtensorMap& tmW, const EmbedArgs& a);
 }  // namespace wm
 
 // dtype / mask codes shared with include/wm_b200.h
