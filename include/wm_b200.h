@@ -70,6 +70,25 @@
  *     detect: the correlation the f32 path gives on x.
  *   A mix of WM_Y10 and WM_Y10_MSB, or of either with a planar or another packed layout, is refused with WM_ERR_ARG, as are wm_rgb2gray,
  *   wm_debug_plane and wm_debug_detect_planes.
+ *
+ * 10-bit 4:2:2 v210, as SDI capture cards hand it over (Blackmagic DeckLink bmdFormat10BitYUV, AJA), and as ffmpeg's v210 codec and
+ * uncompressed 10-bit QuickTime / MOV files hold it:
+ *   WM_PACKED_V210 : a row is a sequence of 16-byte groups of four little-endian 32-bit words, 6 pixels per group, 10-bit fields:
+ *                      w0: Cb0 [0:10)  Y0 [10:20)  Cr0 [20:30)      w1: Y1  [0:10)  Cb1 [10:20)  Y2  [20:30)
+ *                      w2: Cr1 [0:10)  Y3 [10:20)  Cb2 [20:30)      w3: Y4  [0:10)  Cr2 [10:20)  Y5  [20:30)
+ *                    bits 30-31 of every word hold no sample.  The row pitch is WM_V210_PITCH(cols) = ((cols + 47) / 48) * 128 bytes
+ *                    (5,120 at 1920 cols, 10,240 at 3840, 3,456 at 1280); when cols % 6 != 0 the last group holds 2 or 4 pixels and its
+ *                    other luma fields are not pixels.
+ *   (Its value is 12.)  dtype must be WM_U8 and channels 0 (the layout fixes the packing); cols even; `ld` is in BYTES (0 = the pitch,
+ *   otherwise >= the pitch); the data pointer, `ld` and batch strides (bytes) are multiples of 4.  The arithmetic is WM_Y10's: the luma
+ *   sample v is processed as x = v * 0.25f.  Taken by the same entry points as the other packed layouts:
+ *     embed: in_gray = the image, base = NULL or the same image, out = a v210 image not overlapping in.  `a`, the status and the new luma
+ *            v' = (uint16_t)clamp(4.0f*y, 0, 1023) are those of WM_Y10 on the same samples.  In out, exactly the luma fields of the
+ *            image's pixels change: every other bit of a row's first pitch bytes (chroma, bits 30-31, unused luma fields of a partial last
+ *            group, pad groups up to the pitch) is copied from in, and bytes of out past the pitch are not written.  WM_SINGULAR /
+ *            WM_ZERO_MASK: out receives in's pitch bytes unchanged.  wm_embed_verify_host_batch detects on the written words.
+ *     detect: the correlation the f32 path gives on x of the luma.
+ *   A mix of v210 with any other layout is refused with WM_ERR_ARG, as are wm_rgb2gray, wm_debug_plane and wm_debug_detect_planes.
  */
 #ifndef WM_B200_H
 #define WM_B200_H
@@ -83,7 +102,9 @@ extern "C" {
 /* Watermark.hpp:10-14 — enum MASK_TYPE { ME, NVF } */
 enum { WM_MASK_ME = 0, WM_MASK_NVF = 1 };
 enum { WM_COL_MAJOR = 0, WM_ROW_MAJOR = 1, WM_PACKED_RGB = 2, WM_PACKED_BGR = 3, WM_PACKED_RGBA = 4, WM_PACKED_BGRA = 5, WM_PACKED_YUYV = 6,
-       WM_PACKED_UYVY = 7, WM_Y10 = 10, WM_Y10_MSB = 11 };
+       WM_PACKED_UYVY = 7, WM_Y10 = 10, WM_Y10_MSB = 11, WM_PACKED_V210 = 12 };
+/* bytes of a WM_PACKED_V210 row of `cols` pixels: whole 128-byte blocks of 48 pixels */
+#define WM_V210_PITCH(cols) ((((int64_t)(cols) + 47) / 48) * 128)
 enum { WM_F32 = 0, WM_U8 = 1 };
 
 /* return codes: 0 ok; >0 non-fatal (mirrors the reference's fall-backs); <0 errors */
@@ -106,9 +127,9 @@ typedef struct wm_image {
     void *data;            /* DEVICE pointer (wm_*_host entry points take HOST pointers instead) */
     int64_t rows, cols;
     int64_t ld;            /* leading dimension in elements, bytes for packed images (0 = dense) */
-    int32_t channels;      /* 1, or 3 for the RGB base/out of makeWatermark (Watermark.cpp:171); bytes per pixel (2, 3 or 4) for packed images */
+    int32_t channels;      /* 1, or 3 for the RGB base/out of makeWatermark (Watermark.cpp:171); bytes per pixel (2, 3 or 4) for packed images, 0 for v210 */
     int32_t layout;        /* WM_COL_MAJOR | WM_ROW_MAJOR | WM_PACKED_RGB | WM_PACKED_BGR | WM_PACKED_RGBA | WM_PACKED_BGRA | WM_PACKED_YUYV |
-                              WM_PACKED_UYVY | WM_Y10 | WM_Y10_MSB */
+                              WM_PACKED_UYVY | WM_Y10 | WM_Y10_MSB | WM_PACKED_V210 */
     int32_t dtype;         /* WM_F32 | WM_U8 */
     int32_t reserved;
     int64_t plane_stride;  /* elements between channel planes (0 = dense) */
@@ -141,7 +162,7 @@ enum {
     WM_OPT_NARROW_U8 = 14,    /* 1 (default): the stats / apply kernels of u8 frames (TMA path) run on 128-thread CTAs, 4 warps x 8 lines of a tile, four CTAs per SM,
                                  like the sweep; 0: 256-thread CTAs, 8 warps x 4 lines, three per SM.  Same bits */
     WM_OPT_RUN_MB = 15,       /* frames of one run (one batched launch sequence) of wm_process_frames on DEVICE frames fill at most this many MB (default 136, at most
-                                 32 frames; packed frames count their packed bytes, 2 per pixel for 10-bit frames): large enough to amortise a launch's ramp and tail, small enough that a run's watermarked frames are still in L2 when
+                                 32 frames; packed frames count their packed bytes, 2 per pixel for 10-bit frames, the row pitch for v210): large enough to amortise a launch's ramp and tail, small enough that a run's watermarked frames are still in L2 when
                                  the detector's kernels read them back */
     WM_OPT_HOST_RUN_FRAMES = 9, /* frames per run (one batched launch sequence + its copies) of wm_process_frames when frames are in HOST memory; default 4 */
     WM_OPT_F32_SOLVE = 8      /* 0 (default): the 8x8 system is summed and solved in f64 (pivot cut 1e-12 max|Rx|); 1: Rx / rx are rounded to f32
@@ -251,7 +272,11 @@ int64_t wm_launch_count(const wm_ctx *ctx); /* kernels launched by this ctx sinc
  * 10-bit luma frames (layout = WM_Y10 / WM_Y10_MSB: the Y plane of yuv420p10le and the like, or of NVDEC's P010): height rows of 2 * width
  * bytes, `linesize` the row pitch in bytes (>= 2 * width and even, 0 = dense; frame_stride even), `out` dense height x (2 * width)
  * frames.  A gated frame gets exactly what wm_embed / wm_detect give that image with the ME mask; EMBED_VERIFY detects on the written
- * words.  Gated-off frames are copied through, all 16 bits of every word.  The chroma planes stay with the caller, as for 8-bit Y planes. */
+ * words.  Gated-off frames are copied through, all 16 bits of every word.  The chroma planes stay with the caller, as for 8-bit Y planes.
+ * v210 frames (layout = WM_PACKED_V210: DeckLink bmdFormat10BitYUV, ffmpeg v210): height rows, `linesize` the row pitch in bytes (0 = the
+ * format's pitch WM_V210_PITCH(width), otherwise at least that and a multiple of 4; frame_stride a multiple of 4), `out` frames of height
+ * rows at the format's pitch.  A gated frame gets exactly what wm_embed / wm_detect give that image with the ME mask; EMBED_VERIFY detects
+ * on the written frame while it is still on the device.  Gated-off frames are copied through, every byte of a row's pitch. */
 typedef struct wm_video_ctx {
     wm_ctx *watermark;        /* watermarkObj (non-owning) */
     int32_t height, width;
@@ -261,7 +286,7 @@ typedef struct wm_video_ctx {
     int32_t frames_on_device; /* 1: `frames`/`out` are device pointers; 0: host (pinned recommended) */
     int32_t layout;           /* 0 or WM_ROW_MAJOR: Y planes; WM_PACKED_RGB | WM_PACKED_BGR | WM_PACKED_RGBA | WM_PACKED_BGRA: packed u8
                                  colour frames; WM_PACKED_YUYV | WM_PACKED_UYVY: packed 4:2:2 frames; WM_Y10 | WM_Y10_MSB: 10-bit luma
-                                 frames; anything else is refused with WM_ERR_ARG */
+                                 frames; WM_PACKED_V210: v210 frames; anything else is refused with WM_ERR_ARG */
 } wm_video_ctx;
 enum { WM_VIDEO_EMBED = 0, WM_VIDEO_DETECT = 1, WM_VIDEO_EMBED_VERIFY = 2 };
 /* Processes frames [first_index, first_index + n_frames) of a stream: frame i is gated by

@@ -24,8 +24,21 @@ PACKED_RGBA, PACKED_BGRA = 4, 5     # the same with a fourth byte per pixel (row
 PACKED_YUYV, PACKED_UYVY = 6, 7     # packed 4:2:2 (rows, cols, 2): luma at [..., 0] / [..., 1], chroma copied through by the embed
 Y10, Y10_MSB = 10, 11               # 10-bit luma (rows, cols) uint16: the sample in bits 0-9 (yuv420p10le Y) / 6-15 (P010 Y)
 WORD_LAYOUTS = (Y10, Y10_MSB)       # one little-endian 16-bit word per pixel
+PACKED_V210 = 12                    # 10-bit 4:2:2 v210 (rows, >= v210_pitch(cols)) uint8: the bytes of its rows, chroma copied through by the embed
 PACKED_BYTES = {PACKED_RGB: 3, PACKED_BGR: 3, PACKED_RGBA: 4, PACKED_BGRA: 4, PACKED_YUYV: 2, PACKED_UYVY: 2, Y10: 2, Y10_MSB: 2}  # bytes per pixel of each packed layout
 F32, U8 = 0, 1
+
+
+def v210_pitch(cols):
+    """Bytes of a v210 row of `cols` pixels (WM_V210_PITCH): whole 128-byte blocks of 48 pixels."""
+    return (cols + 47) // 48 * 128
+
+
+def row_bytes(layout, cols):
+    """Bytes of a row of `cols` pixels of a packed layout (v210: its pitch)."""
+    return v210_pitch(cols) if layout == PACKED_V210 else PACKED_BYTES[layout] * cols
+
+
 OK, SINGULAR, ZERO_MASK = 0, 1, 2
 OPT_FP16_PRODUCTS, OPT_KERNEL_TIMING, OPT_USE_TMA, OPT_SERIAL_SLOTS, OPT_CUDA_GRAPHS, OPT_MMA_ACCUM, OPT_SPLIT_COST = 1, 2, 3, 4, 5, 6, 7
 OPT_F32_SOLVE, OPT_HOST_RUN_FRAMES, OPT_TMA_STORE, OPT_PDL, OPT_FUSED_SINGLE, OPT_PADDED_UPLOAD, OPT_NARROW_U8, OPT_RUN_MB = 8, 9, 10, 11, 12, 13, 14, 15
@@ -165,20 +178,22 @@ class DeviceArray:
 
     Planar layouts hold (rows, cols) or (3, rows, cols) images, `ld` in elements.  The packed layouts hold a (rows, cols, n) uint8
     image, n = PACKED_BYTES[layout], as interleaved rows of n * cols bytes with a row pitch of `ld` bytes (0 = dense); the 10-bit layouts
-    (WORD_LAYOUTS) a (rows, cols) uint16 image, as rows of little-endian words."""
+    (WORD_LAYOUTS) a (rows, cols) uint16 image, as rows of little-endian words; PACKED_V210 a (rows, >= v210_pitch(cols)) uint8 array of
+    the bytes of its rows, of which the first v210_pitch(cols) are the row (`ld` bytes apart on the device, 0 = the pitch)."""
 
     def __init__(self, wm, rows, cols, layout=COL_MAJOR, dtype=F32, channels=1, ld=0):
-        if layout in PACKED_BYTES:
-            dtype, channels = U8, PACKED_BYTES[layout]
+        packed = layout in PACKED_BYTES or layout == PACKED_V210
+        if packed:
+            dtype, channels = U8, PACKED_BYTES.get(layout, 0)
         self.wm, self.rows, self.cols, self.layout, self.dtype, self.channels = wm, rows, cols, layout, dtype, channels
         P = rows if layout == COL_MAJOR else cols
         Ln = cols if layout == COL_MAJOR else rows
-        if layout in PACKED_BYTES:
-            P = channels * cols  # bytes of a row
+        if packed:
+            P = row_bytes(layout, cols)  # bytes of a row
         self.ld = ld if ld else P
         self.P, self.L = P, Ln
         self.itemsize = 4 if dtype == F32 else 1
-        planes = 1 if layout in PACKED_BYTES else self.channels
+        planes = 1 if packed else self.channels
         self.nbytes = planes * Ln * self.ld * self.itemsize
         self.ptr = lib().wm_dev_alloc(wm._h, self.nbytes)
         if not self.ptr:
@@ -187,8 +202,12 @@ class DeviceArray:
     @classmethod
     def from_numpy(cls, wm, img, layout=COL_MAJOR, ld=0):
         """img: (rows, cols) or (3, rows, cols) numpy array in logical (row, col) indexing; (rows, cols, PACKED_BYTES[layout]) uint8
-        for a packed layout."""
+        for a packed layout; (rows, >= v210_pitch(wm.cols)) uint8 for PACKED_V210, an image of the watermark's width."""
         img = np.asarray(img)
+        if layout == PACKED_V210:
+            d = cls(wm, img.shape[0], wm.cols, layout, ld=ld)
+            d.upload(img)
+            return d
         if layout in PACKED_BYTES:
             d = cls(wm, img.shape[0], img.shape[1], layout, ld=ld)
             d.upload(img)
@@ -200,6 +219,10 @@ class DeviceArray:
         return d
 
     def _to_mem(self, img):
+        if self.layout == PACKED_V210:
+            buf = np.zeros((self.L, self.ld), np.uint8)
+            buf[:, :self.P] = np.asarray(img, np.uint8).reshape(self.rows, -1)[:, :self.P]
+            return buf
         if self.layout in WORD_LAYOUTS:
             img = np.ascontiguousarray(np.asarray(img).astype("<u2", casting="same_kind")).view(np.uint8)
         if self.layout in PACKED_BYTES:
@@ -220,7 +243,7 @@ class DeviceArray:
             raise WatermarkError(rc, "upload failed")
 
     def numpy(self):
-        if self.layout in PACKED_BYTES:
+        if self.layout in PACKED_BYTES or self.layout == PACKED_V210:
             buf = np.empty((self.L, self.ld), np.uint8)
             rc = lib().wm_dev_download(self.wm._h, buf.ctypes.data, self.ptr, buf.nbytes)
             if rc:
@@ -228,6 +251,8 @@ class DeviceArray:
             px = np.ascontiguousarray(buf[:, :self.P])
             if self.layout in WORD_LAYOUTS:
                 return px.view("<u2").astype(np.uint16).reshape(self.rows, self.cols)
+            if self.layout == PACKED_V210:
+                return px
             return px.reshape(self.rows, self.cols, self.channels)
         buf = np.empty((self.channels, self.L, self.ld), _NP_DT[self.dtype])
         rc = lib().wm_dev_download(self.wm._h, buf.ctypes.data, self.ptr, buf.nbytes)
@@ -348,6 +373,10 @@ class Watermark:
 
     # -- hot path, host (numpy) arrays: H2D + compute + D2H inside the call -------------------------
     def _host_desc(self, arr, layout):
+        if layout == PACKED_V210:  # (rows, >= pitch) uint8, the bytes of each row contiguous; rows may be pitched
+            if arr.dtype != np.uint8 or arr.ndim != 2 or arr.strides[1] != 1 or arr.shape[1] < v210_pitch(self.cols):
+                raise TypeError("a v210 host image is a (rows, >= v210_pitch(cols)) uint8 array with contiguous rows")
+            return image_desc(arr.ctypes.data, self.rows, self.cols, layout, U8, arr.strides[0], 0, 0)
         if layout in WORD_LAYOUTS:  # (rows, cols) uint16, pixels contiguous; rows may be pitched
             if arr.dtype != np.uint16 or arr.ndim != 2 or arr.strides[1] != 2:
                 raise TypeError("an image of a 10-bit layout is a (rows, cols) uint16 array with contiguous pixels")
@@ -480,13 +509,14 @@ class VideoProcessingContext:
 
     layout 0 (Y planes), a packed colour layout (PACKED_RGB / BGR / RGBA / BGRA: e.g. the BGR frames of cv2.VideoCapture) or a packed
     4:2:2 layout (PACKED_YUYV / UYVY: e.g. a V4L2 webcam's YUYV) or a 10-bit luma layout (Y10 / Y10_MSB: the Y plane of yuv420p10le or
-    P010); linesize is the row pitch in bytes (default: dense rows of PACKED_BYTES[layout] * width bytes)."""
+    P010) or PACKED_V210 (e.g. a DeckLink's 10-bit YUV); linesize is the row pitch in bytes (default: dense rows of
+    PACKED_BYTES[layout] * width bytes, v210_pitch(width) for v210)."""
 
     def __init__(self, watermark, height, width, watermark_interval, linesize=0, frame_stride=0, frames_on_device=False, layout=0):
         self.watermarkObj, self.height, self.width = watermark, height, width
         self.watermarkInterval = watermark_interval
         self.layout = layout
-        self._c = wm_video_ctx(watermark._h, height, width, watermark_interval, linesize or PACKED_BYTES.get(layout, 1) * width,
+        self._c = wm_video_ctx(watermark._h, height, width, watermark_interval, linesize or (v210_pitch(width) if layout == PACKED_V210 else PACKED_BYTES.get(layout, 1) * width),
                                frame_stride, int(frames_on_device), layout)
 
 

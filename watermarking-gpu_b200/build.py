@@ -75,6 +75,11 @@ def build_video_y10_test(force=False):
     return _build_cpp_test("test_video_y10", force)
 
 
+def build_video_v210_test(force=False):
+    """C++ program running processFramesInMemory (csrc/videoprocessingcontext.hpp) on v210 frames, linked against the .so."""
+    return _build_cpp_test("test_video_v210", force)
+
+
 def _build_cpp_test(name, force):
     src = os.path.join(ROOT, "tests", "cpp", name + ".cpp")
     exe = os.path.join(ROOT, "tests", "cpp", name)
@@ -111,4 +116,5 @@ if __name__ == "__main__":
     print(build_video_packed_test(force="--force" in sys.argv))
     print(build_video_yuv422_test(force="--force" in sys.argv))
     print(build_video_y10_test(force="--force" in sys.argv))
+    print(build_video_v210_test(force="--force" in sys.argv))
     print(build_generator(force="--force" in sys.argv))

@@ -103,8 +103,9 @@ inline float detectFrameWatermark(const VideoProcessingContext& data, int& frame
 // index).  `out` receives the Y planes without row padding (gated-off frames copied through), as embedWatermarkFrame writes them.
 // layout 0 (Y planes), a packed colour layout (WM_PACKED_RGB / BGR / RGBA / BGRA, e.g. the BGR frames of cv2.VideoCapture) or a packed
 // 4:2:2 layout (WM_PACKED_YUYV / UYVY, e.g. a V4L2 webcam's YUYV) or a 10-bit luma layout (WM_Y10 / WM_Y10_MSB: the Y plane of
-// yuv420p10le / P010, 2 bytes per pixel): `linesize` is then the row pitch in bytes and `out` receives dense height x (bytes per pixel *
-// width) frames (wm_video_ctx in wm_b200.h).
+// yuv420p10le / P010, 2 bytes per pixel) or v210 (WM_PACKED_V210, e.g. a DeckLink's bmdFormat10BitYUV): `linesize` is then the row pitch in
+// bytes and `out` receives dense height x (bytes per pixel * width) frames, v210 frames at the format's pitch WM_V210_PITCH(width)
+// (wm_video_ctx in wm_b200.h).
 inline int64_t processFramesInMemory(const std::vector<const Watermark*>& watermarkPerGpu, const int height, const int width,
                                      const int watermarkInterval, const int linesize, const int mode, const uint8_t* frames,
                                      uint8_t* out, const int64_t firstIndex, const int64_t nFrames, float* scalars, const int layout = 0)
@@ -114,6 +115,7 @@ inline int64_t processFramesInMemory(const std::vector<const Watermark*>& waterm
                         : layout == WM_PACKED_YUYV || layout == WM_PACKED_UYVY ? 2
                         : layout == WM_Y10 || layout == WM_Y10_MSB             ? 2
                                                                                : 1;
+    const int64_t rowb = layout == WM_PACKED_V210 ? WM_V210_PITCH(width) : bpp * width;  // bytes of an `out` row
     const int ngpus = (int)watermarkPerGpu.size();
     if (ngpus < 1) throw std::runtime_error("processFramesInMemory: no Watermark object\n");
     if (mode == WM_VIDEO_EMBED_VERIFY && ngpus > 1) throw std::runtime_error("processFramesInMemory: EMBED_VERIFY runs on one GPU per call\n");
@@ -127,7 +129,7 @@ inline int64_t processFramesInMemory(const std::vector<const Watermark*>& waterm
         ctx[(size_t)g] = wm_video_ctx{watermarkPerGpu[(size_t)g]->handle(), height, width, watermarkInterval, linesize, 0, 0, layout};
         pc.push_back(&ctx[(size_t)g]);
         in.push_back(frames + first * (int64_t)height * linesize);
-        ou.push_back(out ? out + first * (int64_t)height * bpp * width : nullptr);
+        ou.push_back(out ? out + first * (int64_t)height * rowb : nullptr);
     }
     const int64_t n = ngpus == 1 ? wm_process_frames(pc[0], mode, in[0], ou[0], firstIndex, nFrames, scalars)
                                  : wm_process_frames_multi(pc.data(), ngpus, mode, in.data(), out ? ou.data() : nullptr, firstIndex, nFrames, scalars);

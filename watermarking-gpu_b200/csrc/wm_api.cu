@@ -121,42 +121,50 @@ int fail(wm_ctx* c, int code, const std::string& msg)
             return fail(ctx, WM_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_));        \
     } while (0)
 
-// The packed layouts: bytes per pixel (0 = not a packed layout), whether B comes before R, the byte of a pixel that holds its luma (-1: a
-// colour or 10-bit layout), the bytes the packed apply kernel moves in one aligned access of a thread's four pixels, and for the 10-bit
-// layouts the bit of the little-endian 16-bit word where the sample starts (-1 otherwise; their pointer, ld and batch strides are even).
-// Every other place reads these facts from here, so a packed layout is described once.
-struct PackedFmt { int bytes; bool bgr; int luma; int apply_vec; int shift; const char* name; };
-constexpr PackedFmt PLANAR = {0, false, -1, 0, -1, ""};
+// The packed layouts: bytes per pixel (0 = not a whole number: v210), whether B comes before R, the byte of a pixel that holds its luma
+// (-1: a colour or 10-bit layout), the bytes the packed apply kernel moves in one aligned access of a thread's four pixels, for the 10-bit
+// layouts the bit of the little-endian 16-bit word where the sample starts (-1 otherwise; the op runs on x = v / 4 when it is >= 0), the
+// bytes the pointer, ld and batch strides are multiples of (16-bit words: 2, v210's 32-bit words: 4), and whether the pixels are packed in
+// v210 groups (6 pixels in 16 bytes, the WM_Y10 apply's words merged into them by k_pack_v210).  Every other place reads these facts from
+// here, so a packed layout is described once.
+struct PackedFmt {
+    int bytes; bool bgr; int luma; int apply_vec; int shift; int word; bool v210; const char* name;
+    long long row_bytes(int P) const { return v210 ? WM_V210_PITCH(P) : (long long)P * bytes; }  // of a P-pixel row; v210: its pitch
+};
+constexpr PackedFmt PLANAR = {0, false, -1, 0, -1, 0, false, ""};
 PackedFmt packed_fmt(int layout)
 {
     switch (layout) {
-    case WM_PACKED_RGB: return {3, false, -1, 16, -1, "RGB"};
-    case WM_PACKED_BGR: return {3, true, -1, 16, -1, "BGR"};
-    case WM_PACKED_RGBA: return {4, false, -1, 16, -1, "RGBA"};
-    case WM_PACKED_BGRA: return {4, true, -1, 16, -1, "BGRA"};
-    case WM_PACKED_YUYV: return {2, false, 0, 8, -1, "YUYV"};
-    case WM_PACKED_UYVY: return {2, false, 1, 8, -1, "UYVY"};
-    case WM_Y10: return {2, false, -1, 8, 0, "Y10"};
-    case WM_Y10_MSB: return {2, false, -1, 8, 6, "Y10_MSB"};
+    case WM_PACKED_RGB: return {3, false, -1, 16, -1, 1, false, "RGB"};
+    case WM_PACKED_BGR: return {3, true, -1, 16, -1, 1, false, "BGR"};
+    case WM_PACKED_RGBA: return {4, false, -1, 16, -1, 1, false, "RGBA"};
+    case WM_PACKED_BGRA: return {4, true, -1, 16, -1, 1, false, "BGRA"};
+    case WM_PACKED_YUYV: return {2, false, 0, 8, -1, 1, false, "YUYV"};
+    case WM_PACKED_UYVY: return {2, false, 1, 8, -1, 1, false, "UYVY"};
+    case WM_Y10: return {2, false, -1, 8, 0, 2, false, "Y10"};
+    case WM_Y10_MSB: return {2, false, -1, 8, 6, 2, false, "Y10_MSB"};
+    case WM_PACKED_V210: return {0, false, -1, 8, 0, 4, true, "v210"};
     default: return PLANAR;
     }
 }
 // bytes of the gray plane one image of a packed layout fills in a slot: f32 L x P for the RGB gray and for x = v / 4 of the 10-bit
-// layouts; for 4:2:2 the u8 luma at a pitch of round_up(P, 16), so that its rows are TMA-loadable like a caller's Y plane at that pitch
+// layouts; for 4:2:2 the u8 luma at a pitch of round_up(P, 16), so that its rows are TMA-loadable like a caller's Y plane at that pitch.
+// v210 adds the L x P 16-bit words of the WM_Y10 apply, after the batch's f32 planes (v210_words)
 long long luma_pitch(int P) { return ((long long)P + 15) / 16 * 16; }
 size_t gray_plane_bytes(const PackedFmt& f, int L, int P)
 {
+    if (f.v210) return (size_t)L * (size_t)P * (sizeof(float) + sizeof(uint16_t)) + 16;
     return f.luma >= 0 ? (size_t)L * (size_t)luma_pitch(P) : (size_t)L * (size_t)P * sizeof(float);
 }
 // An image reduced to planes of L lines x P pixels; ld and pstride are in elements.  A packed image is one plane of L = rows lines of
 // P = cols pixels, ld in bytes, dtype u8 and channels = bytes per pixel.
 struct View {
     void* ptr; int L, P; long long ld, pstride; int channels; int dtype; bool transposed;
-    int layout; PackedFmt fmt;  // fmt.bytes == 0: a planar image
-    bool packed() const { return fmt.bytes != 0; }
+    int layout; PackedFmt fmt;  // fmt.word == 0: a planar image
+    bool packed() const { return fmt.word != 0; }
     long long elem() const { return dtype == WM_F32 ? 4 : 1; }
     int planes() const { return packed() ? 1 : channels; }
-    long long row_bytes() const { return (long long)P * (packed() ? fmt.bytes : elem()); }  // of a line's pixels, without its padding
+    long long row_bytes() const { return packed() ? fmt.row_bytes(P) : P * elem(); }  // of a line's pixels, without its padding
     long long pitch() const { return ld * elem(); }
     long long plane_bytes() const { return pstride * elem(); }
     long long extent() const { return (planes() - 1) * plane_bytes() + (L - 1) * pitch() + row_bytes(); }  // first byte to past the last pixel
@@ -194,9 +202,11 @@ int make_view(wm_ctx* ctx, const wm_image* im, View* v, bool allow_rgb, bool all
         v->channels = f.bytes;
         v->dtype = WM_U8;
         v->ld = im->ld > 0 ? im->ld : v->row_bytes();
-        if (v->ld < v->row_bytes()) return fail(ctx, WM_ERR_ARG, what + ": ld (bytes) smaller than " + std::to_string(f.bytes) + " * cols");
-        if (f.luma >= 0 && im->cols % 2) return fail(ctx, WM_ERR_ARG, what + " has an even number of cols (4:2:2 pairs pixels)");
-        if (f.shift >= 0 && ((uintptr_t)im->data % 2 || v->ld % 2)) return fail(ctx, WM_ERR_ARG, what + " has a 2-byte aligned pointer and an even ld (16-bit words)");
+        if (v->ld < v->row_bytes())
+            return fail(ctx, WM_ERR_ARG, what + ": ld (bytes) smaller than " + (f.v210 ? "the row pitch, ((cols + 47) / 48) * 128" : std::to_string(f.bytes) + " * cols"));
+        if ((f.luma >= 0 || f.v210) && im->cols % 2) return fail(ctx, WM_ERR_ARG, what + " has an even number of cols (4:2:2 pairs pixels)");
+        if ((uintptr_t)im->data % f.word || v->ld % f.word)
+            return fail(ctx, WM_ERR_ARG, what + (f.word == 2 ? " has a 2-byte aligned pointer and an even ld (16-bit words)" : " has a 4-byte aligned pointer and ld (32-bit words)"));
         v->pstride = (long long)v->L * v->ld;
         return WM_OK;
     }
@@ -232,10 +242,11 @@ int packed_align(const void* p, long long ld, long long bstride, long long vec =
 // batch stride conventions (include/wm_b200.h): 0 means dense (plane_stride * channels, i.e. L * ld * channels for dense planes); a stride
 // smaller than one image would make the images of a batch overlap.  Resolved once, so the tensor maps, the plain loaders and the
 // apply kernel's base / out addressing all see the same number.
-// a batch stride in bytes between images of a 10-bit layout keeps their 16-bit words aligned
+// a batch stride in bytes between images of a 10-bit layout keeps their 16-bit (v210: 32-bit) words aligned
 int check_word_stride(wm_ctx* ctx, const View& v, int64_t stride, const char* what)
 {
-    if (v.fmt.shift >= 0 && stride % 2) return fail(ctx, WM_ERR_ARG, std::string(what) + ": the batch stride of a " + v.fmt.name + " batch is even (16-bit words)");
+    if (v.packed() && stride % v.fmt.word)
+        return fail(ctx, WM_ERR_ARG, std::string(what) + ": the batch stride of a " + v.fmt.name + " batch is " + (v.fmt.word == 2 ? "even (16-bit words)" : "a multiple of 4 (32-bit words)"));
     return WM_OK;
 }
 int resolve_stride(wm_ctx* ctx, const View& v, int batch, int64_t* stride, const char* what)
@@ -599,6 +610,7 @@ int reserve_gray(wm_ctx* ctx, Slot& s, size_t need)
 // Packed batch: its gray goes into the slot's planes, and *v / *stride become that gray batch.
 // Colour layouts: the RGB gray, dense f32, so the op runs on it exactly as on a caller's dense f32 gray batch (same tiles, launch plan and
 // partial sums: the scalars of the composed path).  10-bit layouts: x = v / 4, dense f32, the same way (the bits of the f32 path on x).
+// v210 the same way on x of its luma, so a v210 batch gets WM_Y10's bits.
 // 4:2:2 layouts: the luma, u8 at a pitch of round_up(P, 16), so the op runs on it exactly as on a caller's u8 Y plane at that pitch (the
 // same u8 kernels, narrow where TMA holds, and plan: the Y-plane bits).
 int enqueue_packed_gray(wm_ctx* ctx, Slot& s, View* v, int64_t* stride, int batch)
@@ -612,6 +624,9 @@ int enqueue_packed_gray(wm_ctx* ctx, Slot& s, View* v, int64_t* stride, int batc
         const long long lp = luma_pitch(v->P);
         launch_packed_luma((const uint8_t*)v->ptr, v->ld, *stride, batch, f.luma, (uint8_t*)s.gray, lp, v->L, v->P, al, 8 * ctx->sms, s.stream);
         v->ld = lp; v->dtype = WM_U8;
+    } else if (f.v210) {
+        launch_packed_v210((const uint8_t*)v->ptr, v->ld, *stride, batch, (float*)s.gray, v->L, v->P, al, 8 * ctx->sms, s.stream);
+        v->ld = v->P; v->dtype = WM_F32;
     } else if (f.shift >= 0) {
         launch_packed_y10((const uint8_t*)v->ptr, v->ld, *stride, batch, f.shift, (float*)s.gray, v->L, v->P, al, 8 * ctx->sms, s.stream);
         v->ld = v->P; v->dtype = WM_F32;
@@ -626,6 +641,12 @@ int enqueue_packed_gray(wm_ctx* ctx, Slot& s, View* v, int64_t* stride, int batc
     v->fmt = PLANAR;
     *stride = (int64_t)v->pstride;
     return WM_OK;
+}
+
+// the 16-bit words a v210 embed's WM_Y10 apply writes: dense L x P per image, after the batch's f32 planes of x (gray_plane_bytes)
+uint16_t* v210_words(const Slot& s, int L, int P, int batch)
+{
+    return (uint16_t*)((char*)s.gray + ((size_t)batch * L * P * sizeof(float) + 15) / 16 * 16);
 }
 
 size_t stats_part_offset(const Plan& pl, int batch) { return (size_t)batch * (size_t)pl.nsweep * NTOT; }
@@ -718,6 +739,18 @@ int do_embed(wm_ctx* ctx, int slot, const wm_image* in, const wm_image* base, wm
     // packed base / out: alignment levels (the apply kernel's vector access, word or byte accesses)
     ea.base_vec_ok = packed ? packed_align(vb.ptr, vb.ld, base_stride, vb.fmt.apply_vec) : vec_ok(vb.ptr, vb.ld, base_stride, vb.channels > 1 ? vb.pstride : 0, vb.dtype);
     ea.out_vec_ok = packed ? packed_align(vo.ptr, vo.ld, out_stride, vo.fmt.apply_vec) : vec_ok(vo.ptr, vo.ld, out_stride, vo.channels > 1 ? vo.pstride : 0, vo.dtype);
+    // v210: the WM_Y10 apply writes v' into the slot's dense words, and k_pack_v210 merges them into the output's groups afterwards, so
+    // the pack kernel, the op's last, publishes a direct result.  The apply's own copy-through (WM_SINGULAR / WM_ZERO_MASK) copies the
+    // words onto themselves; k_pack_v210 then copies the input groups and reads no word.
+    const bool v210 = vo.fmt.v210;
+    if (v210) {
+        uint16_t* words = v210_words(s, g.L, g.P, batch);
+        ea.base = ea.out = words;
+        ea.base_ld = ea.out_ld = 2LL * g.P;
+        ea.base_bstride = ea.out_bstride = 2LL * g.L * g.P;
+        ea.base_vec_ok = ea.out_vec_ok = packed_align(words, ea.out_ld, ea.out_bstride, vo.fmt.apply_vec);
+        ea.dl = deliver_args(s, false);
+    }
     CUtensorMap tmI, tmW;
     memset(&tmI, 0, sizeof tmI);
     memset(&tmW, 0, sizeof tmW);
@@ -756,9 +789,21 @@ int do_embed(wm_ctx* ctx, int slot, const wm_image* in, const wm_image* base, wm
             else if (packed) launch_apply_packed(kmask, vo.fmt.bytes, vo.fmt.luma, vo.fmt.shift, tma, grid, s.stream, tmI, tmW, ea);
             else launch_apply(vi.dtype, vo.dtype, kmask, vi.transposed, tma, grid, s.stream, tmI, tmW, ea);
         }
+        if (v210) {
+            PackV210Args pa;
+            pa.in = (const uint8_t*)vb.ptr; pa.in_ld = vb.ld; pa.in_bstride = base_stride;
+            pa.words = (const uint16_t*)ea.out;
+            pa.out = (uint8_t*)vo.ptr; pa.out_ld = vo.ld; pa.out_bstride = out_stride;
+            pa.scal = s.scal;
+            pa.L = g.L; pa.P = g.P;
+            pa.dl = deliver_args(s, direct && batch == 1);
+            const bool a16 = packed_align(vb.ptr, vb.ld, base_stride) == 2 && packed_align(vo.ptr, vo.ld, out_stride) == 2;
+            launch_pack_v210(pa, a16, batch, 8 * ctx->sms, s.stream);
+            ctx->launches++;
+        }
     }
     CU(cudaGetLastError());
-    if (direct && batch == 1) return WM_OK;  // the apply kernel's last CTA publishes the scalars itself
+    if (direct && batch == 1) return WM_OK;  // the apply kernel's (v210: the pack kernel's) last CTA publishes the scalars itself
     return push_result(ctx, s, 1, batch);
 }
 

@@ -54,6 +54,13 @@ void launch_apply_packed(int mask, int pixel_bytes, int luma, int shift, bool tm
 #undef WM_PKS
 }
 
+void launch_pack_v210(const PackV210Args& a, bool a16, int batch, int blocks, cudaStream_t st)
+{
+    const dim3 grid((unsigned)(blocks > batch ? blocks / batch : 1), (unsigned)batch);
+    if (a16) k_pack_v210<true><<<grid, 256, 0, st>>>(a);
+    else k_pack_v210<false><<<grid, 256, 0, st>>>(a);
+}
+
 void launch_apply(int in_dtype, int out_dtype, int mask, bool tr, bool tma, dim3 grid, cudaStream_t st, const CUtensorMap& tmI,
                   const CUtensorMap& tmW, const EmbedArgs& a)
 {

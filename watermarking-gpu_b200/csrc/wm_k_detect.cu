@@ -109,6 +109,13 @@ void launch_packed_y10(const uint8_t* src, long long ld, long long bstride, int 
     else k_packed_y10<0><<<grid, 256, 0, st>>>(src, ld, bstride, x, L, P, align);
 }
 
+void launch_packed_v210(const uint8_t* src, long long ld, long long bstride, int batch, float* x, int L, int P, int align, int blocks, cudaStream_t st)
+{
+    const dim3 grid((unsigned)(blocks > batch ? blocks / batch : 1), (unsigned)batch);
+    if (align == 2) k_packed_v210<true><<<grid, 256, 0, st>>>(src, ld, bstride, x, L, P);
+    else k_packed_v210<false><<<grid, 256, 0, st>>>(src, ld, bstride, x, L, P);
+}
+
 void launch_transpose(const float* src, float* dst, int rows, int cols, cudaStream_t st)
 {
     const dim3 blk(32, 8), grd((unsigned)((cols + 31) / 32), (unsigned)((rows + 31) / 32));

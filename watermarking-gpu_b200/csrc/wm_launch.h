@@ -31,6 +31,13 @@ void launch_packed_luma(const uint8_t* src, long long ld, long long bstride, int
 // dense f32 planes [batch][L x P] of x = v / 4; align: 2 = src, ld and bstride are multiples of 16 bytes, 1 = of 4 bytes, 0 = of 2 bytes
 void launch_packed_y10(const uint8_t* src, long long ld, long long bstride, int batch, int shift, float* x, int L, int P, int align, int blocks,
                        cudaStream_t st);
+// v210 batch (byte ld / stride, both multiples of 4; P even) -> dense f32 planes [batch][L x P] of x = v / 4; align: 2 = src, ld and bstride
+// are multiples of 16 bytes, else of 4
+void launch_packed_v210(const uint8_t* src, long long ld, long long bstride, int batch, float* x, int L, int P, int align, int blocks,
+                        cudaStream_t st);
+// v210 output batch: the input groups with their luma fields replaced by the WM_Y10 apply's words (k_pack_v210); a16: in and out
+// (pointers, ld, batch strides) are multiples of 16 bytes
+void launch_pack_v210(const PackV210Args& a, bool a16, int batch, int blocks, cudaStream_t st);
 // apply kernel of a packed image: input = its gray (f32, dense) or, for 4:2:2 images (pixel_bytes 2), its u8 luma plane; base / out = the
 // packed image and the packed output (a.base_vec_ok / a.out_vec_ok: their alignment levels, as for launch_packed_gray; 4:2:2 images: level 2
 // means 8-byte aligned).  shift >= 0: a 10-bit layout, whose input is the f32 plane of launch_packed_y10; the base values come from that
