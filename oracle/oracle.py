@@ -61,6 +61,8 @@ def lib():
         L.wmo_pred_error_mask.argtypes = [fp, C.c_int, C.c_int, op, fp, fp, fp, dp, dp]
         L.wmo_embed.argtypes = [fp, fp, C.c_int, C.c_int, C.c_int, fp, C.c_float, C.c_int, op, fp, fp,
                                 fp, fp, fp]
+        L.wmo_apply.argtypes = [fp, fp, C.c_size_t, C.c_float, C.c_int, fp]
+        L.wmo_apply.restype = None
         L.wmo_detect.argtypes = [fp, C.c_int, C.c_int, fp, C.c_int, op, fp, fp, fp, fp, fp]
         L.wmo_embed_frame_u8.argtypes = [u8p, C.c_int, C.c_int, C.c_int, fp, C.c_float, C.c_int, op, u8p,
                                          fp]
@@ -152,6 +154,18 @@ def embed(img, W, psnr, mask_type, base=None, o=FAITHFUL):
                          out.ctypes.data_as(fp), C.byref(a), mask.ctypes.data_as(fp), u.ctypes.data_as(fp),
                          coef.ctypes.data_as(fp))
     return dict(status=st, out=out, a=a.value, mask=mask, u=u, coef=coef)
+
+
+def apply(base, u, a, o=FAITHFUL):
+    """The apply step of makeWatermark alone (Watermark.cpp:171): clamp(base + u*a, 0, 255) in f32, fused
+    like embed() when o.contract.  base and u: arrays of one shape; a: the strength (rounded to f32)."""
+    base, bp = _f(base)
+    u, up = _f(u)
+    if u.shape != base.shape:
+        raise ValueError("u has shape %s, base %s" % (u.shape, base.shape))
+    out = np.empty_like(base)
+    lib().wmo_apply(bp, up, base.size, C.c_float(a), o.contract, out.ctypes.data_as(C.POINTER(C.c_float)))
+    return out
 
 
 def detect(img, W, mask_type, o=FAITHFUL):

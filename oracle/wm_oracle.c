@@ -319,6 +319,21 @@ int wmo_pred_error_mask(const float *img, int rows, int cols, const wmo_opts *o,
 }
 
 /*
+ * Watermark.cpp:171 — out = clamp(base + u*a, 0, 255) over n pixels of one plane.
+ * ArrayFire JIT fuses clamp(out + u*a) into one OpenCL kernel; FP_CONTRACT defaults ON in
+ * OpenCL C, so the mul-add may fuse (`contract`: one rounding, fmaf).  Exposed on its own so
+ * that tests can apply a strength and a u plane taken from the GPU.
+ */
+void wmo_apply(const float *base, const float *u, size_t n, float a, int contract, float *out)
+{
+#pragma omp parallel for schedule(static)
+    for (size_t i = 0; i < n; i++) {
+        float v = contract ? fmaf(u[i], a, base[i]) : base[i] + u[i] * a;
+        out[i] = v < 0.0f ? 0.0f : (v > 255.0f ? 255.0f : v);
+    }
+}
+
+/*
  * Watermark.cpp:156-172 — makeWatermark.
  * in: gray rows*cols; base/out: channels planes of rows*cols (channels 1 or 3;
  * the reference broadcasts u*a over the RGB planes, Watermark.cpp:171).
@@ -358,17 +373,8 @@ int wmo_embed(const float *in, const float *base, int channels, int rows, int co
             memcpy(out, base, n * channels * sizeof(float));
             status = 2;
         } else {
-            for (int ch = 0; ch < channels; ch++) {
-                const float *b = base + (size_t)ch * n;
-                float *d = out + (size_t)ch * n;
-#pragma omp parallel for schedule(static)
-                for (size_t i = 0; i < n; i++) {
-                    /* ArrayFire JIT fuses clamp(out + u*a) into one OpenCL kernel; FP_CONTRACT
-                     * defaults ON in OpenCL C, so the mul-add may fuse (option `contract`) */
-                    float v = o->contract ? fmaf(u[i], av, b[i]) : b[i] + u[i] * av;
-                    d[i] = v < 0.0f ? 0.0f : (v > 255.0f ? 255.0f : v);
-                }
-            }
+            for (int ch = 0; ch < channels; ch++)
+                wmo_apply(base + (size_t)ch * n, u, n, av, o->contract, out + (size_t)ch * n);
         }
     }
     if (!mask_out) free(mask);

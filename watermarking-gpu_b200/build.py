@@ -80,6 +80,21 @@ def build_video_v210_test(force=False):
     return _build_cpp_test("test_video_v210", force)
 
 
+_scratch = None
+
+
+def _writable_or_scratch(exe):
+    """`exe` itself where its directory can be written; otherwise (a read-only checkout whose program is missing or older than its
+    sources) a path of the same name in a temporary directory of this process, so that a read-only tree still builds and runs it."""
+    global _scratch
+    if os.access(os.path.dirname(exe), os.W_OK):
+        return exe
+    if _scratch is None:
+        import tempfile
+        _scratch = tempfile.mkdtemp(prefix="wm_b200_build_")
+    return os.path.join(_scratch, os.path.basename(exe))
+
+
 def _build_cpp_test(name, force):
     src = os.path.join(ROOT, "tests", "cpp", name + ".cpp")
     exe = os.path.join(ROOT, "tests", "cpp", name)
@@ -88,8 +103,13 @@ def _build_cpp_test(name, force):
     deps = [src, os.path.join(CSRC, "Watermark.hpp"), os.path.join(CSRC, "videoprocessingcontext.hpp"), LIB]
     if not force and os.path.exists(exe) and all(os.path.getmtime(d) <= os.path.getmtime(exe) for d in deps if os.path.exists(d)):
         return exe
+    exe = _writable_or_scratch(exe)
+    if not force and os.path.exists(exe) and all(os.path.getmtime(d) <= os.path.getmtime(exe) for d in deps if os.path.exists(d)):
+        return exe
+    # in the tree the program finds the library relative to itself; from a temporary directory, at its absolute path
+    rpath = "$ORIGIN/../../watermarking-gpu_b200" if exe.startswith(ROOT + os.sep) else HERE
     cmd = ["/usr/bin/g++", "-O2", "-std=c++20", "-I", os.path.join(ROOT, "include"), "-I", CSRC, "-o", exe, src,
-           "-L", HERE, "-lwm_b200", "-Wl,-rpath,$ORIGIN/../../watermarking-gpu_b200", "-ldl", "-lpthread", "-lrt"]
+           "-L", HERE, "-lwm_b200", "-Wl,-rpath," + rpath, "-ldl", "-lpthread", "-lrt"]
     r = subprocess.run(cmd, capture_output=True, text=True)
     if r.returncode != 0:
         raise RuntimeError("g++ failed:\n" + " ".join(cmd) + "\n" + r.stdout + r.stderr)
@@ -102,6 +122,9 @@ def build_generator(force=False):
     exe = os.path.join(ROOT, "tools", "CommonRandomMatrix", "CommonRandomMatrix")
     if not os.path.exists(src):
         return None
+    if not force and os.path.exists(exe) and os.path.getmtime(exe) >= os.path.getmtime(src):
+        return exe
+    exe = _writable_or_scratch(exe)
     if not force and os.path.exists(exe) and os.path.getmtime(exe) >= os.path.getmtime(src):
         return exe
     r = subprocess.run(["/usr/bin/g++", "-O2", "-std=c++17", "-o", exe, src], capture_output=True, text=True)
