@@ -21,12 +21,14 @@ ME, NVF = 0, 1
 
 class Opts(C.Structure):
     _fields_ = [("fp16_products", C.c_int), ("sum_f32", C.c_int), ("solve_f32", C.c_int),
-                ("contract", C.c_int), ("p", C.c_int)]
+                ("contract", C.c_int), ("p", C.c_int), ("rx_f64", C.c_int)]
 
 
-def opts(fp16_products=1, sum_f32=0, solve_f32=0, contract=1, p=3):
-    """Canonical (default) = reference-faithful fp16 products, f64 sums/solve, fused mul-add, 3x3 NVF window."""
-    return Opts(fp16_products, sum_f32, solve_f32, contract, p)
+def opts(fp16_products=1, sum_f32=0, solve_f32=0, contract=1, p=3, rx_f64=0):
+    """Canonical (default) = reference-faithful fp16 products, f64 sums/solve, fused mul-add, 3x3 NVF window.
+    rx_f64=1: rx() adds every term in f64 (RN16(RN32(x*y)) with fp16_products, the exact x*y without) instead of summing
+    64-pixel groups in f32 — a reference without f32 rounding of its own, to bound the GPU's f32 sums by."""
+    return Opts(fp16_products, sum_f32, solve_f32, contract, p, rx_f64)
 
 
 FAITHFUL = opts()

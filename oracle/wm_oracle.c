@@ -34,6 +34,10 @@
  *                       NVIDIA OpenCL behaviour), 0 = separately rounded
  *   p             : NVF window size (3 unless stated; the ME parts are p = 3 only,
  *                   as in the reference)
+ *   rx_f64        : 0 = wmo_rx sums each 64-pixel group in f32 (the reference's
+ *                       work-groups), 1 = every term is added in f64 — RN16(RN32(x*y))
+ *                       with fp16_products, the exact x*y without — so the sums carry
+ *                       no f32 rounding of their own (a reference to bound f32 sums by)
  */
 #include <math.h>
 #include <stdint.h>
@@ -50,6 +54,7 @@ typedef struct {
     int solve_f32;
     int contract;
     int p;              /* NVF window size 3, 5, 7 or 9 (Watermark.cpp:24, kernels/nvf.hpp:14-17); 0 = 3 */
+    int rx_f64;
 } wmo_opts;
 
 enum { WMO_ME = 0, WMO_NVF = 1 }; /* Watermark.hpp:10-14 */
@@ -132,8 +137,45 @@ void wmo_nvf(const float *img, int rows, int cols, float *mask, const wmo_opts *
  * Output: Rx[8*8] (full symmetric), rx[8] as doubles (holding f32 values when
  * sum_f32 is set).
  */
+/* rx_f64: the same 44 terms per pixel (same neighbours, same clamp to the edge), each added in f64: one f64 partial per
+ * row, rows added in ascending order (the same bits for any thread count) */
+static void rx_terms_f64(const float *img, int rows, int cols, int fp16, double *tot)
+{
+    double *part = (double *)calloc((size_t)rows * 44, sizeof(double));
+#pragma omp parallel for schedule(static)
+    for (int r = 0; r < rows; r++) {
+        double acc[44];
+        for (int t = 0; t < 44; t++) acc[t] = 0.0;
+        for (int c = 0; c < cols; c++) {
+            float n[8];
+            for (int k = 0; k < 8; k++) n[k] = px(img, rows, cols, r + DY[k], c + DX[k]);
+            const float cur = img[(size_t)r * cols + c];
+            int t = 0;
+            for (int k = 0; k < 8; k++, t++)
+                acc[t] += fp16 ? (double)round_fp16(n[k] * cur) : (double)n[k] * (double)cur;
+            for (int i = 0; i < 8; i++)
+                for (int j = i; j < 8; j++, t++)
+                    acc[t] += fp16 ? (double)round_fp16(n[i] * n[j]) : (double)n[i] * (double)n[j];
+        }
+        for (int t = 0; t < 44; t++) part[(size_t)r * 44 + t] = acc[t];
+    }
+    for (int t = 0; t < 44; t++) tot[t] = 0.0;
+    for (int r = 0; r < rows; r++)
+        for (int t = 0; t < 44; t++) tot[t] += part[(size_t)r * 44 + t];
+    free(part);
+}
+
 void wmo_rx(const float *img, int rows, int cols, const wmo_opts *o, double *Rx, double *rx)
 {
+    if (o->rx_f64) {
+        double tot[44];
+        rx_terms_f64(img, rows, cols, o->fp16_products, tot);
+        for (int k = 0; k < 8; k++) rx[k] = tot[k];
+        int t = 8;
+        for (int i = 0; i < 8; i++)
+            for (int j = i; j < 8; j++, t++) Rx[i * 8 + j] = Rx[j * 8 + i] = tot[t];
+        return;
+    }
     const int gpr = (cols + 63) / 64; /* groups per row */
     const size_t ngroups = (size_t)rows * gpr;
     float *part = (float *)malloc(ngroups * 44 * sizeof(float)); /* [44][ngroups] */

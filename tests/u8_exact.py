@@ -53,7 +53,7 @@ def gamma(n, u):
     return n * u / (1.0 - n * u)
 
 
-def sum_rel_bound(k, n):
+def sum_rel_bound(k, n, u=U32):
     """Bound on |S_gpu / S_ref - 1| for S = sum of n nonnegative terms t = x^2 of f32 values x (the stats kernel's sum2 = sum (m.W)^2,
     the detector's |e_z|^2 and |e_u|^2).
 
@@ -62,9 +62,10 @@ def sum_rel_bound(k, n):
     f64 exactly and are added there in some tree of at most n values: another gamma_n(2^-53) of the total.
     Reference: the f64 sum of the exact squares (x^2 of an f32 x has 48 significant bits): within gamma_n(2^-53) of the exact sum.
     Together |S_gpu - S_ref| <= (gamma_k(2^-24) + 3 gamma_n(2^-53)) S_exact, and S_exact <= S_ref / (1 - gamma_n(2^-53)).
-    k = 32 (narrow u8 kernels): 1.91e-6."""
+    k = 32 (narrow u8 kernels): 1.91e-6.  u: the relative error of one step of the chain where it is not an f32 round-to-nearest
+    addition (f32_exact.U_MMA: one step of the tensor pipe's accumulation)."""
     g = gamma(n, U64)
-    return (gamma(k, U32) + 3 * g) / (1 - g)
+    return (gamma(k, u) + 3 * g) / (1 - g)
 
 
 def dot_abs_bound(k, n, nz_ref, nu_ref):
